@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- profiled trajectories/s of the batched spline -> motion-profile engine on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config cfg2|cfg3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config cfg2|cfg3] [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (build_path -> tables -> distance sampling -> forward/backward ->
 time-domain resampling) over one batch of synthetic random-node paths.
@@ -19,6 +19,14 @@ time-domain resampling) over one batch of synthetic random-node paths.
 bounded sample of the same workload; the unmodified Python reference itself (baseline/_ref, staged by
 baseline/make_ref.py) is timed next to it as cpu_baseline.reference_python when it travelled with the snapshot.
 Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR: after the timed steps rank 0 writes what the last timed step returned as DIR/<name>.npy (float64, at
+  most 64 MB in all), so that two builds can be compared output for output on the same seeded inputs.  cfg2 (and
+  --profile-step): `summary` [B, 5] (n_out, total length, t_end, max|v|, status) and `n_samples` [B] of every path, and for
+  a fixed, seeded sample of paths (`paths`, ascending) their `nodes_map` / `actions_map` rows (-1 padded) and each output
+  stream (times, positions, linear_vels, accelerations, headings, angular_vels, x, y, and the pass velocities `vel`) with
+  the sampled paths' rows cut at n_out (vel: n_samples) and concatenated in `paths` order.  cfg3 and --impl reference:
+  the `summary` rows the job returns.
 """
 from __future__ import annotations
 
@@ -37,6 +45,7 @@ import numpy as np  # noqa: E402
 
 UNIT = "trajectories/s"
 FACTORY_CONS = dict(max_vel=4.0, max_acc=8.0, max_dec=8.0, friction_coef=0.8, max_jerk=16.0, track_width=12.5 / 12)
+DUMP_BYTES = 64 << 20
 
 
 def metric_name(nodes: int) -> str:
@@ -90,6 +99,61 @@ class ClockSampler:
                     reasons.add(nm)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+def write_dump(dirname, arrays):
+    """Every array as DIR/<name>.npy in float64; more than DUMP_BYTES in all is an error."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed {DUMP_BYTES}")
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), a)
+
+
+def summary_dump(rows, seed=0):
+    """The summary rows of a job; a job too large for DUMP_BYTES keeps a fixed, seeded sample of its rows (`paths`)."""
+    rows = np.asarray(rows)
+    cap = DUMP_BYTES // (8 * (rows.shape[1] + 1))
+    if len(rows) <= cap:
+        return {"summary": rows}
+    paths = np.sort(np.random.default_rng(seed).choice(len(rows), cap, replace=False))
+    return {"summary": rows[paths], "paths": paths}
+
+
+def profile_dump(res, max_paths=256, seed=0):
+    """A ProfileResult as the arrays of --dump-outputs (module docstring).  The seeded sample is the first `max_paths` of
+    a fixed permutation of the batch, halved (the same permutation's shorter prefix) until the arrays fit DUMP_BYTES."""
+    import torch
+    from vexautonomousplanner_b200.engine import OUT_NAMES
+    summary = res.summary.cpu().numpy()
+    n_out = res.n_out.cpu().numpy().astype(np.int64)
+    n_samples = res.n_samples.cpu().numpy().astype(np.int64)
+    n_maps = res.n_maps.cpu().numpy()
+    order = np.random.default_rng(seed).permutation(res.B)
+    width = res.nodes_map.shape[1] + res.actions_map.shape[1]
+
+    def nbytes(p):
+        return 8 * (summary.size + res.B + len(p) * (1 + width) + len(OUT_NAMES) * n_out[p].sum() + n_samples[p].sum())
+
+    k = min(res.B, max_paths)
+    while k > 1 and nbytes(order[:k]) > DUMP_BYTES:
+        k //= 2
+    paths = np.sort(order[:k])
+    idx = torch.as_tensor(paths, device=res.out.device)
+    out = res.out[:, idx, :int(n_out[paths].max())].cpu().numpy()
+    vel = res.vel[idx, :int(n_samples[paths].max())].cpu().numpy()
+    dump = {"summary": summary, "n_samples": n_samples, "paths": paths}
+    for name, maps, lens in (("nodes_map", res.nodes_map, n_maps[paths, 0]), ("actions_map", res.actions_map, n_maps[paths, 1])):
+        m = maps[idx].cpu().numpy().astype(np.int64)
+        m[np.arange(m.shape[1])[None, :] >= lens[:, None]] = -1
+        dump[name] = m
+    for i, name in enumerate(OUT_NAMES):
+        dump[name] = np.concatenate([out[i, j, :n_out[p]] for j, p in enumerate(paths)])
+    dump["vel"] = np.concatenate([vel[j, :n_samples[p]] for j, p in enumerate(paths)])
+    return dump
 
 
 # ------------------------------------------------------------------------------------------------ CPU baselines
@@ -191,8 +255,10 @@ def run_reference(args):
         oracle.full_batch(sub.node_attr, sub.node_flags, sub.cons, threads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.full_batch(sub.node_attr, sub.node_flags, sub.cons, threads=threads)
+        s = oracle.full_batch(sub.node_attr, sub.node_flags, sub.cons, threads=threads)
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, summary_dump(s))
     value = sample * args.steps / el
     pyref = None if args.no_pyref else python_reference_rate(packed, 2 * threads, threads)
     line = {
@@ -355,8 +421,10 @@ def run_cfg2(args):
         l0 = eng.launches
         for _ in range(args.steps):
             flush.zero_()
-            eng.profile(db, reuse_plan=True)
+            res = eng.profile(db, reuse_plan=True)
         torch.cuda.synchronize()
+        if args.dump_outputs and rank == 0:
+            write_dump(args.dump_outputs, profile_dump(res))
         print(json.dumps({"profile_step": True, "steps": args.steps, "launches_per_step": (eng.launches - l0) // args.steps}))
         return
     depth = max(1, args.pipeline)
@@ -368,18 +436,19 @@ def run_cfg2(args):
         gatherer.submit(res.summary)                  # snapshot + all_gather on a side stream: nobody waits for it
 
     def run_steps(K):
-        """K steps enqueued back to back; returns the device time of the whole region (events on the caller's stream)."""
+        """K steps enqueued back to back; returns the events around the whole region (on the caller's stream) and the
+        result of the last step."""
         s = torch.cuda.Event(enable_timing=True); e = torch.cuda.Event(enable_timing=True)
         s.record(main)
         for k in range(K):
             with torch.cuda.stream(pipe.streams[pipe.n % depth]):
                 pipe.streams[pipe.n % depth].wait_stream(main)
                 flush.zero_()                         # L2 flushed before every step (on the step's own stream)
-            pipe.submit(None, consume)
+            last = pipe.submit(None, consume)
         pipe.drain()
         gatherer.wait()
         e.record(main)
-        return s, e
+        return s, e, last
 
     def barrier():
         if world > 1:
@@ -393,7 +462,7 @@ def run_cfg2(args):
     l0 = eng.launches
     barrier()
     wall0 = time.perf_counter()
-    s, e = run_steps(args.steps)
+    s, e, last = run_steps(args.steps)
     barrier()
     wall = time.perf_counter() - wall0
     launches = (eng.launches - l0) // args.steps
@@ -408,6 +477,8 @@ def run_cfg2(args):
     assert bool((res.status == 0).all().item())
     allrows = gatherer.rows()
     assert allrows.shape == (world * B, 5) and bool((allrows[:, 4] == 0).all().item())
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, profile_dump(last))      # before the replays below overwrite the graphs' outputs
 
     # ---------------- unpipelined latency of one step (one graph replay at a time, per-step events)
     lat = []
@@ -632,6 +703,8 @@ def run_cfg3(args):
     assert bool(ok.all().item()), "paths with a non-zero status"
     allrows = gatherer.rows()
     assert allrows.shape == (B, 5)
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, summary_dump(allrows.cpu().numpy()))
 
     # roofline with every path's actual Q, P, D, T (SURVEY.md 8d): B_path = 8 (2Q + 2P + 10D + 9T) + 88 N
     Dsum = float(counters[:Bl, 0].sum().item()); Tsum = float(counters[:Bl, 1].sum().item())
@@ -711,6 +784,8 @@ def main():
     ap.add_argument("--e2e-tiles", type=int, default=1, help="tiles of the end-to-end (host in / host out) run")
     ap.add_argument("--profile-step", action="store_true",
                     help="cfg2: run only warm-up + K eager, unpipelined steps (the command profiles/tools/capture.sh puts under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 3 if args.config == "cfg3" else 10
