@@ -15,7 +15,8 @@
  *   - return value: 0 on success, <0 on a launch/argument error (text via vap_last_error()).
  *     Per-path failures never abort the batch: they are reported in status[B]:
  *        0 ok | -1 reference returns False | -2 reference raises IndexError
- *        -3 reference raises ValueError    | -4 caller capacity (D_cap / T_cap) too small
+ *        -3 reference raises ValueError    | -4 caller capacity too small: D_cap / T_cap, or a max_splines (Q_cap of the
+ *           distance table) below the path's own spline count
  *        -5 the reference's time loop would not terminate for this input (e.g. max_dec >= 20 ft/s^2 makes a step
  *           move backwards) or would emit more than 5e7 rows: the engine stops instead of hanging the GPU
  *        -6 more node crossings / action-point candidates than the per-path event tables hold (N_max wraps,
@@ -96,9 +97,10 @@ int vap_eval(int64_t n, const int32_t* path, const double* t, int which, int N_m
              void* stream);
 
 /* S1  build_lookup_table (spline_manager.py:426-475): samples per spline (reference default 1000).
- *     lut_d/lut_t[B][Q_cap] with Q_cap >= samples * max_b n_splines[b]; total_len[B].               */
+ *     lut_d/lut_t[B][Q_cap] with Q_cap >= samples * max_b n_splines[b]; total_len[B].  status is in/out: a path with
+ *     samples * n_splines[b] > Q_cap gets VAP_ERR_CAPACITY (and total_len 0), which every later stage skips.       */
 int vap_build_lut(int64_t B, int N_max, const double* seg, const int32_t* first_node, const double* param_end,
-                  const int32_t* n_splines, const int32_t* status, int samples, int64_t Q_cap, double* lut_d,
+                  const int32_t* n_splines, int32_t* status, int samples, int64_t Q_cap, double* lut_d,
                   double* lut_t, double* total_len, void* stream);
 /* Optional accelerator of distance_to_time (spline_manager.py:291-318): an inverse index of the distance table, so that
  *     np.searchsorted(distances, d) is one seeded lookup plus a verification against the table instead of a 10-level
@@ -243,10 +245,13 @@ int vap_build_lerp_recip(int64_t n, double dd, double* rden, void* stream);
  * (its true counts are still in n_samples / n_out), the others are unaffected.  need[3] (device i64, may be NULL) receives
  * the batch maxima {distance samples, estimated time samples incl. inserted rows, a sufficient T_cap from the time loop's own
  * iteration count (0 while the distance samples did not fit)} over the paths that
- * are healthy or only lacked capacity: read it back to size a retry.  Paths whose length or travel time is absurd (the
- * reference's loops would not terminate) get VAP_ERR_DIVERGED.
+ * are healthy or only lacked capacity: read it back to size a retry.  need[] does not report the spline count: a path with
+ * more splines than max_splines also gets VAP_ERR_CAPACITY (n_samples = n_out = 0), and the caller finds the batch's true
+ * count from vap_build_path's n_splines.  Paths whose length or travel time is absurd (the reference's loops would not
+ * terminate) get VAP_ERR_DIVERGED.
  * Inputs: the packed node / action-point tables of vap_build_path / vap_velocity_profile; max_splines >= max_b n_splines[b]
- * (1 + the number of reverse / turn nodes; N_max - 1 is always enough); dgrid[n_grid >= D_cap + 2] from vap_build_dgrid and
+ * (1 + the number of interior reverse / turn nodes; N_max - 1 is always enough; a smaller value gives VAP_ERR_CAPACITY on
+ * exactly the paths that have more splines); dgrid[n_grid >= D_cap + 2] from vap_build_dgrid and
  * rden[n_rden] from vap_build_lerp_recip (or NULL): path-independent, depend on dd only, build them once.
  * Outputs: out[8][B][T_cap] (planes out_plane_stride elements apart, 0 = B*T_cap): times, positions, linear_vels,
  * accelerations, headings, angular_vels, x, y; n_out[B]; nodes_map[B][N_max+1]; actions_map[B][max(A_max,1)]; n_maps[B][2];

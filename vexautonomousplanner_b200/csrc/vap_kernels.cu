@@ -310,7 +310,7 @@ __global__ void k_eval(long long n, const int* __restrict__ path, const double* 
 __global__ void __launch_bounds__(256) k_build_lut(int N_max, const double* __restrict__ seg,
                                                    const int* __restrict__ first_node,
                                                    const double* __restrict__ param_end,
-                                                   const int* __restrict__ n_splines, const int* __restrict__ status,
+                                                   const int* __restrict__ n_splines, int* __restrict__ status,
                                                    int samples, long long Q_cap, double* __restrict__ lut_d,
                                                    double* __restrict__ lut_t, double* __restrict__ total_len)
 {
@@ -319,8 +319,15 @@ __global__ void __launch_bounds__(256) k_build_lut(int N_max, const double* __re
     PathGeo g = path_geo(b, N_max, seg, first_node, param_end, n_splines);
     double* od = lut_d + (size_t)b * Q_cap;
     double* ot = lut_t + (size_t)b * Q_cap;
-    if (status[b] != ST_OK || g.S <= 0 || (long long)g.S * samples > Q_cap) {
-        if (threadIdx.x == 0) total_len[b] = 0.0;
+    const int st = status[b];
+    const bool too_many = (long long)g.S * samples > Q_cap;     // more splines than the caller's max_splines
+    if (st != ST_OK || g.S <= 0 || too_many) {
+        __syncthreads();                                         // every thread has read status[b] before it changes
+        if (threadIdx.x == 0) {
+            total_len[b] = 0.0;
+            // the row cannot hold this path's table: a capacity failure the caller retries, never a silent empty path
+            if (st == ST_OK && too_many) status[b] = ST_CAPACITY;
+        }
         return;
     }
     double current = 0.0, prev_param = 0.0;
@@ -1039,7 +1046,7 @@ extern "C" int vap_eval(int64_t n, const int32_t* path, const double* t, int whi
 }
 
 extern "C" int vap_build_lut(int64_t B, int N_max, const double* seg, const int32_t* first_node,
-                             const double* param_end, const int32_t* n_splines, const int32_t* status, int samples,
+                             const double* param_end, const int32_t* n_splines, int32_t* status, int samples,
                              int64_t Q_cap, double* lut_d, double* lut_t, double* total_len, void* stream)
 {
     if (B <= 0) return 0;

@@ -11,7 +11,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 from contextlib import contextmanager
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, replace
 from typing import Dict, Optional
 
 import numpy as np
@@ -183,6 +183,15 @@ class Engine:
 
     def upload(self, p: PackedPaths) -> DeviceBatch:
         return DeviceBatch.from_packed(p, self.device)
+
+    def _with_true_splines(self, db: DeviceBatch, n_splines: Optional[torch.Tensor] = None) -> DeviceBatch:
+        """db, or a DeviceBatch over the same tensors that carries the batch's true spline count when db.max_splines
+        understates it (e.g. a captured graph's static inputs with another batch copied in).  The count is the geometry
+        kernel's own n_splines (0 for failed paths); without them, one vap_build_path runs here (retry path only)."""
+        if n_splines is None:
+            n_splines = self.build_geometry(db).n_splines
+        S = int(n_splines.max().item()) if n_splines.numel() else 0
+        return replace(db, max_splines=S) if S > db.max_splines else db
 
     def dgrid(self, n: int) -> torch.Tensor:
         """Accumulated distance grid d_{i+1} = fl(d_i + dd), cached and grown geometrically."""
@@ -657,6 +666,9 @@ class Engine:
         key = (db.B, db.N_max, db.A_max, db.max_splines)
         if key not in self._plan:
             self.profile(db, reuse_plan=False)
+        if key not in self._plan:
+            # db understates its spline count: profile() redid (and planned) the batch under its true count
+            key = key[:3] + (self._with_true_splines(db).max_splines,)
         D_cap, T_cap = self._plan[key]
         if margin > 1.0:
             D_cap, T_cap = (int(D_cap * margin) + 127) // 128 * 128, int(T_cap * margin) + 64
@@ -701,7 +713,11 @@ class Engine:
         res.extra = dict(need=need, workspace=ws)
         if _retry < MAX_RETRIES and bool((status == ST_CAPACITY).any().item()):
             d_need, t_est, t_exact = (int(v) for v in need.tolist())
-            return self.profile_batch(db, max(D_cap, d_need + 8), max(T_cap, int(max(t_est, t_exact) * 1.10) + 64), _retry + 1)
+            # need[] does not cover paths with more splines than db.max_splines (they were stopped before sampling): the
+            # redo carries the true count, which can only be short once, so that redo does not use up a retry
+            exact = self._with_true_splines(db)
+            return self.profile_batch(exact, max(D_cap, d_need + 8), max(T_cap, int(max(t_est, t_exact) * 1.10) + 64),
+                                      _retry + (1 if exact is db else 0))
         return res
 
     # ------------------------------------------------------------------ whole path
@@ -775,11 +791,13 @@ class Engine:
             # capacity check (one small read-back; also what a caller needs to trim the rows)
             if bool((status == ST_CAPACITY).any().item()):
                 if bool((status_pre == ST_CAPACITY).any().item()):
-                    # distance capacity was too small: drop the plan and redo with exact sizing (bounded: a status that
-                    # survives the exact re-runs is reported, never retried forever)
+                    # distance capacity (or db.max_splines, which sizes the distance table) was too small: drop the plan
+                    # and redo with exact sizing and the geometry's true spline count (bounded: a status that survives
+                    # the exact re-runs is reported, never retried forever)
                     self._plan.pop(key, None)
                     if _retry < MAX_RETRIES:
-                        return self.profile(db, keep=keep, reuse_plan=False, _retry=_retry + 1)
+                        return self.profile(self._with_true_splines(db, g.n_splines), keep=keep, reuse_plan=False,
+                                            _retry=_retry + 1)
                 if self.time_impl == "split":
                     # n_main is exact even on overflow; inserted rows are bounded by the insert estimate
                     T_cap = int(self._n_main.max().item()) + min(int(self._insert_bound(db, status_pre)), int(ROW_LIMIT)) + 8
@@ -851,13 +869,9 @@ class GraphedProfile:
             raise ValueError("graph capture needs the fast path (velocity_impl='chunked', time_impl='split')")
         self.eng, self.db, self.tiles = eng, db, max(1, min(tiles, db.B))
         self.host: Optional[HostResult] = None
-        key = (db.B, db.N_max, db.A_max, db.max_splines)
         warm = eng.profile(db, reuse_plan=True)                # sizes the plan, builds the distance grid
-        self.D_cap, self.T_cap = eng._plan[key]
-        if margin > 1.0:
-            self.D_cap = (int(self.D_cap * margin) + 127) // 128 * 128
-            self.T_cap = int(self.T_cap * margin) + 64
-            eng._plan[key] = (max(self.D_cap, eng._plan[key][0]), max(self.T_cap, eng._plan[key][1]))
+        # the engine's plan stays the exact one: later captures of the same shape apply the margin once, not again
+        self.D_cap, self.T_cap = eng.plan_capacities(db, margin)
         if to_host:
             self.host = HostResult(eng, db.B, db.N_max, db.A_max, self.T_cap, self.tiles)
             self.host_in = [torch.empty(t.shape, dtype=t.dtype, pin_memory=True) for t in
@@ -872,8 +886,17 @@ class GraphedProfile:
             self.res = eng._profile_tiled(db, self.D_cap, self.T_cap, self.tiles, host=self.host)
         self.launches_per_run = self._launches_warm
 
+    def check_shape(self, new) -> None:
+        """Raise ValueError unless `new` (a DeviceBatch or PackedPaths) has this graph's B, N_max and A_max.  There is no
+        max_splines check: more splines than captured are flagged on the device (ST_CAPACITY), also for inputs copied
+        straight into the static buffers."""
+        got, want = (new.B, new.N_max, new.A_max), (self.db.B, self.db.N_max, self.db.A_max)
+        if got != want:
+            raise ValueError(f"batch shape (B, N_max, A_max) = {got} differs from the captured {want}: capture a graph for it")
+
     def run(self, new_db: Optional[DeviceBatch] = None, check: bool = True) -> ProfileResult:
         if new_db is not None:
+            self.check_shape(new_db)
             for name in ("node_attr", "node_flags", "n_nodes", "ap_attr", "ap_flags", "n_ap", "cons"):
                 getattr(self.db, name).copy_(getattr(new_db, name), non_blocking=True)
         self.graph.replay()
@@ -887,6 +910,7 @@ class GraphedProfile:
         stream the dense rows into pinned host memory while other tiles still compute), wait, return the host view."""
         if self.host is None:
             raise ValueError("capture(..., to_host=True) first")
+        self.check_shape(packed)
         srcs = (packed.node_attr, packed.node_flags, packed.n_nodes, packed.ap_attr, packed.ap_flags, packed.n_ap, packed.cons)
         dsts = (self.db.node_attr, self.db.node_flags, self.db.n_nodes, self.db.ap_attr, self.db.ap_flags, self.db.n_ap,
                 self.db.cons)
@@ -910,8 +934,8 @@ class PipelinedProfiler:
     (the per-path time loop runs one warp per scheduler and uses ~6 % of the warp slots, the event replays a few threads)
     overlap the bandwidth-bound front of batch n+1 instead of leaving the GPU idle.  Every batch still runs every kernel.
 
-    submit(new_db, consume): enqueue one batch -- copy `new_db` (None: the slot keeps its inputs) into the slot's static
-    inputs, replay, then call consume(result) with the slot's stream current, so that whatever it enqueues (a copy of the
+    submit(new_db, consume): enqueue one batch -- copy `new_db` (None: the slot keeps its inputs; otherwise B, N_max and
+    A_max must be the constructor's) into the slot's static inputs (every slot starts with its own copy of `db`), replay, then call consume(result) with the slot's stream current, so that whatever it enqueues (a copy of the
     summary rows, an export kernel, a device->host copy ...) is ordered before the slot is reused.  drain() joins all
     streams back into the caller's stream.  Capacity overflows are reported in the status / summary rows as usual
     (ST_CAPACITY); the caller redoes those batches through Engine.profile.
@@ -923,13 +947,16 @@ class PipelinedProfiler:
         def clone(d: DeviceBatch) -> DeviceBatch:
             return DeviceBatch(d.node_attr.clone(), d.node_flags.clone(), d.n_nodes.clone(), d.ap_attr.clone(),
                                d.ap_flags.clone(), d.n_ap.clone(), d.cons.clone(), d.max_splines)
-        self.graphs = [eng.capture(db if k == 0 else clone(db), tiles=1, margin=margin) for k in range(self.depth)]
+        # every slot owns its static inputs: none aliases the caller's `db`, which submit(new_db) would overwrite
+        self.graphs = [eng.capture(clone(db), tiles=1, margin=margin) for _ in range(self.depth)]
         self.streams = [torch.cuda.Stream(device=eng.device) for _ in range(self.depth)]
         self.n = 0
 
     def submit(self, new_db: Optional[DeviceBatch] = None, consume=None) -> ProfileResult:
         k = self.n % self.depth
         g, st = self.graphs[k], self.streams[k]
+        if new_db is not None:
+            g.check_shape(new_db)
         st.wait_stream(torch.cuda.current_stream(self.eng.device))          # inputs prepared on the caller's stream
         with torch.cuda.stream(st):
             if new_db is not None:
