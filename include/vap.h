@@ -105,7 +105,7 @@ int vap_build_lut(int64_t B, int N_max, const double* seg, const int32_t* first_
 /* Optional accelerator of distance_to_time (spline_manager.py:291-318): an inverse index of the distance table, so that
  *     np.searchsorted(distances, d) is one seeded lookup plus a verification against the table instead of a 10-level
  *     binary search (identical result).  lut_inv[B][vap_lut_index_row_ints(Q_cap)] i32; pass it (or NULL) to
- *     vap_dist_sample_events / vap_time_profile.                                                        */
+ *     vap_velocity_profile / vap_time_profile.                                                          */
 int64_t vap_lut_index_row_ints(int64_t Q_cap);
 int vap_build_lut_index(int64_t B, const int32_t* n_splines, const int32_t* status, int samples, int64_t Q_cap,
                         const double* lut_d, const double* total_len, int32_t* lut_inv, void* stream);
@@ -145,47 +145,32 @@ int vap_fwd_bwd(int64_t B, int N_max, int A_max, const double* node_attr, const 
                 double* vel, int E_cap, double* max_accels, int32_t* bidx, int32_t* bval, int32_t* n_ev,
                 double* t_est, int mode, void* stream);
 
-/* v2 of S3 + S4 + S5 (same results, bit for bit, as vap_dist_sample + vap_fwd_bwd; this is the fast path).
- *   vap_dist_sample_events: distance sampling plus sample-parallel event detection and a per-path replay of the
- *     sampling loop's event logic (motion_profile_generator.py:93-176).  Adds the initial-velocity regimes
- *     vr_idx/vr_val[B][E_cap], the stop samples st_idx[B][E_cap] and n_vr[B][2].  t may be NULL (the parameters
- *     are not needed downstream).  ev_scratch: i32 scratch of
- *     vap_event_scratch_ints(B, N_max, A_max) elements.  ins_est[B] f32: rows the time stage will insert for
- *     waits / turn profiles (sizing only).
- *   vap_fwd_bwd_chunked: pre-pass that hoists everything of a step that depends neither on the velocity state nor on
- *     the events (per sample |kappa|, the velocity caps, the static acceleration limit; per step the wheel-acceleration
- *     denominator and its reciprocal), then the forward and backward passes (:188-314) with `chunks` (32, 64, 128 or 256)
- *     speculative chunks per path that are re-run until they merge bitwise with the serial evaluation.  The arrays the
- *     passes stream are chunk-interleaved in blocks of four steps (steps 4k .. 4k+3 of chunk c are one 32-byte sector;
- *     sector (k, c) follows sector (k, c-1)) so that every warp-wide access is one contiguous run and a chunk re-run
- *     alone fetches only bytes it uses: rec [B][RS][5] f64 (per block five field planes of 4 x `chunks` doubles),
- *     statB / vel_f [B][RS] f64 (the backward pass's static acceleration limit, touched only for paths with
+/* v2 of S3 + S4 + S5 in ONE call, the fast path that Engine.profile uses: same results, bit for bit, as vap_dist_sample
+ *     + vap_fwd_bwd.  Distance sampling (motion_profile_generator.py:84-176) with sample-parallel event detection and a
+ *     per-path replay of the sampling loop's event logic (:93-176), then the forward and backward passes (:188-314) with
+ *     `chunks` speculative chunks per path that are re-run until they merge bitwise with the serial evaluation.
+ *   The sampling fills a shared-memory tile from which a pre-pass hoists everything of a step that depends neither on
+ *     the velocity state nor on the events (per sample |kappa|, the velocity caps, the static acceleration limit; per
+ *     step the wheel-acceleration denominator and its reciprocal), so kappa / theta per distance sample never go to
+ *     memory: t / kap / th [B][D_cap] are inspection outputs (pass all three or three NULLs).  The static acceleration
+ *     limits of paths with max_acceleration overrides are rewritten after the event resolution.
+ *   n_samples[B] and status as in vap_dist_sample (status may also get VAP_ERR_EVENTS); max_accels[B][E_cap],
+ *     bidx/bval[B][E_cap] and n_ev[B][2] as in vap_fwd_bwd, E_cap >= N_max + A_max + 2.  vr_idx/vr_val[B][E_cap]:
+ *     the initial-velocity regimes, v0[i] = vr_val[j] for the last j with vr_idx[j] <= i; st_idx[B][E_cap]: the stop
+ *     samples (initial velocity 0.01); n_vr[B][2]: the number of regimes and of stop samples.  ev_scratch: i32 scratch
+ *     of vap_event_scratch_ints(B, N_max, A_max) elements.  ins_est[B] f32: rows the time stage will insert for waits /
+ *     turn profiles (sizing only).
+ *   The arrays the passes stream are chunk-interleaved in blocks of four steps (steps 4k .. 4k+3 of chunk c are one
+ *     32-byte sector; sector (k, c) follows sector (k, c-1)) so that every warp-wide access is one contiguous run and a
+ *     chunk re-run alone fetches only bytes it uses: rec [B][RS][5] f64 (per block five field planes of 4 x `chunks`
+ *     doubles), statB / vel_f [B][RS] f64 (the backward pass's static acceleration limit, touched only for paths with
  *     max_acceleration overrides; forward velocities; both slot order), RS = vap_pass_row_slots(D_cap, chunks).
- *     vel[B][D_cap] (D_cap even): final velocities in sample order, written by the backward pass itself (mode 1: the
- *     forward velocities in sample order); t_est[B] f32; rounds[B][2] fix-up sweeps.     */
-int vap_dist_sample_events(int64_t B, int N_max, int A_max, const double* node_attr, const int32_t* node_flags,
-                           const int32_t* n_nodes, const double* ap_attr, const int32_t* ap_flags, const int32_t* n_ap,
-                           const double* cons, const int32_t* n_splines, int32_t* status, int64_t n_grid,
-                           const double* dgrid, int samples, int64_t Q_cap, const double* lut_d, const double* lut_t,
-                           const double* total_len, int spn, int64_t P_cap, const double* prop_k, const double* prop_h,
-                           int64_t D_cap, int32_t* n_samples, double* t, double* kap, double* th, int E_cap,
-                           double* max_accels, int32_t* bidx, int32_t* bval, int32_t* n_ev, int32_t* vr_idx,
-                           double* vr_val, int32_t* st_idx, int32_t* n_vr, double dt, float* ins_est,
-                           int32_t* ev_scratch, const int32_t* lut_inv, void* stream);
+ *     chunks: a power of two from 8 to 256.
+ *   vel[B][D_cap] (D_cap even): final velocities in sample order, written by the backward pass itself (mode 1: the
+ *     forward velocities in sample order); t_est[B] f32: estimate of the number of time samples (for sizing S6);
+ *     rounds[B][2]: fix-up sweeps of the forward / backward pass.  mode: 0 both passes, 1 forward only (stage tests). */
 int64_t vap_event_scratch_ints(int64_t B, int N_max, int A_max);
 int64_t vap_pass_row_slots(int64_t D_cap, int chunks);
-int vap_fwd_bwd_chunked(int64_t B, const double* cons, const int32_t* status, double dd, double dt, double start_vel,
-                        double end_vel, int64_t D_cap, const int32_t* n_samples, const double* kap, const double* th,
-                        int E_cap, const double* max_accels, const int32_t* bidx, const int32_t* bval,
-                        const int32_t* n_ev, const int32_t* vr_idx, const double* vr_val, const int32_t* st_idx,
-                        const int32_t* n_vr, double* rec, double* statB, double* vel_f, double* vel, float* t_est,
-                        int32_t* rounds, int chunks, int mode, void* stream);
-
-/* S3 + S4 + S5 in ONE call (what Engine.profile uses): vap_dist_sample_events and vap_fwd_bwd_chunked fused.  The distance
- *     sampling (motion_profile_generator.py:84-176) fills the pre-pass's shared-memory tile directly, so kappa / theta per
- *     distance sample never go to memory: t / kap / th [B][D_cap] are inspection outputs (pass all three or three NULLs).
- *     The static acceleration limits of paths with max_acceleration overrides are rewritten after the event resolution
- *     (k_prepass_ovr).  All other arguments as in the two staged entry points above; same bits.                        */
 int vap_velocity_profile(int64_t B, int N_max, int A_max, const double* node_attr, const int32_t* node_flags,
                          const int32_t* n_nodes, const double* ap_attr, const int32_t* ap_flags, const int32_t* n_ap,
                          const double* cons, const int32_t* n_splines, int32_t* status, int64_t n_grid,

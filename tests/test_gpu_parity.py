@@ -244,24 +244,40 @@ def test_cfg2_full_size_properties(eng, ora):
 
 def test_chunked_equals_serial_bitwise():
     """The chunk-speculative velocity passes must reproduce the serial recurrences bit for bit, for every chunk count,
-    including ragged batches, node actions and a path long enough to need many fix-up sweeps."""
+    including ragged batches, node actions, max_acceleration overrides (the pre-pass's override fix-up) and a path long
+    enough to need many fix-up sweeps.  The sampling outputs (t / kappa / theta, max_accels, the boundary map) of the
+    fused sampling + pre-pass kernel must equal the serial ones bit for bit as well."""
     from vexautonomousplanner_b200 import synth
     from vexautonomousplanner_b200.engine import Engine
     ser = Engine("cuda:0", velocity_impl="serial", time_impl="serial")
-    batches = [synth.random_paths(512, 8, seed=5), synth.mixed_paths(512, 8, seed=6), golden_batch()[1],
+    overrides = synth.mixed_paths(320, 8, seed=9)
+    batches = [synth.random_paths(512, 8, seed=5), synth.mixed_paths(512, 8, seed=6), overrides, golden_batch()[1],
                synth.random_paths(3, 120, seed=8)]
     for packed in batches:
         db = ser.upload(packed)
         ref = ser.profile(db, keep=True)
+        D = ref.n_samples.long()
+        m = torch.arange(ref.vel.shape[1], device=D.device)[None, :] < D[:, None]
+        ne = ref.extra["n_ev"].long()
+        em = torch.arange(ref.extra["max_accels"].shape[1], device=D.device)[None, :]
+        m_acc, m_map = em < ne[:, 0:1], em < ne[:, 1:2]
+        if packed is overrides:
+            assert bool((ref.status == 0).all())
+            A0 = db.cons[:, 1:2]
+            assert bool((m_acc & (ref.extra["max_accels"] != A0)).any()), "the batch has no max_acceleration overrides"
         for chunks in (8, 16, 32, 64, 256):
             chk = Engine("cuda:0", velocity_impl="chunked", chunks=chunks, time_impl="split")
             got = chk.profile(db, keep=True)
             torch.cuda.synchronize()
             assert torch.equal(ref.n_samples, got.n_samples)
-            D = ref.n_samples.long()
-            m = torch.arange(ref.vel.shape[1], device=D.device)[None, :] < D[:, None]
+            for key in ("t", "kap", "th"):
+                assert torch.equal(ref.extra[key][m].view(torch.int64), got.extra[key][m].view(torch.int64)), (key, chunks)
             assert torch.equal(ref.vel[m].view(torch.int64), got.vel[m].view(torch.int64)), f"chunks={chunks}"
             assert torch.equal(ref.extra["n_ev"], got.extra["n_ev"])
+            ma_ref, ma_got = ref.extra["max_accels"][m_acc], got.extra["max_accels"][m_acc]
+            assert torch.equal(ma_ref.view(torch.int64), ma_got.view(torch.int64)), f"chunks={chunks}"
+            assert torch.equal(ref.extra["bidx"][m_map], got.extra["bidx"][m_map])
+            assert torch.equal(ref.extra["bval"][m_map], got.extra["bval"][m_map])
             assert torch.equal(ref.n_out, got.n_out)
             n = ref.n_out.long()
             Tm = min(ref.T_cap, got.T_cap)
@@ -1014,38 +1030,3 @@ def test_repeated_runs_are_bitwise_identical():
             assert torch.equal(got.out[i, :, :m][valid[:, :m]], ref.out[i, :, :m][valid[:, :m]]), (k, i)
         dm = min(got.vel.shape[1], ref.vel.shape[1])
         assert torch.equal(got.vel[:, :dm][dvalid[:, :dm]], ref.vel[:, :dm][dvalid[:, :dm]]), k
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("chunks", [8, 32, 64])
-def test_fused_velocity_stage_equals_staged_entry_points(chunks):
-    """vap_velocity_profile (sampling fused with the pre-pass, k_prepass_ovr after the event resolution) against the two
-    staged entry points it replaces (vap_dist_sample_events + vap_fwd_bwd_chunked, kappa / theta through memory): every
-    output of the velocity stage and the final trajectories bit for bit, on a mixed batch with overrides."""
-    from vexautonomousplanner_b200 import synth
-    from vexautonomousplanner_b200.engine import Engine
-    packed = synth.mixed_paths(320, 8, seed=9)
-    a = Engine("cuda:0", chunks=chunks, fused_velocity=True)
-    b = Engine("cuda:0", chunks=chunks, fused_velocity=False)
-    ra = a.profile(a.upload(packed), keep=True)
-    rb = b.profile(b.upload(packed), keep=True)
-    torch.cuda.synchronize()
-    assert torch.equal(ra.status, rb.status) and bool((ra.status == 0).all())
-    assert torch.equal(ra.n_samples, rb.n_samples) and torch.equal(ra.n_out, rb.n_out)
-    D = ra.n_samples.long()
-    dv = torch.arange(ra.vel.shape[1], device=D.device)[None, :] < D[:, None]
-    for key in ("t", "kap", "th"):
-        assert torch.equal(ra.extra[key][dv], rb.extra[key][dv]), key
-    assert torch.equal(ra.vel[dv], rb.vel[dv])
-    for key in ("n_ev", "n_vr"):
-        assert torch.equal(ra.extra[key], rb.extra[key]), key
-    ne = ra.extra["n_ev"].long()
-    em = torch.arange(ra.extra["max_accels"].shape[1], device=D.device)[None, :]
-    assert torch.equal(ra.extra["max_accels"][em < ne[:, 0:1]], rb.extra["max_accels"][em < ne[:, 0:1]])
-    assert torch.equal(ra.extra["bidx"][em < ne[:, 1:2]], rb.extra["bidx"][em < ne[:, 1:2]])
-    assert torch.equal(ra.extra["bval"][em < ne[:, 1:2]], rb.extra["bval"][em < ne[:, 1:2]])
-    T = ra.n_out.long()
-    tv = torch.arange(min(ra.T_cap, rb.T_cap), device=D.device)[None, :] < T[:, None]
-    m = tv.shape[1]
-    for i in range(8):
-        assert torch.equal(ra.out[i, :, :m][tv], rb.out[i, :, :m][tv]), i

@@ -22,8 +22,8 @@ NVCC_FLAGS = os.environ.get("VAP_NVCC_EXTRA", "").split() + ["-O3", "-std=c++17"
 SYMBOLS = [
     "vap_version", "vap_last_error", "vap_build_path", "vap_fit_splines", "vap_eval", "vap_build_lut",
     "vap_lut_index_row_ints", "vap_build_lut_index", "vap_build_props", "vap_query_tables", "vap_build_dgrid", "vap_dist_sample", "vap_fwd_bwd", "vap_resample",
-    "vap_gl", "vap_turn_profile", "vap_lerp", "vap_wheel_trajectory", "vap_dist_sample_events",
-    "vap_event_scratch_ints", "vap_pass_row_slots", "vap_fwd_bwd_chunked", "vap_velocity_profile", "vap_time_profile", "vap_workspace_bytes", "vap_profile_batch", "vap_summary", "vap_pack_rows", "vap_export_rows", "vap_format_doubles", "vap_row_text_stride",
+    "vap_gl", "vap_turn_profile", "vap_lerp", "vap_wheel_trajectory",
+    "vap_event_scratch_ints", "vap_pass_row_slots", "vap_velocity_profile", "vap_time_profile", "vap_workspace_bytes", "vap_profile_batch", "vap_summary", "vap_pack_rows", "vap_export_rows", "vap_format_doubles", "vap_row_text_stride",
     "vap_format_rows", "vap_compact_rows", "vap_row_kinds", "vap_bench_dfma", "vap_test_div_const", "vap_test_div_recip", "vap_build_lerp_recip", "vap_diag_read",
 ]
 

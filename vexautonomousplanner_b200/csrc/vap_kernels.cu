@@ -1208,89 +1208,58 @@ extern "C" int vap_wheel_trajectory(int64_t n, const double* lin, const double* 
 }
 
 // ---- v2 velocity path ------------------------------------------------------------------------------------------
-extern "C" int vap_dist_sample_events(int64_t B, int N_max, int A_max, const double* node_attr,
-                                      const int32_t* node_flags, const int32_t* n_nodes, const double* ap_attr,
-                                      const int32_t* ap_flags, const int32_t* n_ap, const double* cons,
-                                      const int32_t* n_splines, int32_t* status, int64_t n_grid, const double* dgrid,
-                                      int samples, int64_t Q_cap, const double* lut_d, const double* lut_t,
-                                      const double* total_len, int spn, int64_t P_cap, const double* prop_k,
-                                      const double* prop_h, int64_t D_cap, int32_t* n_samples, double* t, double* kap,
-                                      double* th, int E_cap, double* max_accels, int32_t* bidx, int32_t* bval,
-                                      int32_t* n_ev, int32_t* vr_idx, double* vr_val, int32_t* st_idx, int32_t* n_vr,
-                                      double dt, float* ins_est, int32_t* ev_scratch, const int32_t* lut_inv,
-                                      void* stream)
-{
-    if (B <= 0) return 0;
-    if (E_cap < N_max + A_max + 2) return arg_err("vap_dist_sample_events: E_cap < N_max + A_max + 2");
-    int Am = A_max > 0 ? A_max : 1;
-    // ev_scratch: wrap[B][N_max] | nwrap[B] | apc[B][Am][EV_AP_CAND] | napc[B][Am]
-    int32_t* ev_wrap = ev_scratch;
-    int32_t* ev_nwrap = ev_wrap + (size_t)B * N_max;
-    int32_t* ev_apc = ev_nwrap + B;
-    int32_t* ev_napc = ev_apc + (size_t)B * Am * EV_AP_CAND;
-    cudaError_t e = cudaMemsetAsync(ev_nwrap, 0, sizeof(int32_t) * (size_t)B, STREAM);
-    if (e != cudaSuccess) return set_err("vap_dist_sample_events/memset", e);
-    e = cudaMemsetAsync(ev_napc, 0, sizeof(int32_t) * (size_t)B * Am, STREAM);
-    if (e != cudaSuccess) return set_err("vap_dist_sample_events/memset", e);
-    k_count_samples<<<blocks_for(B, 128), 128, 0, STREAM>>>(B, status, status, n_grid, dgrid, total_len, D_cap, n_samples);
-    CHECK_LAUNCH("vap_dist_sample_events/count");
-    const unsigned tx = blocks_for(D_cap, 256);
-    if ((long long)tx * B > 2147483647LL) return arg_err("vap_dist_sample_events: more than 2^31 CTAs (tile the batch)");
-    const unsigned grid = tx * (unsigned)B;
-    k_dist_sample_ev<<<grid, 256, 0, STREAM>>>(N_max, Am, n_nodes, n_splines, status, ap_attr, n_ap, dgrid, samples, Q_cap,
-                                               lut_d, lut_t, total_len, spn, P_cap, prop_k, prop_h, D_cap, n_samples, t,
-                                               kap, th, ev_wrap, ev_nwrap, ev_apc, ev_napc, lut_inv, tx);
-    CHECK_LAUNCH("vap_dist_sample_events/sample");
-    k_resolve_events<<<blocks_for(B, 64), 64, 0, STREAM>>>(B, N_max, Am, node_attr, node_flags, n_nodes, ap_attr, ap_flags,
-                                                          n_ap, cons, status, ev_wrap, ev_nwrap, ev_apc, ev_napc, E_cap,
-                                                          max_accels, bidx, bval, n_ev, vr_idx, vr_val, st_idx, n_vr, dt, ins_est);
-    CHECK_LAUNCH("vap_dist_sample_events/resolve");
-    return 0;
-}
-
 extern "C" int64_t vap_event_scratch_ints(int64_t B, int N_max, int A_max)
 {
     int Am = A_max > 0 ? A_max : 1;
     return B * N_max + B + B * Am * EV_AP_CAND + B * Am;
 }
 
+// the event candidates of the sampling kernels in ev_scratch (vap_event_scratch_ints elements, Am = max(A_max, 1)):
+// wrap[B][N_max] | nwrap[B] | apc[B][Am][EV_AP_CAND] | napc[B][Am]; the two candidate counters start at zero
+struct EventScratch { int32_t *wrap, *nwrap, *apc, *napc; };
+static cudaError_t event_scratch(int32_t* ev_scratch, int64_t B, int N_max, int Am, cudaStream_t st, EventScratch& c)
+{
+    c.wrap = ev_scratch;
+    c.nwrap = c.wrap + (size_t)B * N_max;
+    c.apc = c.nwrap + B;
+    c.napc = c.apc + (size_t)B * Am * EV_AP_CAND;
+    cudaError_t e = cudaMemsetAsync(c.nwrap, 0, sizeof(int32_t) * (size_t)B, st);
+    if (e != cudaSuccess) return e;
+    return cudaMemsetAsync(c.napc, 0, sizeof(int32_t) * (size_t)B * Am, st);
+}
+
 // slots per path row of the chunk-interleaved pass arrays (records, override limits, forward velocities): the samples, one
 // block of four rows per chunk for rounding the chunk length up, one more for the passes' look-ahead loads, the tail slot
 extern "C" int64_t vap_pass_row_slots(int64_t D_cap, int chunks) { return ((D_cap + 8 * (int64_t)chunks + 64 + 1) / 2) * 2; }
 
-template <int NT, bool TMA>
-static int launch_passes_v(int64_t B, size_t ss, cudaStream_t st, const double* cons, const int32_t* status, double dd, double dt,
-                           double start_vel, double end_vel, long long RS, long long D_cap, const int32_t* n_samples,
-                           const double* rec, int E_cap, const double* max_accels, const int32_t* bidx, const int32_t* bval,
-                           const int32_t* n_ev, const int32_t* vr_idx, const double* vr_val, const int32_t* st_idx,
-                           const int32_t* n_vr, double* vel_f, double* vel, float* t_est, int32_t* rounds, bool backward,
-                           int warm, int max_rounds, const double* statB)
+template <int NT>
+static int launch_passes(int64_t B, size_t ss, cudaStream_t st, const double* cons, const int32_t* status, double dd, double dt,
+                         double start_vel, double end_vel, long long RS, long long D_cap, const int32_t* n_samples,
+                         const double* rec, int E_cap, const double* max_accels, const int32_t* bidx, const int32_t* bval,
+                         const int32_t* n_ev, const int32_t* vr_idx, const double* vr_val, const int32_t* st_idx,
+                         const int32_t* n_vr, double* vel_f, double* vel, float* t_est, int32_t* rounds, bool backward,
+                         int warm, int max_rounds, const double* statB)
 {
-    // TMA variant: behind the tables every warp has a two-stage ring of 5 (forward) / 6 (backward) planes of 1 KB + 2 mbarriers
+    // behind the tables every warp has a two-stage ring of 5 (forward) / 6 (backward) planes of 1 KB + 2 mbarriers
     const int warps = (NT + 31) / 32;
     const int ring_off = (int)((ss + 127) / 128 * 128);
     const int planes = backward ? 6 : 5;
-    const size_t smem = TMA ? (size_t)ring_off + (size_t)warps * (2 * planes * TMA_PLANE_DOUBLES * 8 + 16) : ss;
+    const size_t smem = (size_t)ring_off + (size_t)warps * (2 * planes * TMA_PLANE_DOUBLES * 8 + 16);
     cudaError_t e = cudaSuccess;
     if (!backward) {
-        if (smem > 48 * 1024) e = cudaFuncSetAttribute(k_fwd_chunked<NT, TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return set_err("vap_fwd_bwd_chunked/attr", e);
-        k_fwd_chunked<NT, TMA><<<(unsigned)B, NT, smem, st>>>(status, cons, dd, start_vel, end_vel, RS, n_samples, rec, E_cap,
-                                                             max_accels, bidx, bval, n_ev, vr_idx, vr_val, st_idx, n_vr, vel_f,
-                                                             rounds, warm, max_rounds, ring_off);
+        if (smem > 48 * 1024) e = cudaFuncSetAttribute(k_fwd_chunked<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_err("vap_velocity_profile/attr", e);
+        k_fwd_chunked<NT><<<(unsigned)B, NT, smem, st>>>(status, cons, dd, start_vel, end_vel, RS, n_samples, rec, E_cap,
+                                                           max_accels, bidx, bval, n_ev, vr_idx, vr_val, st_idx, n_vr, vel_f,
+                                                           rounds, warm, max_rounds, ring_off);
     } else {
-        if (smem > 48 * 1024) e = cudaFuncSetAttribute(k_bwd_chunked<NT, TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return set_err("vap_fwd_bwd_chunked/attr", e);
-        k_bwd_chunked<NT, TMA><<<(unsigned)B, NT, smem, st>>>(status, cons, dd, dt, end_vel, RS, D_cap, n_samples, rec, E_cap,
-                                                             max_accels, bidx, bval, n_ev, vel_f, vel, t_est, rounds, warm,
-                                                             max_rounds, statB, ring_off);
+        if (smem > 48 * 1024) e = cudaFuncSetAttribute(k_bwd_chunked<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_err("vap_velocity_profile/attr", e);
+        k_bwd_chunked<NT><<<(unsigned)B, NT, smem, st>>>(status, cons, dd, dt, end_vel, RS, D_cap, n_samples, rec, E_cap,
+                                                           max_accels, bidx, bval, n_ev, vel_f, vel, t_est, rounds, warm,
+                                                           max_rounds, statB, ring_off);
     }
     return 0;
-}
-template <int NT, typename... Args>
-static int launch_passes(bool tma, Args... args)
-{
-    return tma ? launch_passes_v<NT, true>(args...) : launch_passes_v<NT, false>(args...);
 }
 
 // forward and backward passes (+ the forward-only mode's slot order -> sample order) over records that are already in place
@@ -1313,12 +1282,9 @@ static int run_passes(int64_t B, const double* cons, const int32_t* status, doub
     if (const char* ev = getenv("VAP_CHUNK_MAXROUNDS")) max_rounds = atoi(ev);
 #endif
     if (warm < 0) warm = 0;
-    // first sweeps staged through shared memory by TMA bulk copies (default) or loaded by the lanes (VAP_PASS_TMA=0; same bits)
-    bool tma = true;
-    if (const char* ev = getenv("VAP_PASS_TMA")) tma = atoi(ev) != 0;
     auto passes = [&](bool backward) -> int {
         switch (chunks) {
-#define VAP_PASS_CASE(N_) case N_: return launch_passes<N_>(tma, B, ss, STREAM, cons, status, dd, dt, start_vel, end_vel, RS, D_cap,   \
+#define VAP_PASS_CASE(N_) case N_: return launch_passes<N_>(B, ss, STREAM, cons, status, dd, dt, start_vel, end_vel, RS, D_cap,    \
                                               n_samples, rec, E_cap, max_accels, bidx, bval, n_ev, vr_idx, vr_val, st_idx, n_vr,  \
                                               vel_f, vel, t_est, rounds, backward, warm, max_rounds, statB);
             VAP_PASS_CASE(8) VAP_PASS_CASE(16) VAP_PASS_CASE(32) VAP_PASS_CASE(64) VAP_PASS_CASE(128) VAP_PASS_CASE(256)
@@ -1327,16 +1293,16 @@ static int run_passes(int64_t B, const double* cons, const int32_t* status, doub
         return 0;
     };
     if (int rc = passes(false)) return rc;
-    CHECK_LAUNCH("vap_fwd_bwd_chunked/fwd");
+    CHECK_LAUNCH("vap_velocity_profile/fwd");
     if (mode == 1) {                 // forward velocities only: slot order -> sample order
         const unsigned tx2 = blocks_for(D_cap, 256);
-        if ((long long)tx2 * B > 2147483647LL) return arg_err("vap_fwd_bwd_chunked: more than 2^31 CTAs (tile the batch)");
+        if ((long long)tx2 * B > 2147483647LL) return arg_err("vap_velocity_profile: more than 2^31 CTAs (tile the batch)");
         k_untranspose<<<tx2 * (unsigned)B, 256, 0, STREAM>>>(status, n_samples, D_cap, RS, chunks, vel_f, vel, tx2);
-        CHECK_LAUNCH("vap_fwd_bwd_chunked/untranspose");
+        CHECK_LAUNCH("vap_velocity_profile/untranspose");
         return 0;
     }
     if (int rc = passes(true)) return rc;      // writes vel in sample order itself
-    CHECK_LAUNCH("vap_fwd_bwd_chunked/bwd");
+    CHECK_LAUNCH("vap_velocity_profile/bwd");
     return 0;
 }
 
@@ -1347,29 +1313,6 @@ static int check_pass_args(const char* who, int64_t B, int64_t D_cap, int chunks
     if (D_cap > 400000000LL) { snprintf(g_err, sizeof(g_err), "%s: D_cap too large", who); return -1; }
     if (D_cap & 1) { snprintf(g_err, sizeof(g_err), "%s: D_cap must be even (the passes move 16-byte pairs)", who); return -1; }
     return 0;
-}
-
-extern "C" int vap_fwd_bwd_chunked(int64_t B, const double* cons, const int32_t* status, double dd, double dt,
-                                   double start_vel, double end_vel, int64_t D_cap, const int32_t* n_samples,
-                                   const double* kap, const double* th, int E_cap, const double* max_accels,
-                                   const int32_t* bidx, const int32_t* bval, const int32_t* n_ev, const int32_t* vr_idx,
-                                   const double* vr_val, const int32_t* st_idx, const int32_t* n_vr, double* rec,
-                                   double* statB, double* vel_f, double* vel, float* t_est, int32_t* rounds,
-                                   int chunks, int mode, void* stream)
-{
-    if (B <= 0) return 0;
-    if (check_pass_args("vap_fwd_bwd_chunked", B, D_cap, chunks)) return -1;
-    const long long RS = vap_pass_row_slots(D_cap, chunks);
-    const unsigned tx = blocks_for(D_cap + 4 * chunks, 256 * PP_TILES);
-    if ((long long)tx * B > 2147483647LL) return arg_err("vap_fwd_bwd_chunked: more than 2^31 CTAs (tile the batch)");
-    const unsigned grid = tx * (unsigned)B;
-    // the kappa / theta tile: min(chunks, 64) columns x (256 / columns + 1) rows, odd stride; two buffers
-    const size_t sm = 2 * 2 * sizeof(double) * (size_t)prepass_tile_cols(chunks) * prepass_tile_stride(chunks);
-    k_prepass<<<grid, 256, sm, STREAM>>>(status, cons, D_cap, n_samples, kap, th, chunks, RS, rec, E_cap, max_accels, bidx,
-                                         bval, n_ev, statB, tx);
-    CHECK_LAUNCH("vap_fwd_bwd_chunked/prepass");
-    return run_passes(B, cons, status, dd, dt, start_vel, end_vel, D_cap, n_samples, E_cap, max_accels, bidx, bval, n_ev, vr_idx,
-                      vr_val, st_idx, n_vr, rec, statB, vel_f, vel, t_est, rounds, chunks, mode, STREAM);
 }
 
 // S3 + S4 + S5 in one call, the fast path: distance sampling fused with the pre-pass (kappa / theta stay on chip), event
@@ -1392,14 +1335,8 @@ extern "C" int vap_velocity_profile(int64_t B, int N_max, int A_max, const doubl
     if ((t != nullptr) != (kap != nullptr) || (t != nullptr) != (th != nullptr))
         return arg_err("vap_velocity_profile: t, kap and th are inspection outputs: pass all three or none");
     int Am = A_max > 0 ? A_max : 1;
-    int32_t* ev_wrap = ev_scratch;
-    int32_t* ev_nwrap = ev_wrap + (size_t)B * N_max;
-    int32_t* ev_apc = ev_nwrap + B;
-    int32_t* ev_napc = ev_apc + (size_t)B * Am * EV_AP_CAND;
-    cudaError_t e = cudaMemsetAsync(ev_nwrap, 0, sizeof(int32_t) * (size_t)B, STREAM);
-    if (e != cudaSuccess) return set_err("vap_velocity_profile/memset", e);
-    e = cudaMemsetAsync(ev_napc, 0, sizeof(int32_t) * (size_t)B * Am, STREAM);
-    if (e != cudaSuccess) return set_err("vap_velocity_profile/memset", e);
+    EventScratch cand;
+    if (cudaError_t e = event_scratch(ev_scratch, B, N_max, Am, STREAM, cand)) return set_err("vap_velocity_profile/memset", e);
     k_count_samples<<<blocks_for(B, 128), 128, 0, STREAM>>>(B, status, status, n_grid, dgrid, total_len, D_cap, n_samples);
     CHECK_LAUNCH("vap_velocity_profile/count");
     const long long RS = vap_pass_row_slots(D_cap, chunks);
@@ -1409,11 +1346,11 @@ extern "C" int vap_velocity_profile(int64_t B, int N_max, int A_max, const doubl
     const size_t sm = 2 * 3 * sizeof(double) * (size_t)tc * (((256 / tc) + 2) | 1);
     k_sample_prepass<<<tx * (unsigned)B, 256, sm, STREAM>>>(N_max, Am, n_nodes, n_splines, status, cons, ap_attr, n_ap, dgrid,
                                                            samples, Q_cap, lut_d, lut_t, total_len, spn, P_cap, prop_k, prop_h,
-                                                           D_cap, n_samples, t, kap, th, ev_wrap, ev_nwrap, ev_apc, ev_napc,
+                                                           D_cap, n_samples, t, kap, th, cand.wrap, cand.nwrap, cand.apc, cand.napc,
                                                            lut_inv, chunks, RS, rec, tx);
     CHECK_LAUNCH("vap_velocity_profile/sample_prepass");
     k_resolve_events<<<blocks_for(B, 64), 64, 0, STREAM>>>(B, N_max, Am, node_attr, node_flags, n_nodes, ap_attr, ap_flags,
-                                                          n_ap, cons, status, ev_wrap, ev_nwrap, ev_apc, ev_napc, E_cap,
+                                                          n_ap, cons, status, cand.wrap, cand.nwrap, cand.apc, cand.napc, E_cap,
                                                           max_accels, bidx, bval, n_ev, vr_idx, vr_val, st_idx, n_vr, dt, ins_est);
     CHECK_LAUNCH("vap_velocity_profile/resolve");
     k_prepass_ovr<<<(unsigned)B, 256, 0, STREAM>>>(status, cons, n_samples, chunks, RS, rec, E_cap, max_accels, bidx, bval, n_ev,
@@ -1442,18 +1379,12 @@ extern "C" int vap_time_profile(int64_t B, int N_max, int A_max, const double* n
     if (E_cap < N_max + A_max + 2) return arg_err("vap_time_profile: E_cap < N_max + A_max + 2");
     int Am = A_max > 0 ? A_max : 1;
     const int64_t M_cap = T_cap;
-    int32_t* ev_wrap = ev_scratch;
-    int32_t* ev_nwrap = ev_wrap + (size_t)B * N_max;
-    int32_t* ev_apc = ev_nwrap + B;
-    int32_t* ev_napc = ev_apc + (size_t)B * Am * EV_AP_CAND;
     int32_t* seg_k = seg_tab;
     int32_t* seg_off = seg_k + (size_t)B * E_cap;
     int32_t* seg_rev = seg_off + (size_t)B * E_cap;
     int32_t* n_seg = seg_rev + (size_t)B * E_cap;
-    cudaError_t e = cudaMemsetAsync(ev_nwrap, 0, sizeof(int32_t) * (size_t)B, STREAM);
-    if (e != cudaSuccess) return set_err("vap_time_profile/memset", e);
-    e = cudaMemsetAsync(ev_napc, 0, sizeof(int32_t) * (size_t)B * Am, STREAM);
-    if (e != cudaSuccess) return set_err("vap_time_profile/memset", e);
+    EventScratch cand;
+    if (cudaError_t e = event_scratch(ev_scratch, B, N_max, Am, STREAM, cand)) return set_err("vap_time_profile/memset", e);
     if (D_cap % 128 != 0) return arg_err("vap_time_profile: D_cap must be a multiple of 128 (rows are staged in 128-sample blocks)");
     // Serial per-path chains are latency-bound (about 4.6 cycles per dependent instruction, measured): spread the paths
     // over the warp schedulers (148 SMs x 4) with few paths per warp, so that one path's data-dependent branches stall
@@ -1486,12 +1417,12 @@ extern "C" int vap_time_profile(int64_t B, int N_max, int A_max, const double* n
     const unsigned grid = tx * (unsigned)B;
     k_time_sample<<<grid, 256, 0, STREAM>>>(B, N_max, Am, n_nodes, status, ap_attr, n_ap, seg, first_node, param_end,
                                             n_splines, samples, Q_cap, lut_d, lut_t, total_len, spn, P_cap, prop_k, prop_h,
-                                            M_cap, n_main, stage, ev_wrap, ev_nwrap, ev_apc, ev_napc, lut_inv, tx);
+                                            M_cap, n_main, stage, cand.wrap, cand.nwrap, cand.apc, cand.napc, lut_inv, tx);
     CHECK_LAUNCH("vap_time_profile/sample");
     k_time_events<<<blocks_for(B, lanes), lanes, 0, STREAM>>>(B, N_max, Am, node_attr, node_flags, n_nodes, ap_attr, n_ap, cons,
                                                        status, dt, seg, first_node, param_end, n_splines, spn, P_cap,
-                                                       prop_h, total_len, M_cap, n_main, stage, ev_wrap, ev_nwrap, ev_apc,
-                                                       ev_napc, E_cap, seg_k, seg_off, seg_rev, n_seg, T_cap, oplane,
+                                                       prop_h, total_len, M_cap, n_main, stage, cand.wrap, cand.nwrap, cand.apc,
+                                                       cand.napc, E_cap, seg_k, seg_off, seg_rev, n_seg, T_cap, oplane,
                                                        out, nodes_map, actions_map, n_maps, n_out, summary);
     CHECK_LAUNCH("vap_time_profile/events");
     k_time_finalize<<<grid, 256, 0, STREAM>>>(B, status, M_cap, n_main, stage, E_cap, seg_k, seg_off, seg_rev, n_seg,

@@ -21,63 +21,6 @@ __device__ __forceinline__ double4 ldg_d4(const double4* p)
     return make_double4(a.x, a.y, b.x, b.y);
 }
 
-// ---- S3 (parallel): t, kappa, theta per distance sample + event candidates -----------------------------------
-// wrap candidates: samples with frac(t[i-1]) > frac(t[i]) and t[i] < N-1  (motion_profile_generator.py:124)
-// action candidates: samples with t[i-1] < ap.t <= t[i]                   (:142-146)
-__global__ void __launch_bounds__(256, 8) k_dist_sample_ev(
-    int N_max, int A_max, const int* __restrict__ n_nodes, const int* __restrict__ n_splines,
-    const int* __restrict__ status, const double* __restrict__ ap_attr, const int* __restrict__ n_ap,
-    const double* __restrict__ dgrid, int samples, long long Q_cap, const double* __restrict__ lut_d,
-    const double* __restrict__ lut_t, const double* __restrict__ total_len, int spn, long long P_cap,
-    const double* __restrict__ prop_k, const double* __restrict__ prop_h, long long D_cap,
-    const int* __restrict__ n_samples, double* __restrict__ t_out, double* __restrict__ kap, double* __restrict__ th,
-    int* __restrict__ ev_wrap, int* __restrict__ ev_nwrap, int* __restrict__ ev_apc, int* __restrict__ ev_napc,
-    const int* __restrict__ lut_inv, unsigned tiles_x)
-{
-    __shared__ double s_t[257];
-    const PathTile pt = path_tile(tiles_x);
-    long long b = pt.b;
-    if (status[b] != ST_OK) return;
-    const int D = n_samples[b];
-    const int i0 = pt.x * blockDim.x;
-    if (i0 >= D) return;
-    const int i = i0 + threadIdx.x;
-    const int n = n_nodes[b];
-    const double* ld = lut_d + (size_t)b * Q_cap;
-    const double* lt = lut_t + (size_t)b * Q_cap;
-    const int Q = samples * n_splines[b];
-    const double L = total_len[b];
-    const PropGrid pg = prop_grid(spn, n);
-    const int* inv = lut_inv ? lut_inv + (size_t)b * (Q_cap + LUT_INV_HDR + 2) : nullptr;
-    auto d2t = [&](double d) { return inv ? distance_to_time_inv(ld, lt, inv, Q, L, n, d) : distance_to_time32(ld, lt, Q, L, n, d); };
-    double t = 0.0;
-    if (i < D) {
-        t = (i == D - 1) ? (double)(n - 1) : d2t(dgrid[i]);
-        double k, h;
-        snap_gather2_32(prop_k + (size_t)b * P_cap, prop_h + (size_t)b * P_cap, t, pg, k, h);
-        size_t o = (size_t)b * D_cap + i;
-        if (t_out) t_out[o] = t;           // the parameters themselves are only an inspection output
-        kap[o] = k; th[o] = h;
-    }
-    s_t[threadIdx.x + 1] = t;
-    if (threadIdx.x == 0) s_t[0] = (i0 > 0) ? d2t(dgrid[i0 - 1]) : 0.0;   // prev_t of sample 0 is 0
-    __syncthreads();
-    if (i >= D - 1) return;            // the final appended sample takes no part in the event logic
-    double tp = s_t[threadIdx.x];
-    if (frac1(tp) > frac1(t) && t < (double)(n - 1)) {
-        int slot = atomicAdd(ev_nwrap + b, 1);
-        if (slot < N_max) ev_wrap[(size_t)b * N_max + slot] = (int)i;
-    }
-    int A = n_ap ? n_ap[b] : 0;
-    for (int k = 0; k < A; k++) {
-        double x = ap_attr[((size_t)b * A_max + k) * APA + P_T];
-        if (tp < x && t >= x) {
-            int slot = atomicAdd(ev_napc + (size_t)b * A_max + k, 1);
-            if (slot < EV_AP_CAND) ev_apc[((size_t)b * A_max + k) * EV_AP_CAND + slot] = (int)i;
-        }
-    }
-}
-
 // ---- S3 (per path): replay the sampling loop's event logic over the candidate samples only --------------------
 // Outputs the reference's max_accels / boundary_map plus the piecewise-constant initial-velocity regimes:
 //   vr_idx/vr_val: v0[i] = vr_val[j] for the last j with vr_idx[j] <= i      (max_velocity before sample i's events)
@@ -315,133 +258,17 @@ __device__ __forceinline__ SampleTerms prepass_sample(double V, double acc_f, do
     return t;
 }
 
-// per-slot work of the pre-pass for a path WITH max_acceleration overrides: the forward regime of the sample is looked up and
-// the backward limit goes to its own array.  Out of line: the common (override-free) path keeps its 32 registers.
-__device__ __noinline__ void prepass_slot_ovr(long long b, int e, int j, int steps, int D, int NT, long long RS, int E_cap,
-                                             double V, double w, double max_angular_vel, double max_angular_accel,
-                                             double k_e, double k_last, double gh,
-                                             const double* __restrict__ max_accels, const int* __restrict__ bidx,
-                                             const int* __restrict__ bval, const int* __restrict__ n_ev,
-                                             double* __restrict__ pr, size_t o, double* __restrict__ statB)
-{
-    const int nb = n_ev[2 * b + 1];
-    const double dec_b = max_accels[(size_t)b * E_cap + bval[(size_t)b * E_cap + nb - 1]];       // backward max_dec
-    const double acc_f = max_accels[(size_t)b * E_cap + bval[(size_t)b * E_cap + last_le(bidx + (size_t)b * E_cap, nb, e)]];
-    const SampleTerms t = prepass_sample<true>(V, acc_f, dec_b, w, max_angular_vel, max_angular_accel, k_e);
-    const int PS = PB * NT;
-    pr[o] = t.ak; pr[o + PS] = t.G; pr[o + 2 * PS] = t.stat; pr[o + 3 * PS] = gh; pr[o + 4 * PS] = recip_for_pass(gh);
-    statB[(size_t)b * RS + j] = t.stat_b;
-    if (e == steps - 1) {
-        const SampleTerms u = prepass_sample<true>(V, dec_b, dec_b, w, max_angular_vel, max_angular_accel, k_last);
-        pr[5 * RS - 3] = u.ak; pr[5 * RS - 2] = u.G; pr[5 * RS - 1] = u.stat;
-        statB[(size_t)b * RS + RS - 1] = u.stat_b;
-    }
-}
-
-// One thread per SLOT (coalesced stores: 256 consecutive slots are whole 32-byte blocks of min(NT, 64) columns); kappa /
-// theta come through a shared-memory tile of TC = min(NT, 64) columns x TR = 256 / TC rows (+ one halo row for the heading
-// difference) whose loads run ALONG the columns (contiguous samples).
-#define PP_TILES 4          // 256-slot tiles per pre-pass CTA: the per-path preamble (status, sizes, override test, constants) is paid once
-__host__ __device__ __forceinline__ int prepass_tile_cols(int NT) { return NT < 64 ? NT : 64; }
-__host__ __device__ __forceinline__ int prepass_tile_stride(int NT) { return ((256 / prepass_tile_cols(NT)) + 1) | 1; }   // odd
-__global__ void __launch_bounds__(256, 8) k_prepass(
-    const int* __restrict__ status, const double* __restrict__ cons, long long D_cap, const int* __restrict__ n_samples,
-    const double* __restrict__ kap, const double* __restrict__ th, int NT, long long RS, double* __restrict__ rec,
-    int E_cap, const double* __restrict__ max_accels, const int* __restrict__ bidx, const int* __restrict__ bval,
-    const int* __restrict__ n_ev, double* __restrict__ statB, unsigned tiles_x)
-{
-    extern __shared__ double s_tile[];               // two tile buffers: one barrier per tile
-    const PathTile pt = path_tile(tiles_x);
-    const long long b = pt.b;
-    if (status[b] != ST_OK) return;
-    const int D = n_samples[b];
-    // does some node / action point override max_acceleration?  One regime per thread, loaded here and compared at the
-    // barrier, so that the latency overlaps the tile's (paths with more than blockDim.x regimes: a loop for the rest)
-    const bool o_in = (int)threadIdx.x < E_cap;
-    const int o_n = n_ev[2 * b];
-    const double o_ma = o_in ? max_accels[(size_t)b * E_cap + threadIdx.x] : 0.0;
-    const double o_A0 = cons[b * 6 + 1];
-    const int steps = D - 1;
-    const int sh = 31 - __clz(NT);                   // NT is a power of two: every index split below is a shift
-    const int Lc = chunk_len(steps, NT);
-    const int jend = Lc << sh;
-    int j0 = pt.x * (blockDim.x * PP_TILES);
-    if (steps <= 0 || j0 >= jend) return;
-    const double* kr = kap + (size_t)b * D_cap;
-    const double* tr = th + (size_t)b * D_cap;
-    const int tcsh = sh < 6 ? sh : 6;                // blockDim.x == 256: TC = min(NT, 64) columns x TR = 256 / TC rows per tile
-    const int TC = 1 << tcsh;
-    const int trsh = 8 - tcsh;
-    const int TR = 1 << trsh;
-    const int st = (TR + 1) | 1;                     // odd tile stride
-    __shared__ double s_c[2];                        // per-path constants: one thread divides, not all 256
-    if (threadIdx.x == 0) {
-        const double V_ = cons[b * 6 + 0], A0_ = cons[b * 6 + 1], w_ = cons[b * 6 + 5];
-        s_c[0] = 2 * V_ / w_;                        // max_angular_vel   (:81)
-        s_c[1] = 2 * A0_ / w_;                       // max_angular_accel (:82)
-    }
-    int p_ovr = o_in & ((int)threadIdx.x < o_n) & (o_ma != o_A0);
-    for (int q = threadIdx.x + blockDim.x; q < o_n; q += blockDim.x) p_ovr |= (max_accels[(size_t)b * E_cap + q] != o_A0);
-    const double V = cons[b * 6 + 0], A0 = cons[b * 6 + 1], w = cons[b * 6 + 5];
-    double* pr = rec + (size_t)b * RS * 5;
-    const int PS = PB * NT;                          // plane stride inside a block
-    int ovr = 0;
-    for (int it = 0; it < PP_TILES && j0 < jend; ++it, j0 += blockDim.x) {
-        double* t_th = s_tile + (it & 1) * (2 * TC * st);
-        double* t_k = t_th + TC * st;
-        const int c0 = (j0 >> 2) & (NT - 1);         // first column of the tile (0 unless NT > 64)
-        const int s0 = (j0 >> (sh + 2)) << 2;        // first row of the tile
-        {
-            const int cc = threadIdx.x >> trsh, r = threadIdx.x & (TR - 1);
-            int ee = (c0 + cc) * Lc + s0 + r;
-            ee = ee > D - 1 ? D - 1 : ee;
-            t_th[cc * st + r] = tr[ee];
-            t_k[cc * st + r] = kr[ee];
-            if ((int)threadIdx.x < TC) {             // the halo row
-                int eh = (c0 + threadIdx.x) * Lc + s0 + TR;
-                eh = eh > D - 1 ? D - 1 : eh;
-                t_th[threadIdx.x * st + TR] = tr[eh];
-            }
-        }
-        // the barrier of the first tile also carries the override vote and publishes s_c; the other buffer is free again
-        // one barrier later, when every thread has left the tile before
-        if (it == 0) ovr = __syncthreads_or(p_ovr); else __syncthreads();
-        const int j = j0 + threadIdx.x;
-        const int c = (j >> 2) & (NT - 1);
-        const int s = ((j >> (sh + 2)) << 2) + (j & 3);
-        const int e = c * Lc + s;              // this slot's edge = the sample whose terms this thread evaluates
-        if (s >= Lc || e >= steps) continue;
-        const double max_angular_vel = s_c[0];
-        const double max_angular_accel = s_c[1];
-        const int tl = (c - c0) * st + (s - s0);
-        const double gh = 2 * fabs(t_th[tl + 1] - t_th[tl]);
-        // without overrides both passes use the path's A0 (the common case, kept free of any table code); with them the
-        // forward regime of this sample is looked up and the backward limit goes to its own slot-order array
-        const size_t o = (size_t)(j >> (sh + 2)) * (5 * PS) + (size_t)(j & (PS - 1));
-        if (ovr) {                                  // uniform over the CTA; rare
-            prepass_slot_ovr(b, e, j, steps, D, NT, RS, E_cap, V, w, max_angular_vel, max_angular_accel, t_k[tl], kr[D - 1],
-                             gh, max_accels, bidx, bval, n_ev, pr, o, statB);
-            continue;
-        }
-        const SampleTerms t = prepass_sample<false>(V, A0, A0, w, max_angular_vel, max_angular_accel, t_k[tl]);
-        pr[o] = t.ak; pr[o + PS] = t.G; pr[o + 2 * PS] = t.stat; pr[o + 3 * PS] = gh; pr[o + 4 * PS] = recip_for_pass(gh);
-        if (e == steps - 1) {                       // the final sample (no edge starts there): the backward pass starts on it
-            const SampleTerms u = prepass_sample<false>(V, A0, A0, w, max_angular_vel, max_angular_accel, kr[D - 1]);
-            pr[5 * RS - 3] = u.ak; pr[5 * RS - 2] = u.G; pr[5 * RS - 1] = u.stat;
-        }
-    }
-}
-
-// ---- S3 + pre-pass fused: distance sampling, event candidates and the pass records in ONE kernel -------------------------
-// k_dist_sample_ev wrote kappa / theta per distance sample (16 bytes) only for k_prepass to read them back through a
-// shared-memory tile; here the tile is FILLED by the sampling itself (distance_to_time + snap gathers, one sample per thread,
-// lanes running along a chunk's consecutive samples) and the records are made from it in slot order, so kappa / theta never
-// go to HBM (t / kappa / theta are written only when the caller asks for them: inspection outputs).  A CTA walks PP_TILES
-// tiles DOWN the rows of its columns; a tile computes rows s0+1 .. s0+TR and takes rows s0-1 (parameter only: the event test
-// needs t of the previous sample) and s0 from the tile before (the first tile computes them itself), so the halo costs
-// 2 TC extra samples per CTA instead of per tile.
+// ---- S3 + pre-pass: distance sampling, event candidates and the pass records in ONE kernel -------------------------------
+// The sampling (distance_to_time + snap gathers, one sample per thread, lanes running along a chunk's consecutive samples)
+// fills a shared-memory tile of t / theta / kappa of TC = min(NT, 64) columns x TR = 256 / TC rows, and the records are made
+// from that tile one thread per slot (coalesced stores: 256 consecutive slots are whole 32-byte blocks of TC columns), so
+// kappa / theta never go to HBM (t / kappa / theta are written only when the caller asks for them: inspection outputs).
+// A CTA walks SP_TILES tiles DOWN the rows of its columns; a tile computes rows s0+1 .. s0+TR and takes rows s0-1 (parameter
+// only: the event test needs t of the previous sample) and s0 from the tile before (the first tile computes them itself), so
+// the halo costs 2 TC extra samples per CTA instead of per tile.
 // The records written here use the path's own max_acc: the regimes are not known yet (k_resolve_events runs on the event
 // candidates this kernel emits).  k_prepass_ovr rewrites the static limits of the paths that turn out to have overrides.
+__host__ __device__ __forceinline__ int prepass_tile_cols(int NT) { return NT < 64 ? NT : 64; }
 #ifndef VAP_SP_MINB
 #define VAP_SP_MINB 8
 #endif
@@ -734,17 +561,14 @@ __device__ __forceinline__ double bwd_step(double ak, double gh, double rg, doub
 // soon as two consecutive velocities equal the stored ones bitwise (from there the old values ARE the serial values).
 // Rounds end when no chunk had to re-run; then, by induction from chunk 0, every value is the serial value.
 //
-// The kernels are bound by the latency of the dependent fp64 chain of one step, so they are written for residency
-// (72 registers: 28 one-warp CTAs per SM, 4144 >= 4096 paths in one wave) and a short chain: event tables in shared
-// memory, 32-bit indices, records fetched one step ahead into two named buffers (no register rotation), the division's
-// reciprocal from the pre-pass, coalesced slot-order streams.
+// The kernels are bound by the latency of the dependent fp64 chain of one step, so they are written for a short chain:
+// event tables in shared memory, 32-bit indices, the division's reciprocal from the pre-pass, coalesced slot-order streams.
+// The lockstep first sweep takes its records from a per-warp shared-memory ring that TMA bulk copies fill a whole block
+// ahead; the fix-up re-runs and the warm-up are out of line and load their records one pair ahead themselves.
 // ------------------------------------------------------------------------------------------------------------------
 #define CH_INT_MAX 2147483647
-#ifndef VAP_PASS_REGS
-#define VAP_PASS_REGS 72     // one-warp CTAs: 28 per SM, 4144 >= 4096 paths in one wave
-#endif
 #ifndef VAP_PASS_REGS_TMA
-#define VAP_PASS_REGS_TMA 112 // the TMA variant is limited by its shared-memory rings (10 - 12 KB per warp), not by registers; 112 keeps the
+#define VAP_PASS_REGS_TMA 112 // residency is limited by the shared-memory rings (10 - 12 KB per warp), not by registers; 112 keeps the
                               // out-of-line re-run functions free of spills (96: 3.69 ms per cfg2 step, 112: 3.47, 128: 3.56)
 #endif
 
@@ -776,7 +600,6 @@ struct FwdTables {
 // the path's last chunk writes it (to the tail slot).  Records come as 16-byte pairs, two steps per pair, the next pair
 // fetched while the current one is being used (two named buffers, no register rotation).  NT is a compile-time constant:
 // every access is pointer + immediate.  old_end: what this lane's previous run produced for sample lo+len (RUN_RERUN).
-#define RUN_SWEEP 0     // first sweep: plain stores
 #define RUN_RERUN 1     // fix-up: bitwise merge detection against the stored velocities
 #define RUN_DRY 2       // warm-up before a speculative chunk: state only, no stores
 template <int NT, int MODE>
@@ -787,7 +610,6 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
     constexpr int PS = PB * NT, BS = 5 * PS;
     constexpr bool RERUN = (MODE == RUN_RERUN);
     constexpr bool DRY = (MODE == RUN_DRY);
-    constexpr bool SWEEP = (MODE == RUN_SWEEP);
     int j = 0;
     while (j + 1 < T.n_b && T.bi[j + 1] <= lo) j++;
     double acc = T.acc[j];
@@ -841,7 +663,6 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
         if (RERUN) oA = *reinterpret_cast<const double2*>(q + PS);
         FWD_ONE(akB.x, GB.x, stB.x, ghB.x, rgB.x, oB.y)
         if (RERUN) st_d2(q + 2, v2, v);
-        if (SWEEP) { st_d2(q, vin, v1); st_d2(q + 2, v2, v); }   // the whole 32-byte sector at once
         FWD_ONE(akB.y, GB.y, stB.y, ghB.y, rgB.y, ((e + 1 < hi) ? oA.x : old_end))
         q += PS;
     }
@@ -1011,8 +832,8 @@ __device__ __noinline__ void fwd_dry(const double* p, int lo, int len, FwdTables
 
 // Forward pass.  Chunk c = thread c.  vfT: forward velocities in slot order (vfT[slot(e)] = velocity at sample e), the
 // velocity of the last sample in slot RS-1.
-template <int NT, bool TMA>
-__global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_fwd_chunked(
+template <int NT>
+__global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_fwd_chunked(
     const int* __restrict__ status, const double* __restrict__ cons, double dd, double start_vel, double end_vel,
     long long RS, const int* __restrict__ n_samples, const double* __restrict__ rec, int E_cap,
     const double* __restrict__ max_accels, const int* __restrict__ bidx, const int* __restrict__ bval,
@@ -1076,23 +897,21 @@ __global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_fwd_chunk
     const double* P = rec + (size_t)b * RS * 5;
     double* tail = (active && lo + len == steps) ? vf + (RS - 1) : nullptr;  // only the last chunk stores the final sample
     const double hw = cons[b * 6 + 5] * 0.5;
-    // TMA variant: every warp owns a two-stage ring (5 planes of 1 KB per stage) and two mbarriers behind the tables
+    // every warp owns a two-stage ring (5 planes of 1 KB per stage) and two mbarriers behind the tables
     WarpRing R;
-    if (TMA) {
-        constexpr int WARPS = (NT + 31) / 32;
-        const int w = c >> 5;
-        R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 5 * TMA_PLANE_DOUBLES;
-        R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8 + 16 * w);
-        R.planes = 5;
-        R.bytes = (NT < 32 ? NT : 32) * PB * 8;
+    constexpr int WARPS = (NT + 31) / 32;
+    const int w = c >> 5;
+    R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 5 * TMA_PLANE_DOUBLES;
+    R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8 + 16 * w);
+    R.planes = 5;
+    R.bytes = (NT < 32 ? NT : 32) * PB * 8;
 #ifdef VAP_BOUNDS_CHECK
-        R.rec_lo = P; R.rec_hi = P + 5 * RS; R.x_lo = R.x_hi = nullptr;
-        R.smem_lo = (unsigned)__cvta_generic_to_shared(s_mem + ring_off);
-        R.smem_hi = R.smem_lo + WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8;
-        R.bar_hi = R.smem_hi + 16 * WARPS;
+    R.rec_lo = P; R.rec_hi = P + 5 * RS; R.x_lo = R.x_hi = nullptr;
+    R.smem_lo = (unsigned)__cvta_generic_to_shared(s_mem + ring_off);
+    R.smem_hi = R.smem_lo + WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8;
+    R.bar_hi = R.smem_hi + 16 * WARPS;
 #endif
-        if ((c & 31) == 0) { mbar_init(R.bar, 1); mbar_init(R.bar + 8, 1); fence_mbar_init(); }
-    }
+    if ((c & 31) == 0) { mbar_init(R.bar, 1); mbar_init(R.bar + 8, 1); fence_mbar_init(); }
     __syncthreads();
     FwdTables T;
     T.bi = s_bi; T.acc = s_acc; T.n_b = n_b; T.vi = s_vi; T.vv = s_vv; T.n_v = s_nv;
@@ -1126,9 +945,8 @@ __global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_fwd_chunk
             // extent of what this lane's runs touch (look-ahead block included): record rows and forward-velocity row
             VAP_CHECK(4, c * PB + PB <= PB * NT && (size_t)(((len + 3) >> 2) + 1) * 5 * PB * NT <= (size_t)(5 * RS - 3) &&
                              (size_t)(((len + 3) >> 2) + 1) * PB * NT <= (size_t)(RS - 1) && lo + len <= steps);
-            if (!TMA) fwd_run<NT, RUN_SWEEP>(P + c * PB, vf + c * PB, tail, 0.0, lo, len, T, hw, dd, v, sq, false);
         }
-        if (TMA) fwd_sweep_tma<NT>(R, P + (c & ~31) * PB, c & 31, vf + c * PB, tail, lo, active ? len : 0, T, hw, dd, v, sq);
+        fwd_sweep_tma<NT>(R, P + (c & ~31) * PB, c & 31, vf + c * PB, tail, lo, active ? len : 0, T, hw, dd, v, sq);
         s_endv[c] = v; s_endw[c] = sq;
     }
     __syncthreads();
@@ -1174,7 +992,6 @@ __device__ __forceinline__ bool bwd_run(const double* __restrict__ p, const doub
     constexpr int PS = PB * NT, BS = 5 * PS;
     constexpr bool RERUN = (MODE == RUN_RERUN);
     constexpr bool DRY = (MODE == RUN_DRY);
-    constexpr bool SWEEP = (MODE == RUN_SWEEP);
     // regime at the chunk start (walking down from D-1): the smallest boundary index > i was the last one applied
     int e = lo + len - 1;                            // current edge; the reference's loop index is i = e + 1
     int j = n_b - 1;
@@ -1258,7 +1075,6 @@ __device__ __forceinline__ bool bwd_run(const double* __restrict__ p, const doub
         const double v1 = v;
         BWD_ONE(akA.y, GA.y, stA.y, ghA.x, rgA.x, fA.x, oA.x, oA.y)
         if (RERUN) st_d2(o, v, v1);
-        if (SWEEP) { st_d2(o, v, v1); st_d2(o + 2, v2, v3); }        // the whole 32-byte sector at once
         if (!more) break;
         oup = oA.x;
         tak = akA.x; tG = GA.x; tst = stA.x;
@@ -1359,8 +1175,8 @@ __device__ __noinline__ void bwd_dry(const BwdArgs a, double* st)
 // Backward pass.  Thread k walks column nch-1-k (the k-th chunk counted from the end), so states flow from thread k-1 to
 // thread k as in the forward kernel.  Reads the forward velocities (slot order) and writes the final ones straight into
 // vel[B][D_cap] in sample order.  Also accumulates the travel-time estimate used to size the time-domain outputs.
-template <int NT, bool TMA>
-__global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_bwd_chunked(
+template <int NT>
+__global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_bwd_chunked(
     const int* __restrict__ status, const double* __restrict__ cons, double dd, double dt, double end_vel,
     long long RS, long long D_cap, const int* __restrict__ n_samples, const double* __restrict__ rec, int E_cap,
     const double* __restrict__ max_accels, const int* __restrict__ bidx, const int* __restrict__ bval,
@@ -1401,23 +1217,21 @@ __global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_bwd_chunk
     // with max_acceleration overrides the static limit of this pass is in statB (slot order, written by the pre-pass)
     const bool ovr = pass_has_override(max_accels + (size_t)b * E_cap, n_ev[2 * b], cons[b * 6 + 1]) != 0;
     const double* SB = statB + (size_t)b * RS;
-    // TMA variant: every warp owns a two-stage ring (6 planes of 1 KB per stage) and two mbarriers behind the tables
+    // every warp owns a two-stage ring (6 planes of 1 KB per stage) and two mbarriers behind the tables
     WarpRing R;
-    if (TMA) {
-        constexpr int WARPS = (NT + 31) / 32;
-        const int w = k >> 5;
-        R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 6 * TMA_PLANE_DOUBLES;
-        R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 6 * TMA_PLANE_DOUBLES * 8 + 16 * w);
-        R.planes = 6;
-        R.bytes = (NT < 32 ? NT : 32) * PB * 8;
+    constexpr int WARPS = (NT + 31) / 32;
+    const int w = k >> 5;
+    R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 6 * TMA_PLANE_DOUBLES;
+    R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 6 * TMA_PLANE_DOUBLES * 8 + 16 * w);
+    R.planes = 6;
+    R.bytes = (NT < 32 ? NT : 32) * PB * 8;
 #ifdef VAP_BOUNDS_CHECK
-        R.rec_lo = P; R.rec_hi = P + 5 * RS; R.x_lo = vf; R.x_hi = vf + RS;
-        R.smem_lo = (unsigned)__cvta_generic_to_shared(s_mem + ring_off);
-        R.smem_hi = R.smem_lo + WARPS * 2 * 6 * TMA_PLANE_DOUBLES * 8;
-        R.bar_hi = R.smem_hi + 16 * WARPS;
+    R.rec_lo = P; R.rec_hi = P + 5 * RS; R.x_lo = vf; R.x_hi = vf + RS;
+    R.smem_lo = (unsigned)__cvta_generic_to_shared(s_mem + ring_off);
+    R.smem_hi = R.smem_lo + WARPS * 2 * 6 * TMA_PLANE_DOUBLES * 8;
+    R.bar_hi = R.smem_hi + 16 * WARPS;
 #endif
-        if ((k & 31) == 0) { mbar_init(R.bar, 1); mbar_init(R.bar + 8, 1); fence_mbar_init(); }
-    }
+    if ((k & 31) == 0) { mbar_init(R.bar, 1); mbar_init(R.bar + 8, 1); fence_mbar_init(); }
     __syncthreads();
 
     auto rec_of = [&](int x, int fld) {                             // field fld (0-2) of sample x
@@ -1468,20 +1282,12 @@ __global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_bwd_chunk
             VAP_CHECK(5, col >= 0 && col * PB + PB <= PB * NT && (size_t)(((len + 3) >> 2) + 1) * 5 * PB * NT <= (size_t)(5 * RS - 3) &&
                              (size_t)(((len + 3) >> 2) + 1) * PB * NT <= (size_t)(RS - 1) && A.o + len <= vo + D - 1 &&
                              lo + len <= steps && D <= D_cap);
-            if (!TMA) {
-                if (ovr) bwd_run<NT, RUN_SWEEP, true>(A.p, A.f, A.o, A.sb, lo, len, top_ak, top_G, top_st, s_bi, s_acc, n_b, acc0, hw,
-                                                      dd, v, sq, false, est, A.dd_over_dt);
-                else bwd_run<NT, RUN_SWEEP, false>(A.p, A.f, A.o, A.sb, lo, len, top_ak, top_G, top_st, s_bi, s_acc, n_b, acc0, hw,
-                                                   dd, v, sq, false, est, A.dd_over_dt);
-            }
         }
-        if (TMA) {
-            // the warp's columns: lane 0 has the highest (nch-1-32w); the ring holds the 32 columns that end there
-            const int col_hi = nch - 1 - (k & ~31);
-            const int cs = col_hi > 31 ? col_hi - 31 : 0;
-            bwd_sweep_tma<NT>(R, P + cs * PB, vf + cs * PB, ovr ? SB + cs * PB : nullptr, active ? col - cs : 0, vo + lo, lo,
-                              active ? len : 0, top_ak, top_G, top_st, s_bi, s_acc, n_b, acc0, hw, dd, v, sq, est, A.dd_over_dt);
-        }
+        // the warp's columns: lane 0 has the highest (nch-1-32w); the ring holds the 32 columns that end there
+        const int col_hi = nch - 1 - (k & ~31);
+        const int cs = col_hi > 31 ? col_hi - 31 : 0;
+        bwd_sweep_tma<NT>(R, P + cs * PB, vf + cs * PB, ovr ? SB + cs * PB : nullptr, active ? col - cs : 0, vo + lo, lo,
+                          active ? len : 0, top_ak, top_G, top_st, s_bi, s_acc, n_b, acc0, hw, dd, v, sq, est, A.dd_over_dt);
         s_endv[k] = v; s_endw[k] = sq;
     }
     __syncthreads();
@@ -1520,7 +1326,7 @@ __global__ void __maxnreg__(TMA ? VAP_PASS_REGS_TMA : VAP_PASS_REGS) k_bwd_chunk
     }
 }
 
-// slot order -> sample order (only the forward-only mode of vap_fwd_bwd_chunked needs it: the backward pass writes sample
+// slot order -> sample order (only the forward-only mode of vap_velocity_profile needs it: the backward pass writes sample
 // order itself): vel[e] = vT[slot(e)], the last sample from slot RS-1.  One thread per sample.
 __global__ void __launch_bounds__(256) k_untranspose(const int* __restrict__ status, const int* __restrict__ n_samples,
                                                      long long D_cap, long long RS, int NT,

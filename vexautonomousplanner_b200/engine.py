@@ -129,8 +129,7 @@ class Engine:
 
     def __init__(self, device="cuda:0", dt: float = 0.01, dd: float = 0.005, lut_samples: int = 1000,
                  samples_per_node: int = 1000, start_vel: float = 0.01, end_vel: float = 0.01,
-                 velocity_impl: str = "chunked", chunks: int = 32, time_impl: str = "split", accelerators: bool = True,
-                 fused_velocity: bool = True):
+                 velocity_impl: str = "chunked", chunks: int = 32, time_impl: str = "split", accelerators: bool = True):
         if not torch.cuda.is_available():
             raise _lib.VapError("no CUDA device: vexautonomousplanner_b200 has no CPU fallback")
         self.lib = _lib.lib()
@@ -147,9 +146,6 @@ class Engine:
         # accelerators=False passes NULL for the inverse LUT index and the lerp reciprocals (binary search / plain division
         # instead: same bits, slower); tests use it to pin the equivalence
         self.accelerators = bool(accelerators)
-        # fused_velocity=False runs S3 and S4+S5 through the two staged entry points (vap_dist_sample_events +
-        # vap_fwd_bwd_chunked: kappa / theta go through memory) instead of vap_velocity_profile: same bits, tests pin it
-        self.fused_velocity = bool(fused_velocity)
         self._dgrid: Optional[torch.Tensor] = None
         self._rden: Optional[torch.Tensor] = None
         self._retired: list = []                # outgrown path-independent tables, kept alive for captured graphs
@@ -314,19 +310,16 @@ class Engine:
         return vel, ma, bidx, bval, n_ev, t_est
 
     def velocity_chunked(self, db: DeviceBatch, g: Geometry, t: Tables, status: torch.Tensor, D_cap: int, mode: int = 0,
-                         outs: Optional[dict] = None, want_t: bool = True, fused: Optional[bool] = None):
+                         outs: Optional[dict] = None, want_t: bool = True):
         """S3 + events + S4 + S5, fast path: sampling fused with the hoisted pre-pass (vap_velocity_profile), sample-parallel
-        events, chunk-speculative passes.  want_t: also write t / kappa / theta per distance sample (inspection outputs).
-        fused=False runs the two staged entry points instead (vap_dist_sample_events + vap_fwd_bwd_chunked: same bits)."""
+        events, chunk-speculative passes.  want_t: also write t / kappa / theta per distance sample (inspection outputs)."""
         B = db.B
-        fused = self.fused_velocity if fused is None else fused
         E_cap = db.N_max + db.A_max + 2
         grid = self.dgrid(D_cap + 2)
         n_samples = outs["n_samples"] if outs else self._empty((B,), torch.int32)
-        need_kth = want_t or not fused
-        tq = self._empty((B, D_cap)) if need_kth else None      # t / kappa / theta per distance sample: inspection outputs
-        kap = self._empty((B, D_cap)) if need_kth else None
-        th = self._empty((B, D_cap)) if need_kth else None
+        tq = self._empty((B, D_cap)) if want_t else None      # t / kappa / theta per distance sample: inspection outputs
+        kap = self._empty((B, D_cap)) if want_t else None
+        th = self._empty((B, D_cap)) if want_t else None
         ma = self._empty((B, E_cap)); bidx = self._empty((B, E_cap), torch.int32); bval = self._empty((B, E_cap), torch.int32)
         n_ev = self._empty((B, 2), torch.int32)
         vr_idx = self._empty((B, E_cap), torch.int32); vr_val = self._empty((B, E_cap))
@@ -341,37 +334,18 @@ class Engine:
         t_est = self._empty((B,), torch.float32)
         rounds = torch.zeros((B, 2), dtype=torch.int32, device=self.device)
         inv = t.lut_inv if self.accelerators else None
-        if fused:
-            with self._stage("S345_velocity"):
-                _lib.check(self.lib.vap_velocity_profile(
-                    C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), _p(db.node_attr), _p(db.node_flags), _p(db.n_nodes),
-                    _p(db.ap_attr), _p(db.ap_flags), _p(db.n_ap), _p(db.cons), _p(g.n_splines), _p(status),
-                    C.c_int64(grid.numel()), _p(grid), C.c_int(t.samples), C.c_int64(t.Q_cap), _p(t.lut_d), _p(t.lut_t),
-                    _p(t.total_len), C.c_int(t.spn), C.c_int64(t.P_cap), _p(t.prop_k), _p(t.prop_h), _p(inv),
-                    C.c_double(self.dd), C.c_double(self.dt), C.c_double(self.start_vel), C.c_double(self.end_vel),
-                    C.c_int64(D_cap), _p(n_samples), _p(tq), _p(kap), _p(th), C.c_int(E_cap), _p(ma), _p(bidx), _p(bval),
-                    _p(n_ev), _p(vr_idx), _p(vr_val), _p(st_idx), _p(n_vr), _p(ins_est), _p(scr), _p(rec), _p(statB),
-                    _p(vel_f), _p(vel), _p(t_est), _p(rounds), C.c_int(chunks), C.c_int(mode), self._stream()),
-                    "vap_velocity_profile")
-                self.launches += 6 if mode == 0 else 6
-        else:
-            with self._stage("S3_dist_sample"):
-                _lib.check(self.lib.vap_dist_sample_events(
-                    C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), _p(db.node_attr), _p(db.node_flags), _p(db.n_nodes),
-                    _p(db.ap_attr), _p(db.ap_flags), _p(db.n_ap), _p(db.cons), _p(g.n_splines), _p(status),
-                    C.c_int64(grid.numel()), _p(grid), C.c_int(t.samples), C.c_int64(t.Q_cap), _p(t.lut_d), _p(t.lut_t),
-                    _p(t.total_len), C.c_int(t.spn), C.c_int64(t.P_cap), _p(t.prop_k), _p(t.prop_h), C.c_int64(D_cap),
-                    _p(n_samples), _p(tq), _p(kap), _p(th), C.c_int(E_cap), _p(ma), _p(bidx), _p(bval), _p(n_ev), _p(vr_idx),
-                    _p(vr_val), _p(st_idx), _p(n_vr), C.c_double(self.dt), _p(ins_est), _p(scr), _p(inv), self._stream()),
-                    "vap_dist_sample_events")
-                self.launches += 3
-            with self._stage("S45_fwd_bwd"):
-                _lib.check(self.lib.vap_fwd_bwd_chunked(
-                    C.c_int64(B), _p(db.cons), _p(status), C.c_double(self.dd), C.c_double(self.dt), C.c_double(self.start_vel),
-                    C.c_double(self.end_vel), C.c_int64(D_cap), _p(n_samples), _p(kap), _p(th), C.c_int(E_cap), _p(ma),
-                    _p(bidx), _p(bval), _p(n_ev), _p(vr_idx), _p(vr_val), _p(st_idx), _p(n_vr), _p(rec), _p(statB),
-                    _p(vel_f), _p(vel), _p(t_est), _p(rounds), C.c_int(chunks), C.c_int(mode), self._stream()), "vap_fwd_bwd_chunked")
-                self.launches += 3
+        with self._stage("S345_velocity"):
+            _lib.check(self.lib.vap_velocity_profile(
+                C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), _p(db.node_attr), _p(db.node_flags), _p(db.n_nodes),
+                _p(db.ap_attr), _p(db.ap_flags), _p(db.n_ap), _p(db.cons), _p(g.n_splines), _p(status),
+                C.c_int64(grid.numel()), _p(grid), C.c_int(t.samples), C.c_int64(t.Q_cap), _p(t.lut_d), _p(t.lut_t),
+                _p(t.total_len), C.c_int(t.spn), C.c_int64(t.P_cap), _p(t.prop_k), _p(t.prop_h), _p(inv),
+                C.c_double(self.dd), C.c_double(self.dt), C.c_double(self.start_vel), C.c_double(self.end_vel),
+                C.c_int64(D_cap), _p(n_samples), _p(tq), _p(kap), _p(th), C.c_int(E_cap), _p(ma), _p(bidx), _p(bval),
+                _p(n_ev), _p(vr_idx), _p(vr_val), _p(st_idx), _p(n_vr), _p(ins_est), _p(scr), _p(rec), _p(statB),
+                _p(vel_f), _p(vel), _p(t_est), _p(rounds), C.c_int(chunks), C.c_int(mode), self._stream()),
+                "vap_velocity_profile")
+            self.launches += 6
         extra = dict(t=tq, kap=kap, th=th, max_accels=ma, bidx=bidx, bval=bval, n_ev=n_ev, vel_f=vel_f, rounds=rounds,
                      vr_idx=vr_idx, vr_val=vr_val, st_idx=st_idx, n_vr=n_vr)
         return n_samples, vel, t_est + ins_est, extra
