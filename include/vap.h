@@ -151,9 +151,10 @@ int vap_fwd_bwd(int64_t B, int N_max, int A_max, const double* node_attr, const 
  *     `chunks` speculative chunks per path that are re-run until they merge bitwise with the serial evaluation.
  *   The sampling fills a shared-memory tile from which a pre-pass hoists everything of a step that depends neither on
  *     the velocity state nor on the events (per sample |kappa|, the velocity caps, the static acceleration limit; per
- *     step the wheel-acceleration denominator and its reciprocal), so kappa / theta per distance sample never go to
- *     memory: t / kap / th [B][D_cap] are inspection outputs (pass all three or three NULLs).  The static acceleration
- *     limits of paths with max_acceleration overrides are rewritten after the event resolution.
+ *     step the wheel-acceleration denominator; the passes make its reciprocal themselves), so kappa / theta per
+ *     distance sample never go to memory: t / kap / th [B][D_cap] are inspection outputs (pass all three or three
+ *     NULLs).  The static acceleration limits of paths with max_acceleration overrides are rewritten after the event
+ *     resolution.
  *   n_samples[B] and status as in vap_dist_sample (status may also get VAP_ERR_EVENTS); max_accels[B][E_cap],
  *     bidx/bval[B][E_cap] and n_ev[B][2] as in vap_fwd_bwd, E_cap >= N_max + A_max + 2.  vr_idx/vr_val[B][E_cap]:
  *     the initial-velocity regimes, v0[i] = vr_val[j] for the last j with vr_idx[j] <= i; st_idx[B][E_cap]: the stop
@@ -162,8 +163,8 @@ int vap_fwd_bwd(int64_t B, int N_max, int A_max, const double* node_attr, const 
  *     turn profiles (sizing only).
  *   The arrays the passes stream are chunk-interleaved in blocks of four steps (steps 4k .. 4k+3 of chunk c are one
  *     32-byte sector; sector (k, c) follows sector (k, c-1)) so that every warp-wide access is one contiguous run and a
- *     chunk re-run alone fetches only bytes it uses: rec [B][RS][5] f64 (per block five field planes of 4 x `chunks`
- *     doubles), statB / vel_f [B][RS] f64 (the backward pass's static acceleration limit, touched only for paths with
+ *     chunk re-run alone fetches only bytes it uses: rec [B][RS][4] f64 (per block four field planes of 4 x `chunks`
+ *     doubles, 32 bytes per sample), statB / vel_f [B][RS] f64 (the backward pass's static acceleration limit, touched only for paths with
  *     max_acceleration overrides; forward velocities; both slot order), RS = vap_pass_row_slots(D_cap, chunks).
  *     chunks: a power of two from 8 to 256.
  *   vel[B][D_cap] (D_cap even): final velocities in sample order, written by the backward pass itself (mode 1: the

@@ -1240,10 +1240,10 @@ static int launch_passes(int64_t B, size_t ss, cudaStream_t st, const double* co
                          const int32_t* n_vr, double* vel_f, double* vel, float* t_est, int32_t* rounds, bool backward,
                          int warm, int max_rounds, const double* statB)
 {
-    // behind the tables every warp has a two-stage ring of 5 (forward) / 6 (backward) planes of 1 KB + 2 mbarriers
+    // behind the tables every warp has a two-stage ring of 4 (forward) / 5 (backward) planes of 1 KB + 2 mbarriers
     const int warps = (NT + 31) / 32;
     const int ring_off = (int)((ss + 127) / 128 * 128);
-    const int planes = backward ? 6 : 5;
+    const int planes = backward ? 5 : 4;
     const size_t smem = (size_t)ring_off + (size_t)warps * (2 * planes * TMA_PLANE_DOUBLES * 8 + 16);
     cudaError_t e = cudaSuccess;
     if (!backward) {
@@ -1730,7 +1730,7 @@ static size_t carve_batch(char* base, int64_t B, int N_max, int A_max, int max_s
     s.t_est = w.take<float>(B);
     s.scr = w.take<int32_t>(nscr);
     s.rounds = w.take<int32_t>((size_t)B * 2);
-    s.rec = w.take<double>((size_t)B * s.RS * 5);
+    s.rec = w.take<double>((size_t)B * s.RS * 4);
     s.statB = w.take<double>((size_t)B * s.RS);
     s.vel_f = w.take<double>((size_t)B * s.RS);
     s.stage = w.take<double>((size_t)8 * B * (T_cap + 1));

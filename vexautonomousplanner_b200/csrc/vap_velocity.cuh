@@ -1,5 +1,5 @@
 // vap_velocity.cuh -- stages S3-events / S4 / S5: sample-parallel event detection, a pre-pass that hoists every term of
-// the forward / backward recurrences that depends neither on the velocity state nor on the events into five values per
+// the forward / backward recurrences that depends neither on the velocity state nor on the events into four values per
 // sample (chunk-interleaved rows, written once), and chunk-speculative kernels that run the exact serial recurrences on
 // many chunks of one path at once over coalesced streams.
 //
@@ -142,8 +142,6 @@ __global__ void k_resolve_events(long long B, int N_max, int A_max, const double
     }
 }
 
-__device__ __forceinline__ double recip_for_pass(double g);   // defined with the pass kernels below
-
 // ---- chunk-interleaved, block-of-four layout of everything the passes stream ------------------------------------------
 // A path's D-1 steps ("edges" e = 0 .. D-2: forward step e goes from sample e to e+1, backward step e+1 from sample e+1
 // to e) are cut into NT chunks of Lc edges (Lc = ceil((D-1)/NT) rounded up to a multiple of PB = 4); chunk c owns edges
@@ -163,24 +161,24 @@ __device__ __forceinline__ int edge_slot(int e, int Lc, int NT)
     const int c = e / Lc, r = e - c * Lc;
     return ((r >> 2) * NT + c) * PB + (r & 3);
 }
-// record element (row r, field f, column c) of a path: rec[((r / 4) * 5 + f) * 4 NT + 4 c + r % 4]
+// record element (row r, field f, column c) of a path: rec[((r / 4) * 4 + f) * 4 NT + 4 c + r % 4]
 __device__ __forceinline__ size_t rec_index(int r, int f, int c, int NT)
 {
-    return ((size_t)(r >> 2) * 5 + f) * (PB * NT) + (size_t)c * PB + (r & 3);
+    return ((size_t)(r >> 2) * 4 + f) * (PB * NT) + (size_t)c * PB + (r & 3);
 }
 
 // ---- pre-pass (parallel): everything of a pass step that depends neither on the velocity state nor on the events --------
-// Per block of four chunk positions five field planes of 4 NT doubles: element (row s, field f, column c) of a path is
-// rec[rec_index(s, f, c)]; the terms of the final sample D-1 sit in the last three doubles of the path's 5 RS.
+// Per block of four chunk positions four field planes of 4 NT doubles: element (row s, field f, column c) of a path is
+// rec[rec_index(s, f, c)]; the terms of the final sample D-1 sit in the last three doubles of the path's 4 RS.
 // fields 0-2, per sample i (row / column of edge i):
 //    { |kappa_i|, G_i, stat_i }
 //       G_i    = min(vlim_i, cap_i)                         velocity caps (:212-218, :239)
 //       stat_i = min(max_ang_acc/|k|, 2 A0/(w|k|+2), A0)    the state-independent acceleration limits for the path's own
 //                (A0 when straight)                         max_acc A0 -- forward a_static AND backward d_static as long as
 //                                                           no node / action point overrides max_acceleration
-// fields 3-4, per edge e:
-//    { gh_e = 2|theta_{e+1} - theta_e|, recip_for_pass(gh_e) }   denominator of the wheel-acceleration term of forward
-//                                                                step e and of backward step e+1, and its reciprocal
+// field 3, per edge e:
+//    gh_e = 2|theta_{e+1} - theta_e|       denominator of the wheel-acceleration term of forward step e and of backward
+//                                          step e+1 (the passes make its reciprocal themselves, see recip_for_pass)
 // What depends on the events is applied by the passes themselves from small shared-memory tables: the initial velocity
 // v0[i+1] (regimes, stops, end velocity) enters as C_i = min(v0[i+1], G_i).  Only a path with max_acceleration overrides
 // makes the pre-pass look at the regime table: stat then uses the forward regime's max_acc and the backward pass's limit
@@ -330,7 +328,7 @@ __global__ void __launch_bounds__(256, VAP_SP_MINB) k_sample_prepass(
     const int st = (TR + 2) | 1;                     // odd stride; row r of the tile sits at index r + 1 (index 0: row s0-1)
     const double V = cons[b * 6 + 0], A0 = cons[b * 6 + 1], w = cons[b * 6 + 5];
     const int A = n_ap ? n_ap[b] : 0;
-    double* pr = rec + (size_t)b * RS * 5;
+    double* pr = rec + (size_t)b * RS * 4;
     const int PS = PB * NT;
     const size_t orow = (size_t)b * D_cap;
     for (int it = 0; it < SP_TILES && j0 < jend; ++it, j0 += blockDim.x) {
@@ -396,15 +394,15 @@ __global__ void __launch_bounds__(256, VAP_SP_MINB) k_sample_prepass(
         }
         // ---- the records of slot j
         const double gh = 2 * fabs(t_th[tl + 1] - t_th[tl]);
-        const size_t o = (size_t)(j >> (sh + 2)) * (5 * PS) + (size_t)(j & (PS - 1));
-        VAP_CHECK(9, tl >= 1 && tl + 1 < TC * st && o + 4 * PS < (size_t)(5 * RS - 3) && c - c0 >= 0 && c - c0 < TC && s - s0 >= 0 && s - s0 < TR);
+        const size_t o = (size_t)(j >> (sh + 2)) * (4 * PS) + (size_t)(j & (PS - 1));
+        VAP_CHECK(9, tl >= 1 && tl + 1 < TC * st && o + 3 * PS < (size_t)(4 * RS - 3) && c - c0 >= 0 && c - c0 < TC && s - s0 >= 0 && s - s0 < TR);
         const SampleTerms tm = prepass_sample<false>(V, A0, A0, w, s_c[0], s_c[1], t_k[tl]);
-        pr[o] = tm.ak; pr[o + PS] = tm.G; pr[o + 2 * PS] = tm.stat; pr[o + 3 * PS] = gh; pr[o + 4 * PS] = recip_for_pass(gh);
+        pr[o] = tm.ak; pr[o + PS] = tm.G; pr[o + 2 * PS] = tm.stat; pr[o + 3 * PS] = gh;
         if (e == steps - 1) {                        // the final sample (no edge starts there): the backward pass starts on it
             double kl, hl;
             snap_gather2_32(pk, ph, tn, pg, kl, hl);
             const SampleTerms u = prepass_sample<false>(V, A0, A0, w, s_c[0], s_c[1], kl);
-            pr[5 * RS - 3] = u.ak; pr[5 * RS - 2] = u.G; pr[5 * RS - 1] = u.stat;
+            pr[4 * RS - 3] = u.ak; pr[4 * RS - 2] = u.G; pr[4 * RS - 1] = u.stat;
             if (t_out) { t_out[orow + D - 1] = tn; kap_out[orow + D - 1] = kl; th_out[orow + D - 1] = hl; }
         }
     }
@@ -430,7 +428,7 @@ __global__ void __launch_bounds__(256) k_prepass_ovr(
     const double V = cons[b * 6 + 0], w = cons[b * 6 + 5];
     const double mav = 2 * V / w, maa = 2 * A0 / w;
     const int PS = PB * NT;
-    double* pr = rec + (size_t)b * RS * 5;
+    double* pr = rec + (size_t)b * RS * 4;
     const int nb = n_ev[2 * b + 1];
     const double dec_b = max_accels[(size_t)b * E_cap + bval[(size_t)b * E_cap + nb - 1]];       // backward max_dec
     for (int j = threadIdx.x; j < (Lc << sh); j += blockDim.x) {
@@ -438,14 +436,14 @@ __global__ void __launch_bounds__(256) k_prepass_ovr(
         const int s = ((j >> (sh + 2)) << 2) + (j & 3);
         const int e = c * Lc + s;
         if (e >= steps) continue;
-        const size_t o = (size_t)(j >> (sh + 2)) * (5 * PS) + (size_t)(j & (PS - 1));
+        const size_t o = (size_t)(j >> (sh + 2)) * (4 * PS) + (size_t)(j & (PS - 1));
         const double acc_f = max_accels[(size_t)b * E_cap + bval[(size_t)b * E_cap + last_le(bidx + (size_t)b * E_cap, nb, e)]];
         const SampleTerms t = prepass_sample<true>(V, acc_f, dec_b, w, mav, maa, pr[o]);
         pr[o + 2 * PS] = t.stat;
         statB[(size_t)b * RS + j] = t.stat_b;
         if (e == steps - 1) {
-            const SampleTerms u = prepass_sample<true>(V, dec_b, dec_b, w, mav, maa, pr[5 * RS - 3]);
-            pr[5 * RS - 1] = u.stat;
+            const SampleTerms u = prepass_sample<true>(V, dec_b, dec_b, w, mav, maa, pr[4 * RS - 3]);
+            pr[4 * RS - 1] = u.stat;
             statB[(size_t)b * RS + RS - 1] = u.stat_b;
         }
     }
@@ -481,9 +479,10 @@ __device__ __noinline__ double accel_ang_div(double num, double h2)
     return qnan;                                         // NaN denominator (the pre-pass's "straight" marker)
 }
 
-// Reciprocal of the division's denominator g = 2|dtheta|, made ONCE per sample by the pre-pass (it does not depend on the
-// velocity state), so that the state-dependent chain of a pass step holds one multiplication and two fused residual
-// corrections instead of a reciprocal refinement:
+// Reciprocal of the division's denominator g = 2|dtheta|.  It does not depend on the velocity state, so the passes make it
+// off the chain -- the lockstep sweeps for the four steps of a ring stage at once when the stage lands, the fix-up re-runs
+// for a pair of steps two steps after loading it -- and the state-dependent chain of a step holds one multiplication and
+// two fused residual corrections instead of a reciprocal refinement:
 //    > 0 and finite : RN(1/g), g a normal number whose significand is not all ones (Markstein's exception)
 //    +inf           : g == 0 (two samples snapped to the same heading entry; ~44 % of the samples)
 //    -1             : anything else (g NaN / subnormal / all-ones significand): the pass takes the generic division
@@ -497,6 +496,7 @@ __device__ __forceinline__ double recip_for_pass(double g)
     const double r = 1.0 / d;
     return safe ? r : ((g == 0.0) ? __longlong_as_double(0x7ff0000000000000LL) : -1.0);
 }
+__device__ __forceinline__ double2 recip_for_pass(double2 g) { return make_double2(recip_for_pass(g.x), recip_for_pass(g.y)); }
 
 // num / h2 given rce = recip_for_pass(h2) (or NaN when h2 is the straight marker).  q0 = num * r, then two residual
 // corrections: after the first the quotient is faithful, and with the correctly rounded reciprocal one more gives the
@@ -562,14 +562,15 @@ __device__ __forceinline__ double bwd_step(double ak, double gh, double rg, doub
 // Rounds end when no chunk had to re-run; then, by induction from chunk 0, every value is the serial value.
 //
 // The kernels are bound by the latency of the dependent fp64 chain of one step, so they are written for a short chain:
-// event tables in shared memory, 32-bit indices, the division's reciprocal from the pre-pass, coalesced slot-order streams.
+// event tables in shared memory, 32-bit indices, the division's reciprocal made off the chain, coalesced slot-order streams.
 // The lockstep first sweep takes its records from a per-warp shared-memory ring that TMA bulk copies fill a whole block
 // ahead; the fix-up re-runs and the warm-up are out of line and load their records one pair ahead themselves.
 // ------------------------------------------------------------------------------------------------------------------
 #define CH_INT_MAX 2147483647
 #ifndef VAP_PASS_REGS_TMA
-#define VAP_PASS_REGS_TMA 112 // residency is limited by the shared-memory rings (10 - 12 KB per warp), not by registers; 112 keeps the
-                              // out-of-line re-run functions free of spills (96: 3.69 ms per cfg2 step, 112: 3.47, 128: 3.56)
+#define VAP_PASS_REGS_TMA 112 // 112 x 32 registers allow 18 one-warp CTAs per SM; with cfg2's tables the shared-memory rings (8 KB
+                              // forward, 10 KB backward per warp) allow 21 / 18.  Fewer registers make the out-of-line re-run
+                              // functions spill more (96: 3.69 ms per cfg2 step, 112: 3.47, 128: 3.56)
 #endif
 
 // 16-byte read-only load of two consecutive doubles
@@ -607,7 +608,7 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
                                         double old_end, int lo, int len, const FwdTables& T, double hw,
                                         double dd, double& v, double& sq, bool prev_same)
 {
-    constexpr int PS = PB * NT, BS = 5 * PS;
+    constexpr int PS = PB * NT, BS = 4 * PS;
     constexpr bool RERUN = (MODE == RUN_RERUN);
     constexpr bool DRY = (MODE == RUN_DRY);
     int j = 0;
@@ -630,7 +631,8 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
             prev_same = same;                                                                                        \
         }                                                                                                            \
         ++e;
-    double2 akA = ldg_d2(p), GA = ldg_d2(p + PS), stA = ldg_d2(p + 2 * PS), ghA = ldg_d2(p + 3 * PS), rgA = ldg_d2(p + 4 * PS);
+    // a pair's reciprocals are made two steps after its loads, just before its own steps
+    double2 akA = ldg_d2(p), GA = ldg_d2(p + PS), stA = ldg_d2(p + 2 * PS), ghA = ldg_d2(p + 3 * PS), rgA;
     double2 akB, GB, stB, ghB, rgB;
     double2 oA = make_double2(0.0, 0.0), oB = oA;    // old velocities (RERUN): pair A = samples e, e+1; pair B = e+2, e+3
     if (RERUN) oA = *reinterpret_cast<const double2*>(q);
@@ -640,18 +642,19 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
         for (int k = 1; k < RERUN_PF; k++)
             if (k < (len >> 2)) {
 #pragma unroll
-                for (int f = 0; f < 5; f++) l2_prefetch(p + (size_t)k * BS + f * PS);
+                for (int f = 0; f < 4; f++) l2_prefetch(p + (size_t)k * BS + f * PS);
                 l2_prefetch(q + (size_t)k * PS);
             }
     }
     for (int blk = len >> 2; blk > 0; --blk) {
         if (RERUN && blk > RERUN_PF) {
 #pragma unroll
-            for (int f = 0; f < 5; f++) l2_prefetch(p + (size_t)RERUN_PF * BS + f * PS);
+            for (int f = 0; f < 4; f++) l2_prefetch(p + (size_t)RERUN_PF * BS + f * PS);
             l2_prefetch(q + (size_t)RERUN_PF * PS);
         }
-        akB = ldg_d2(p + 2); GB = ldg_d2(p + PS + 2); stB = ldg_d2(p + 2 * PS + 2); ghB = ldg_d2(p + 3 * PS + 2); rgB = ldg_d2(p + 4 * PS + 2);
+        akB = ldg_d2(p + 2); GB = ldg_d2(p + PS + 2); stB = ldg_d2(p + 2 * PS + 2); ghB = ldg_d2(p + 3 * PS + 2);
         if (RERUN) oB = *reinterpret_cast<const double2*>(q + 2);
+        rgA = recip_for_pass(ghA);
         const double vin = v;
         FWD_ONE(akA.x, GA.x, stA.x, ghA.x, rgA.x, oA.y)
         const double v1 = v;
@@ -659,8 +662,9 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
         FWD_ONE(akA.y, GA.y, stA.y, ghA.y, rgA.y, oB.x)
         const double v2 = v;
         p += BS;
-        akA = ldg_d2(p); GA = ldg_d2(p + PS); stA = ldg_d2(p + 2 * PS); ghA = ldg_d2(p + 3 * PS); rgA = ldg_d2(p + 4 * PS);
+        akA = ldg_d2(p); GA = ldg_d2(p + PS); stA = ldg_d2(p + 2 * PS); ghA = ldg_d2(p + 3 * PS);
         if (RERUN) oA = *reinterpret_cast<const double2*>(q + PS);
+        rgB = recip_for_pass(ghB);
         FWD_ONE(akB.x, GB.x, stB.x, ghB.x, rgB.x, oB.y)
         if (RERUN) st_d2(q + 2, v2, v);
         FWD_ONE(akB.y, GB.y, stB.y, ghB.y, rgB.y, ((e + 1 < hi) ? oA.x : old_end))
@@ -670,6 +674,7 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
     if (e < hi) {
         if (!DRY) q[0] = v;
         const int rem = hi - e;
+        rgA = recip_for_pass(ghA);
         {
             const double old = RERUN ? ((rem > 1) ? oA.y : old_end) : 0.0;
             FWD_ONE(akA.x, GA.x, stA.x, ghA.x, rgA.x, old)
@@ -681,9 +686,8 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
             if (!DRY && e < hi) q[2] = v;
         }
         if (e < hi) {
-            const double a2 = __ldg(p + 2), g2 = __ldg(p + PS + 2), s2 = __ldg(p + 2 * PS + 2), h2 = __ldg(p + 3 * PS + 2),
-                         r2 = __ldg(p + 4 * PS + 2);
-            FWD_ONE(a2, g2, s2, h2, r2, old_end)
+            const double a2 = __ldg(p + 2), g2 = __ldg(p + PS + 2), s2 = __ldg(p + 2 * PS + 2), h2 = __ldg(p + 3 * PS + 2);
+            FWD_ONE(a2, g2, s2, h2, recip_for_pass(h2), old_end)
         }
     }
 #undef FWD_ONE
@@ -694,15 +698,16 @@ __device__ __forceinline__ bool fwd_run(const double* __restrict__ p, double* __
 // ---- sweeps staged through shared memory by TMA -------------------------------------------------------------------------
 // In the block-of-four layout the share of one WARP (32 columns) in one block row is a contiguous 1 KB per field plane, so
 // the lockstep first sweep does not load records into registers at all: one lane issues one cp.async.bulk per plane and
-// block row (five for the forward pass; six for the backward pass, which also streams the forward velocities) into a two-stage
-// shared-memory ring that completes on an mbarrier, a whole block (four steps) ahead of its use.  A step then takes its five
-// values from shared memory.  Nothing of the stream passes through L1, no look-ahead buffers live in registers, and the HBM
-// reads are 1 KB bursts issued thousands of cycles before they are needed.
+// block row (four for the forward pass; five for the backward pass, which also streams the forward velocities) into a
+// two-stage shared-memory ring that completes on an mbarrier, a whole block (four steps) ahead of its use.  When a stage has
+// landed, each lane makes the reciprocals of its four gh values together (kept in registers) and then takes everything
+// else of a step from shared memory.  Nothing of the stream passes through L1, no look-ahead buffers live in registers, and
+// the HBM reads are 1 KB bursts issued thousands of cycles before they are needed.
 #define TMA_PLANE_DOUBLES (PB * 32)                    // one plane of one stage: 32 columns x 4 rows
 struct WarpRing {
     double* stage;       // this warp's two stages
     unsigned bar;        // shared-memory address of its two mbarriers
-    int planes;          // field planes per stage (5 forward, 6 backward)
+    int planes;          // field planes per stage (4 forward, 5 backward)
     unsigned bytes;      // bytes of one plane copy (32 bytes per column of the warp)
 #ifdef VAP_BOUNDS_CHECK
     const double *rec_lo, *rec_hi, *x_lo, *x_hi;     // the path's record rows / slot-order rows (forward velocities, override limits)
@@ -714,22 +719,22 @@ template <int NT>
 __device__ __forceinline__ void ring_issue(const WarpRing& R, int s, const double* rec_row0, const double* x_row0,
                                            const double* sb_row0, int rb)
 {
-    constexpr int PS = PB * NT, BS = 5 * PS;
+    constexpr int PS = PB * NT, BS = 4 * PS;
     const unsigned bar = R.bar + 8 * s;
     const unsigned dst = (unsigned)__cvta_generic_to_shared(R.stage + (size_t)s * R.planes * TMA_PLANE_DOUBLES);
     fence_proxy_async();                                   // the lanes' reads of this stage precede the TMA writes
     mbar_expect_tx(bar, R.bytes * R.planes);
     const double* src = rec_row0 + (size_t)rb * BS;
     if (NT == 32 && !sb_row0) {
-        // 32 chunks: the five planes of a block row are contiguous in memory and in the stage: ONE 5 KB copy
+        // 32 chunks: the four planes of a block row are contiguous in memory and in the stage: ONE 4 KB copy
 #ifdef VAP_BOUNDS_CHECK
-        VAP_CHECK(1, rb >= 0 && src >= R.rec_lo && src + 5 * R.bytes / 8 <= R.rec_hi && (reinterpret_cast<uintptr_t>(src) & 15) == 0);
-        VAP_CHECK(2, dst >= R.smem_lo && dst + 5 * R.bytes <= R.smem_hi && bar >= R.smem_hi && bar + 8 <= R.bar_hi);
+        VAP_CHECK(1, rb >= 0 && src >= R.rec_lo && src + 4 * R.bytes / 8 <= R.rec_hi && (reinterpret_cast<uintptr_t>(src) & 15) == 0);
+        VAP_CHECK(2, dst >= R.smem_lo && dst + 4 * R.bytes <= R.smem_hi && bar >= R.smem_hi && bar + 8 <= R.bar_hi);
 #endif
-        bulk_g2s(dst, src, 5 * R.bytes, bar);
+        bulk_g2s(dst, src, 4 * R.bytes, bar);
     } else
 #pragma unroll
-    for (int f = 0; f < 5; f++) {
+    for (int f = 0; f < 4; f++) {
         const double* g = (f == 2 && sb_row0) ? sb_row0 + (size_t)rb * PS : src + f * PS;
 #ifdef VAP_BOUNDS_CHECK
         if (f == 2 && sb_row0) VAP_CHECK(0, rb >= 0 && (reinterpret_cast<uintptr_t>(g) & 15) == 0);
@@ -741,9 +746,9 @@ __device__ __forceinline__ void ring_issue(const WarpRing& R, int s, const doubl
     if (x_row0) {
 #ifdef VAP_BOUNDS_CHECK
         VAP_CHECK(3, x_row0 + (size_t)rb * PS >= R.x_lo && x_row0 + (size_t)rb * PS + R.bytes / 8 <= R.x_hi);
-        VAP_CHECK(2, dst + 5 * TMA_PLANE_DOUBLES * 8 + R.bytes <= R.smem_hi);
+        VAP_CHECK(2, dst + 4 * TMA_PLANE_DOUBLES * 8 + R.bytes <= R.smem_hi);
 #endif
-        bulk_g2s(dst + 5 * TMA_PLANE_DOUBLES * 8, x_row0 + (size_t)rb * PS, R.bytes, bar);
+        bulk_g2s(dst + 4 * TMA_PLANE_DOUBLES * 8, x_row0 + (size_t)rb * PS, R.bytes, bar);
     }
 }
 
@@ -776,8 +781,7 @@ __device__ __forceinline__ void fwd_sweep_tma(const WarpRing& R, const double* _
     const int nfull = len >> 2;
 #define FWD_T(ROW_)                                                                                                  \
         {                                                                                                            \
-            const double ak_ = S[ROW_], G_ = S[PD + ROW_], st_ = S[2 * PD + ROW_], gh_ = S[3 * PD + ROW_],             \
-                         rg_ = S[4 * PD + ROW_];                                                                     \
+            const double ak_ = S[ROW_], G_ = S[PD + ROW_], st_ = S[2 * PD + ROW_], gh_ = gh[ROW_], rg_ = rg[ROW_];    \
             if (e == nb_next) { j++; acc = T.acc[j]; nb_next = (j + 1 < T.n_b) ? T.bi[j + 1] : CH_INT_MAX; }          \
             if (e + 1 == nv_next) { jv++; v0n = T.vv[jv]; nv_next = (jv + 1 < T.n_v) ? T.vi[jv + 1] : CH_INT_MAX; }  \
             v = fwd_step(ak_, gh_, rg_, st_, pymin(v0n, G_), v, sq, acc, hw, dd);                                    \
@@ -786,8 +790,13 @@ __device__ __forceinline__ void fwd_sweep_tma(const WarpRing& R, const double* _
     for (int blk = 0; blk < nbw; ++blk) {
         const int s = blk & 1;
         mbar_wait(R.bar + 8 * s, (blk >> 1) & 1);
-        const double* S = R.stage + (size_t)s * 5 * PD + lc * PB;
-        VAP_CHECK(6, lc >= 0 && lc < 32 && (unsigned)__cvta_generic_to_shared(S + 4 * PD + 3) + 8 <= R.smem_hi);
+        const double* S = R.stage + (size_t)s * 4 * PD + lc * PB;
+        VAP_CHECK(6, lc >= 0 && lc < 32 && (unsigned)__cvta_generic_to_shared(S + 3 * PD + 3) + 8 <= R.smem_hi);
+        double gh[PB], rg[PB];
+#pragma unroll
+        for (int r = 0; r < PB; r++) gh[r] = S[3 * PD + r];
+#pragma unroll
+        for (int r = 0; r < PB; r++) rg[r] = recip_for_pass(gh[r]);
         if (blk < nfull) {                           // a whole block of this lane's chunk
             const double vin = v;
             FWD_T(0)
@@ -894,21 +903,21 @@ __global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_fwd_chunked(
     const bool active = c < nch;
     const int lo = c * Lc;
     const int len = (lo + Lc < steps) ? Lc : steps - lo;
-    const double* P = rec + (size_t)b * RS * 5;
+    const double* P = rec + (size_t)b * RS * 4;
     double* tail = (active && lo + len == steps) ? vf + (RS - 1) : nullptr;  // only the last chunk stores the final sample
     const double hw = cons[b * 6 + 5] * 0.5;
-    // every warp owns a two-stage ring (5 planes of 1 KB per stage) and two mbarriers behind the tables
+    // every warp owns a two-stage ring (4 planes of 1 KB per stage) and two mbarriers behind the tables
     WarpRing R;
     constexpr int WARPS = (NT + 31) / 32;
     const int w = c >> 5;
-    R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 5 * TMA_PLANE_DOUBLES;
-    R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8 + 16 * w);
-    R.planes = 5;
+    R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 4 * TMA_PLANE_DOUBLES;
+    R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 4 * TMA_PLANE_DOUBLES * 8 + 16 * w);
+    R.planes = 4;
     R.bytes = (NT < 32 ? NT : 32) * PB * 8;
 #ifdef VAP_BOUNDS_CHECK
-    R.rec_lo = P; R.rec_hi = P + 5 * RS; R.x_lo = R.x_hi = nullptr;
+    R.rec_lo = P; R.rec_hi = P + 4 * RS; R.x_lo = R.x_hi = nullptr;
     R.smem_lo = (unsigned)__cvta_generic_to_shared(s_mem + ring_off);
-    R.smem_hi = R.smem_lo + WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8;
+    R.smem_hi = R.smem_lo + WARPS * 2 * 4 * TMA_PLANE_DOUBLES * 8;
     R.bar_hi = R.smem_hi + 16 * WARPS;
 #endif
     if ((c & 31) == 0) { mbar_init(R.bar, 1); mbar_init(R.bar + 8, 1); fence_mbar_init(); }
@@ -943,7 +952,7 @@ __global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_fwd_chunked(
             }
             s_usev[c] = v; s_usew[c] = sq;
             // extent of what this lane's runs touch (look-ahead block included): record rows and forward-velocity row
-            VAP_CHECK(4, c * PB + PB <= PB * NT && (size_t)(((len + 3) >> 2) + 1) * 5 * PB * NT <= (size_t)(5 * RS - 3) &&
+            VAP_CHECK(4, c * PB + PB <= PB * NT && (size_t)(((len + 3) >> 2) + 1) * 4 * PB * NT <= (size_t)(4 * RS - 3) &&
                              (size_t)(((len + 3) >> 2) + 1) * PB * NT <= (size_t)(RS - 1) && lo + len <= steps);
         }
         fwd_sweep_tma<NT>(R, P + (c & ~31) * PB, c & 31, vf + c * PB, tail, lo, active ? len : 0, T, hw, dd, v, sq);
@@ -978,8 +987,8 @@ __global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_fwd_chunked(
 // chunk's FIRST block of the record rows / forward velocities / override limits, o at sample lo of the path's final
 // velocities, which this pass writes in SAMPLE order (16-byte pairs: the time stage and the API read them as they are).
 // Edge e = lo + r (the reference's step i = e+1 -> e) uses the terms of sample e+1 (fields 0-2 of row r+1: carried over from
-// the pair above; for the chunk's top edge the three `top` values), gh / rg (fields 3-4) and the forward velocity of row r,
-// and writes the final velocity of sample e.
+// the pair above; for the chunk's top edge the three `top` values), gh (field 3) of row r with its reciprocal, and the
+// forward velocity of row r, and writes the final velocity of sample e.
 // OVR: the path has max_acceleration overrides; the static limit of the backward pass then comes from its own slot-order
 // array `sb` (same slots as the forward velocities) instead of field 2 of the record rows.
 template <int NT, int MODE, bool OVR>
@@ -989,7 +998,7 @@ __device__ __forceinline__ bool bwd_run(const double* __restrict__ p, const doub
                                         double dd, double& v, double& sq, bool prev_same, float& est, float dd_over_dt,
                                         double old_top = 0.0)
 {
-    constexpr int PS = PB * NT, BS = 5 * PS;
+    constexpr int PS = PB * NT, BS = 4 * PS;
     constexpr bool RERUN = (MODE == RUN_RERUN);
     constexpr bool DRY = (MODE == RUN_DRY);
     // regime at the chunk start (walking down from D-1): the smallest boundary index > i was the last one applied
@@ -1020,44 +1029,45 @@ __device__ __forceinline__ bool bwd_run(const double* __restrict__ p, const doub
     double oup = old_top;                            // velocity of sample e+1 in this lane's previous run (its start state then)
     // ragged top of the path's last chunk: up to three edges (rows 4 blk + rem-1 .. 4 blk), one at a time
     for (int r = (len & 3) - 1; r >= 0; --r) {
-        const double gh = __ldg(p + 3 * PS + r), rg = __ldg(p + 4 * PS + r), fv = __ldg(f + r);
+        const double gh = __ldg(p + 3 * PS + r), fv = __ldg(f + r);
         const double old = RERUN ? o[r] : 0.0;
-        BWD_ONE(tak, tG, tst, gh, rg, fv, old, oup)
+        BWD_ONE(tak, tG, tst, gh, recip_for_pass(gh), fv, old, oup)
         if (!DRY) o[r] = v;
         oup = old;
         tak = __ldg(p + r); tG = __ldg(p + PS + r); tst = OVR ? __ldg(sb + r) : __ldg(p + 2 * PS + r);
     }
     if (blk == 0) return false;
     // whole blocks, top down: pair B (rows 2, 3) then pair A (rows 0, 1) of each; the next pair is fetched while the current
-    // one is being used
+    // one is being used, and its reciprocals are made two steps later, just before its own steps
     p -= BS; f -= PS; sb -= PS; if (!DRY) o -= PB;
     if (RERUN) {
 #pragma unroll
         for (int k = 1; k < RERUN_PF; k++)
             if (k < blk) {
 #pragma unroll
-                for (int fl = 0; fl < 5; fl++) if (!(OVR && fl == 2)) l2_prefetch(p - (size_t)k * BS + fl * PS);
+                for (int fl = 0; fl < 4; fl++) if (!(OVR && fl == 2)) l2_prefetch(p - (size_t)k * BS + fl * PS);
                 l2_prefetch(f - (size_t)k * PS);
                 l2_prefetch(o - k * PB);
                 if (OVR) l2_prefetch(sb - (size_t)k * PS);
             }
     }
     double2 akB = ldg_d2(p + 2), GB = ldg_d2(p + PS + 2), stB = OVR ? ldg_d2(sb + 2) : ldg_d2(p + 2 * PS + 2),
-            ghB = ldg_d2(p + 3 * PS + 2), rgB = ldg_d2(p + 4 * PS + 2), fB = ldg_d2(f + 2);
-    double2 akA, GA, stA, ghA, rgA, fA;
+            ghB = ldg_d2(p + 3 * PS + 2), fB = ldg_d2(f + 2);
+    double2 akA, GA, stA, ghA, fA;
     double2 oA = make_double2(0.0, 0.0), oB = oA;
     if (RERUN) oB = *reinterpret_cast<const double2*>(o + 2);
     while (true) {
         if (RERUN && blk > RERUN_PF) {
 #pragma unroll
-            for (int fl = 0; fl < 5; fl++) if (!(OVR && fl == 2)) l2_prefetch(p - (size_t)RERUN_PF * BS + fl * PS);
+            for (int fl = 0; fl < 4; fl++) if (!(OVR && fl == 2)) l2_prefetch(p - (size_t)RERUN_PF * BS + fl * PS);
             l2_prefetch(f - (size_t)RERUN_PF * PS);
             l2_prefetch(o - RERUN_PF * PB);
             if (OVR) l2_prefetch(sb - (size_t)RERUN_PF * PS);
         }
-        akA = ldg_d2(p); GA = ldg_d2(p + PS); stA = OVR ? ldg_d2(sb) : ldg_d2(p + 2 * PS); ghA = ldg_d2(p + 3 * PS); rgA = ldg_d2(p + 4 * PS);
+        akA = ldg_d2(p); GA = ldg_d2(p + PS); stA = OVR ? ldg_d2(sb) : ldg_d2(p + 2 * PS); ghA = ldg_d2(p + 3 * PS);
         fA = ldg_d2(f);
         if (RERUN) oA = *reinterpret_cast<const double2*>(o);
+        const double2 rgB = recip_for_pass(ghB);
         BWD_ONE(tak, tG, tst, ghB.y, rgB.y, fB.y, oB.y, oup)
         const double v3 = v;
         BWD_ONE(akB.y, GB.y, stB.y, ghB.x, rgB.x, fB.x, oB.x, oB.y)
@@ -1068,9 +1078,10 @@ __device__ __forceinline__ bool bwd_run(const double* __restrict__ p, const doub
         const bool more = --blk > 0;
         if (more) {                                                  // pair B of the block below
             akB = ldg_d2(p - BS + 2); GB = ldg_d2(p - BS + PS + 2); stB = OVR ? ldg_d2(sb - PS + 2) : ldg_d2(p - BS + 2 * PS + 2);
-            ghB = ldg_d2(p - BS + 3 * PS + 2); rgB = ldg_d2(p - BS + 4 * PS + 2); fB = ldg_d2(f - PS + 2);
+            ghB = ldg_d2(p - BS + 3 * PS + 2); fB = ldg_d2(f - PS + 2);
             if (RERUN) oB = *reinterpret_cast<const double2*>(o - PB + 2);
         }
+        const double2 rgA = recip_for_pass(ghA);
         BWD_ONE(a2, g2, s2, ghA.y, rgA.y, fA.y, oA.y, ob0)
         const double v1 = v;
         BWD_ONE(akA.y, GA.y, stA.y, ghA.x, rgA.x, fA.x, oA.x, oA.y)
@@ -1084,8 +1095,8 @@ __device__ __forceinline__ bool bwd_run(const double* __restrict__ p, const doub
     return false;
 }
 
-// backward first sweep of one warp (see fwd_sweep_tma).  The stage holds six planes: |kappa|, G, the static limit (field 2,
-// or the override array), gh, its reciprocal, and the forward velocities.  rec_w / vf_w / sb_w: block row 0 at the warp's
+// backward first sweep of one warp (see fwd_sweep_tma).  The stage holds five planes: |kappa|, G, the static limit (field 2,
+// or the override array), gh, and the forward velocities; the reciprocals of gh are made when the stage lands.  rec_w / vf_w / sb_w: block row 0 at the warp's
 // LOWEST column; lc: this lane's column minus that one; o: sample lo of the final velocities (sample order).
 template <int NT>
 __device__ __forceinline__ void bwd_sweep_tma(const WarpRing& R, const double* __restrict__ rec_w, const double* __restrict__ vf_w,
@@ -1110,7 +1121,7 @@ __device__ __forceinline__ void bwd_sweep_tma(const WarpRing& R, const double* _
     double tak = top_ak, tG = top_G, tst = top_st;   // terms of sample e+1
 #define BWD_T(ROW_)                                                                                                  \
         {                                                                                                            \
-            const double gh_ = S[3 * PD + ROW_], rg_ = S[4 * PD + ROW_], f_ = S[5 * PD + ROW_];                       \
+            const double gh_ = gh[ROW_], rg_ = rg[ROW_], f_ = S[4 * PD + ROW_];                                     \
             if (e + 1 == nb_next) { acc = s_acc[j]; j--; nb_next = (j >= 0) ? s_bi[j] : -1; }                         \
             const double vup = v;                                                                                    \
             v = bwd_step(tak, gh_, rg_, tst, pymin(f_, tG), v, sq, acc, hw, dd);                                     \
@@ -1124,8 +1135,13 @@ __device__ __forceinline__ void bwd_sweep_tma(const WarpRing& R, const double* _
         const int rb = nbw - 1 - it;                 // block row
         const int s = it & 1;
         mbar_wait(R.bar + 8 * s, (it >> 1) & 1);
-        const double* S = R.stage + (size_t)s * 6 * PD + lc * PB;
-        VAP_CHECK(7, lc >= 0 && lc < 32 && (unsigned)__cvta_generic_to_shared(S + 5 * PD + 3) + 8 <= R.smem_hi);
+        const double* S = R.stage + (size_t)s * 5 * PD + lc * PB;
+        VAP_CHECK(7, lc >= 0 && lc < 32 && (unsigned)__cvta_generic_to_shared(S + 4 * PD + 3) + 8 <= R.smem_hi);
+        double gh[PB], rg[PB];
+#pragma unroll
+        for (int r = 0; r < PB; r++) gh[r] = S[3 * PD + r];
+#pragma unroll
+        for (int r = 0; r < PB; r++) rg[r] = recip_for_pass(gh[r]);
         if (rb < nfull) {                            // a whole block of this lane's chunk: rows 3 .. 0
             o -= PB;
             BWD_T(3)
@@ -1211,24 +1227,24 @@ __global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_bwd_chunked(
     const int col = active ? nch - 1 - k : 0;                      // column (forward chunk index)
     const int lo = col * Lc;
     const int len = (lo + Lc < steps) ? Lc : steps - lo;
-    const double* P = rec + (size_t)b * RS * 5;
+    const double* P = rec + (size_t)b * RS * 4;
     const double* vf = vfT + (size_t)b * RS;
     const double hw = cons[b * 6 + 5] * 0.5;
     // with max_acceleration overrides the static limit of this pass is in statB (slot order, written by the pre-pass)
     const bool ovr = pass_has_override(max_accels + (size_t)b * E_cap, n_ev[2 * b], cons[b * 6 + 1]) != 0;
     const double* SB = statB + (size_t)b * RS;
-    // every warp owns a two-stage ring (6 planes of 1 KB per stage) and two mbarriers behind the tables
+    // every warp owns a two-stage ring (5 planes of 1 KB per stage) and two mbarriers behind the tables
     WarpRing R;
     constexpr int WARPS = (NT + 31) / 32;
     const int w = k >> 5;
-    R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 6 * TMA_PLANE_DOUBLES;
-    R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 6 * TMA_PLANE_DOUBLES * 8 + 16 * w);
-    R.planes = 6;
+    R.stage = reinterpret_cast<double*>(s_mem + ring_off) + (size_t)w * 2 * 5 * TMA_PLANE_DOUBLES;
+    R.bar = (unsigned)__cvta_generic_to_shared(s_mem + ring_off + (size_t)WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8 + 16 * w);
+    R.planes = 5;
     R.bytes = (NT < 32 ? NT : 32) * PB * 8;
 #ifdef VAP_BOUNDS_CHECK
-    R.rec_lo = P; R.rec_hi = P + 5 * RS; R.x_lo = vf; R.x_hi = vf + RS;
+    R.rec_lo = P; R.rec_hi = P + 4 * RS; R.x_lo = vf; R.x_hi = vf + RS;
     R.smem_lo = (unsigned)__cvta_generic_to_shared(s_mem + ring_off);
-    R.smem_hi = R.smem_lo + WARPS * 2 * 6 * TMA_PLANE_DOUBLES * 8;
+    R.smem_hi = R.smem_lo + WARPS * 2 * 5 * TMA_PLANE_DOUBLES * 8;
     R.bar_hi = R.smem_hi + 16 * WARPS;
 #endif
     if ((k & 31) == 0) { mbar_init(R.bar, 1); mbar_init(R.bar + 8, 1); fence_mbar_init(); }
@@ -1236,7 +1252,7 @@ __global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_bwd_chunked(
 
     auto rec_of = [&](int x, int fld) {                             // field fld (0-2) of sample x
         if (fld == 2 && ovr) return __ldg(SB + (x >= steps ? (int)(RS - 1) : edge_slot(x, Lc, NT)));
-        if (x >= steps) return __ldg(P + 5 * RS - 3 + fld);
+        if (x >= steps) return __ldg(P + 4 * RS - 3 + fld);
         const int cx = x / Lc, rx = x - cx * Lc;
         return __ldg(P + rec_index(rx, fld, cx, NT));
     };
@@ -1279,7 +1295,7 @@ __global__ void __maxnreg__(VAP_PASS_REGS_TMA) k_bwd_chunked(
                 }
             }
             s_usev[k] = v; s_usew[k] = sq;
-            VAP_CHECK(5, col >= 0 && col * PB + PB <= PB * NT && (size_t)(((len + 3) >> 2) + 1) * 5 * PB * NT <= (size_t)(5 * RS - 3) &&
+            VAP_CHECK(5, col >= 0 && col * PB + PB <= PB * NT && (size_t)(((len + 3) >> 2) + 1) * 4 * PB * NT <= (size_t)(4 * RS - 3) &&
                              (size_t)(((len + 3) >> 2) + 1) * PB * NT <= (size_t)(RS - 1) && A.o + len <= vo + D - 1 &&
                              lo + len <= steps && D <= D_cap);
         }

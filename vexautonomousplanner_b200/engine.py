@@ -329,7 +329,7 @@ class Engine:
         scr = self._empty((nscr,), torch.int32)
         chunks = self.chunks if D_cap <= 65536 else 256
         RS = int(self.lib.vap_pass_row_slots(C.c_int64(D_cap), C.c_int(chunks)))     # chunk-interleaved rows of the pass arrays
-        rec = self._empty((B, RS, 5)); statB = self._empty((B, RS))
+        rec = self._empty((B, RS, 4)); statB = self._empty((B, RS))
         vel_f = self._empty((B, RS)); vel = outs["vel"] if outs else self._empty((B, D_cap))
         t_est = self._empty((B,), torch.float32)
         rounds = torch.zeros((B, 2), dtype=torch.int32, device=self.device)
