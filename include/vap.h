@@ -298,8 +298,9 @@ int vap_export_rows(int64_t B, int64_t T_cap, int64_t out_plane_stride, const do
  *   vap_format_doubles: n values -> 32-byte NUL-padded slots out32[n][32] + lens[n].
  *   vap_format_rows: export rows[R][7] -> one line per row ("0 t x y heading v omega \n", every value followed by a
  *     blank) in slots[R][vap_row_text_stride()] + lens[R]; kinds[R] (u8 bit set from vap_row_kinds, may be NULL) prints
- *     the columns that hold a Python int in the reference as "0" instead of "0.0".  vap_compact_rows then gathers the
- *     lines at offsets[R] (exclusive prefix sum of lens, i64) into one contiguous text buffer.
+ *     the columns that hold a Python int in the reference as "0" instead of "0.0".  vap_compact_rows then copies line r
+ *     to text + offsets[r] (offsets[R] i64: the byte position of line r; the exclusive prefix sum of lens gives one
+ *     contiguous text buffer, the line_dst of vap_splice_plan leaves the gaps for the action rows).
  *   vap_row_kinds: per result row of every path, which entries of generate_motion_profile's lists are Python ints
  *     (motion_profile_generator.py:425, 448-453, 459-476, 487-518, 548-553): bit 1 times[r] (row 0 without a prologue),
  *     bit 2 linear_vels / accelerations (inserted turn / wait rows), bit 4 angular_vels (wait rows, first turn row),
@@ -313,6 +314,32 @@ int vap_format_doubles(int64_t n, const double* x, char* out32, int32_t* lens, v
 int vap_row_text_stride(void);
 int vap_format_rows(int64_t R, const double* rows, const uint8_t* kinds, char* slots, int32_t* lens, void* stream);
 int vap_compact_rows(int64_t R, const char* slots, const int32_t* lens, const int64_t* offsets, char* text, void* stream);
+
+/* "Next" row f1, the whole .txt body of every path (save_nodes_to_file, gui_manager.py:284-316): the path's trajectory
+ * lines with the action rows inserted as the reference does it, list.insert(nodes_map[i] + i, row) for i < n_maps[b][0],
+ * then list.insert(actions_map[j] + j, row) for j < n_maps[b][1] (Python's clamping: an index past the end appends, a
+ * negative one counts from the end and stops at 0; the action-point indices do not count the node rows before them).
+ *   vap_splice_plan: the lines of path b are the dense rows row_offsets[b] .. row_offsets[b+1] of vap_export_rows;
+ *     line_offsets[R+1] (i64) = exclusive prefix sum of the line lengths of vap_format_rows (R = row_offsets[B]).  The
+ *     action rows are caller text (the host formats [1, *action_values] with f"{v} "): act_text[act_off[i] .. act_off[i+1])
+ *     is row i of n_act, act_off[n_act+1] i64; the rows of path b start at act_first[b] (i64), its act_rows[b][0] node
+ *     rows first, then its act_rows[b][1] action-point rows.  nodes_map / actions_map / n_maps as vap_time_profile writes
+ *     them (rows of N_max + 1 and max(A_max, 1) entries).
+ *     Outputs: path_offsets[B+1] (i64): path b's body is text[path_offsets[b] .. path_offsets[b+1]); line_dst[R] (i64): byte
+ *     position of every trajectory line, for vap_compact_rows; act_dst[n_act] (i64): byte position of every action row,
+ *     -1 for rows that are in no body; flags[B] (i32): 0 assembled, 1 status[b] != 0 (no action rows; vap_export_rows
+ *     gives such a path no lines either, so its body is empty), 2 the maps need more
+ *     rows than act_rows passes (or n_maps exceeds the map rows): nothing of the action rows is read, the body holds
+ *     the trajectory lines only.  Read path_offsets[B] back to size `text`.  Shared memory per path:
+ *     32 * (N_max + 1 + max(A_max, 1)) bytes.
+ *   vap_splice_actions: copies row i of act_text to text + act_dst[i] (after vap_compact_rows with line_dst, or before).  */
+int vap_splice_plan(int64_t B, int N_max, int A_max, const int32_t* status, const int32_t* nodes_map,
+                    const int32_t* actions_map, const int32_t* n_maps, const int64_t* row_offsets,
+                    const int64_t* line_offsets, const int64_t* act_first, const int32_t* act_rows, int64_t n_act,
+                    const int64_t* act_off, int64_t* path_offsets, int64_t* line_dst, int64_t* act_dst, int32_t* flags,
+                    void* stream);
+int vap_splice_actions(int64_t n_act, const char* act_text, const int64_t* act_off, const int64_t* act_dst, char* text,
+                       void* stream);
 
 /* Bounds diagnostics of a -DVAP_BOUNDS_CHECK build (profiles/tools/bounds_check.py; compute-sanitizer is closed on the GPU
  * pool this was developed on): out_host[32] (HOST memory) = violations per check site (0..15) and checks executed per site

@@ -24,7 +24,7 @@ SYMBOLS = [
     "vap_lut_index_row_ints", "vap_build_lut_index", "vap_build_props", "vap_query_tables", "vap_build_dgrid", "vap_dist_sample", "vap_fwd_bwd", "vap_resample",
     "vap_gl", "vap_turn_profile", "vap_lerp", "vap_wheel_trajectory",
     "vap_event_scratch_ints", "vap_pass_row_slots", "vap_velocity_profile", "vap_time_profile", "vap_workspace_bytes", "vap_profile_batch", "vap_summary", "vap_pack_rows", "vap_export_rows", "vap_format_doubles", "vap_row_text_stride",
-    "vap_format_rows", "vap_compact_rows", "vap_row_kinds", "vap_bench_dfma", "vap_test_div_const", "vap_test_div_recip", "vap_build_lerp_recip", "vap_diag_read",
+    "vap_format_rows", "vap_compact_rows", "vap_splice_plan", "vap_splice_actions", "vap_row_kinds", "vap_bench_dfma", "vap_test_div_const", "vap_test_div_recip", "vap_build_lerp_recip", "vap_diag_read",
 ]
 
 _lib = None

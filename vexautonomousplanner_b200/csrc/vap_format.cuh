@@ -234,4 +234,141 @@ __global__ void __launch_bounds__(256) k_compact_rows(long long R, const char* _
     int n = lens[r];
     for (int k = lane; k < n; k += 32) d[k] = s[k];
 }
+
+// ---- The .txt body of every path: trajectory lines with the action rows spliced in (gui_manager.py:297-310) ----------
+// The reference starts from the path's trajectory lines and calls list.insert(nodes_map[i] + i, row) for the node rows,
+// then list.insert(actions_map[j] + j, row) for the action-point rows.  Inserted row j ends at a final position P_j; with
+// the P_j sorted, Q_j = P_j - j never decreases and trajectory line k has exactly #{j : Q_j <= k} inserted rows in front
+// of it.  So one warp per path replays the <= N_max + 1 + A_max inserts on the positions alone (shared memory), ranks
+// them, and writes the byte position of every inserted row and every trajectory line; k_compact_rows and
+// k_splice_actions then copy the bytes.  Action rows of path b: act_first[b] .. + act_rows[b][0] node rows, then
+// act_rows[b][1] action-point rows; row i is act_text[act_off[i] .. act_off[i+1]).
+#define SPLICE_OK 0
+#define SPLICE_FAILED 1       // status != 0: no action rows (and no lines from vap_export_rows: zero bytes)
+#define SPLICE_SHORT 2        // the maps need more action rows than were passed: the body holds the trajectory lines only
+
+// bytes of path b's body and its flag
+__device__ __forceinline__ long long splice_path_bytes(long long b, int N_max, int A_stride, const int* __restrict__ status,
+                                                       const int* __restrict__ n_maps, const long long* __restrict__ row_off,
+                                                       const long long* __restrict__ line_off,
+                                                       const long long* __restrict__ act_first, const int* __restrict__ act_rows,
+                                                       long long n_act, const long long* __restrict__ act_off, int& flag)
+{
+    const long long lines = line_off[row_off[b + 1]] - line_off[row_off[b]];
+    if (status[b] != 0) { flag = SPLICE_FAILED; return lines; }   // vap_export_rows gives such a path no lines
+    const int nm = n_maps[2 * b], am = n_maps[2 * b + 1];
+    const long long n0 = act_rows[2 * b], n1 = act_rows[2 * b + 1], a0 = act_first[b];
+    if (nm < 0 || am < 0 || nm > N_max + 1 || am > A_stride || n0 < 0 || n1 < 0 || nm > n0 || am > n1 || a0 < 0 ||
+        a0 + n0 + n1 > n_act) { flag = SPLICE_SHORT; return lines; }
+    flag = SPLICE_OK;
+    return lines + (act_off[a0 + nm] - act_off[a0]) + (act_off[a0 + n0 + am] - act_off[a0 + n0]);
+}
+
+// path_offsets[B+1] = exclusive scan of the body sizes (one block, as k_row_offsets), flags[B]
+__global__ void __launch_bounds__(1024) k_splice_offsets(long long B, int N_max, int A_stride, const int* __restrict__ status,
+                                                         const int* __restrict__ n_maps, const long long* __restrict__ row_off,
+                                                         const long long* __restrict__ line_off,
+                                                         const long long* __restrict__ act_first,
+                                                         const int* __restrict__ act_rows, long long n_act,
+                                                         const long long* __restrict__ act_off,
+                                                         long long* __restrict__ path_off, int* __restrict__ flags)
+{
+    __shared__ long long s_part[1024];
+    const int t = threadIdx.x, NT = blockDim.x;
+    const long long per = (B + NT - 1) / NT;
+    const long long lo = (long long)t * per, hi = (lo + per < B) ? lo + per : B;
+    long long sum = 0;
+    int f;
+    for (long long b = lo; b < hi; b++)
+        sum += splice_path_bytes(b, N_max, A_stride, status, n_maps, row_off, line_off, act_first, act_rows, n_act, act_off, f);
+    s_part[t] = sum;
+    __syncthreads();
+    if (t == 0) {
+        long long acc = 0;
+        for (int k = 0; k < NT; k++) { long long v = s_part[k]; s_part[k] = acc; acc += v; }
+        path_off[B] = acc;
+    }
+    __syncthreads();
+    long long acc = s_part[t];
+    for (long long b = lo; b < hi; b++) {
+        path_off[b] = acc;
+        acc += splice_path_bytes(b, N_max, A_stride, status, n_maps, row_off, line_off, act_first, act_rows, n_act, act_off, f);
+        flags[b] = f;
+    }
+}
+
+// One warp per path.  Shared memory per warp: four arrays of M_cap = N_max + 1 + A_stride entries.
+__global__ void __launch_bounds__(128) k_splice_plan(long long B, int N_max, int A_stride, const int* __restrict__ nodes_map,
+                                                     const int* __restrict__ actions_map, const int* __restrict__ n_maps,
+                                                     const long long* __restrict__ row_off, const long long* __restrict__ line_off,
+                                                     const long long* __restrict__ act_first, const int* __restrict__ act_rows,
+                                                     const long long* __restrict__ act_off, const long long* __restrict__ path_off,
+                                                     const int* __restrict__ flags, long long* __restrict__ line_dst,
+                                                     long long* __restrict__ act_dst)
+{
+    extern __shared__ long long s_splice[];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const long long b = (long long)blockIdx.x * (blockDim.x >> 5) + w;
+    if (b >= B) return;
+    const int M_cap = N_max + 1 + A_stride;
+    long long* pos = s_splice + (size_t)w * 4 * M_cap;    // final position of inserted row j (insert order)
+    long long* len = pos + M_cap;                          // its bytes
+    long long* sQ = len + M_cap;                           // Q of the inserted rows in final order
+    long long* sC = sQ + M_cap;                            // inclusive byte sum of the inserted rows in final order
+    const long long r0 = row_off[b], n_lines = row_off[b + 1] - r0, L0 = line_off[r0], base = path_off[b];
+    const int flag = flags[b];
+    if (flag != SPLICE_OK) {                               // status != 0 has no lines; a short path keeps its lines only
+        for (long long k = lane; k < n_lines; k += 32) line_dst[r0 + k] = base + line_off[r0 + k] - L0;
+        return;
+    }
+    const int nm = n_maps[2 * b], am = n_maps[2 * b + 1], M = nm + am;
+    const long long a0 = act_first[b], ap0 = a0 + act_rows[2 * b];
+    const int* nmap = nodes_map + (size_t)b * (N_max + 1);
+    const int* amap = actions_map + (size_t)b * A_stride;
+    for (int j = lane; j < M; j += 32) {
+        const long long ri = j < nm ? a0 + j : ap0 + (j - nm);
+        len[j] = act_off[ri + 1] - act_off[ri];
+    }
+    for (int j = 0; j < M; j++) {                          // list.insert(idx, row) on a list of n_lines + j entries
+        long long idx = j < nm ? (long long)nmap[j] + j : (long long)amap[j - nm] + (j - nm);
+        const long long cur = n_lines + j;
+        if (idx < 0) { idx += cur; if (idx < 0) idx = 0; }
+        if (idx > cur) idx = cur;
+        for (int i = lane; i < j; i += 32) if (pos[i] >= idx) pos[i]++;
+        __syncwarp();
+        if (lane == 0) pos[j] = idx;
+        __syncwarp();
+    }
+    for (int j = lane; j < M; j += 32) {
+        const long long p = pos[j];
+        long long rank = 0, before = 0;
+        for (int i = 0; i < M; i++) if (pos[i] < p) { rank++; before += len[i]; }
+        const long long q = p - rank;                      // trajectory lines in front of the row
+        const long long ri = j < nm ? a0 + j : ap0 + (j - nm);
+        act_dst[ri] = base + (line_off[r0 + q] - L0) + before;
+        sQ[rank] = q;
+        sC[rank] = before + len[j];
+    }
+    __syncwarp();
+    for (long long k = lane; k < n_lines; k += 32) {
+        int lo = 0, hi = M;                                // first rank with Q > k
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (sQ[mid] <= k) lo = mid + 1; else hi = mid; }
+        line_dst[r0 + k] = base + (line_off[r0 + k] - L0) + (lo > 0 ? sC[lo - 1] : 0);
+    }
+}
+
+// the inserted rows into their gaps (one warp per row; rows with act_dst < 0 are not part of any body)
+__global__ void __launch_bounds__(256) k_splice_actions(long long n_act, const char* __restrict__ act_text,
+                                                        const long long* __restrict__ act_off,
+                                                        const long long* __restrict__ act_dst, char* __restrict__ text)
+{
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (i >= n_act) return;
+    const long long d = act_dst[i];
+    if (d < 0) return;
+    const char* s = act_text + act_off[i];
+    const long long n = act_off[i + 1] - act_off[i];
+    for (long long k = lane; k < n; k += 32) text[d + k] = s[k];
+}
 #endif  // VAP_FORMAT_HOST_TEST

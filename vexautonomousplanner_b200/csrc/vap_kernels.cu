@@ -1633,6 +1633,57 @@ extern "C" int vap_compact_rows(int64_t R, const char* slots, const int32_t* len
     return 0;
 }
 
+extern "C" int vap_splice_plan(int64_t B, int N_max, int A_max, const int32_t* status, const int32_t* nodes_map,
+                               const int32_t* actions_map, const int32_t* n_maps, const int64_t* row_offsets,
+                               const int64_t* line_offsets, const int64_t* act_first, const int32_t* act_rows, int64_t n_act,
+                               const int64_t* act_off, int64_t* path_offsets, int64_t* line_dst, int64_t* act_dst,
+                               int32_t* flags, void* stream)
+{
+    if (B <= 0) return 0;
+    if (N_max < 1 || A_max < 0 || n_act < 0) return arg_err("vap_splice_plan: N_max >= 1, A_max >= 0 and n_act >= 0 required");
+    const int A_stride = A_max > 0 ? A_max : 1;
+    const size_t warp_bytes = (size_t)4 * sizeof(long long) * (size_t)(N_max + 1 + A_stride);
+    int max_smem = 0, dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e != cudaSuccess) return set_err("vap_splice_plan/attr", e);
+    if (warp_bytes > (size_t)max_smem) return arg_err("vap_splice_plan: N_max + A_max too large for one warp's shared memory");
+    int warps = 4;
+    while (warps > 1 && warps * warp_bytes > 48 * 1024) warps >>= 1;
+    const size_t smem = warps * warp_bytes;
+    if (smem > 48 * 1024) {
+        e = cudaFuncSetAttribute(k_splice_plan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_err("vap_splice_plan/attr", e);
+    }
+    if (n_act > 0) {
+        e = cudaMemsetAsync(act_dst, 0xff, (size_t)n_act * sizeof(int64_t), STREAM);     // -1: the row is in no body
+        if (e != cudaSuccess) return set_err("vap_splice_plan/memset", e);
+    }
+    const long long* ro = reinterpret_cast<const long long*>(row_offsets);
+    const long long* lo = reinterpret_cast<const long long*>(line_offsets);
+    const long long* af = reinterpret_cast<const long long*>(act_first);
+    const long long* ao = reinterpret_cast<const long long*>(act_off);
+    long long* po = reinterpret_cast<long long*>(path_offsets);
+    k_splice_offsets<<<1, 1024, 0, STREAM>>>(B, N_max, A_stride, status, n_maps, ro, lo, af, act_rows, n_act, ao, po, flags);
+    CHECK_LAUNCH("vap_splice_plan/offsets");
+    k_splice_plan<<<blocks_for(B, warps), warps * 32, smem, STREAM>>>(B, N_max, A_stride, nodes_map, actions_map, n_maps, ro, lo,
+                                                                     af, act_rows, ao, po, flags,
+                                                                     reinterpret_cast<long long*>(line_dst),
+                                                                     reinterpret_cast<long long*>(act_dst));
+    CHECK_LAUNCH("vap_splice_plan");
+    return 0;
+}
+
+extern "C" int vap_splice_actions(int64_t n_act, const char* act_text, const int64_t* act_off, const int64_t* act_dst,
+                                  char* text, void* stream)
+{
+    if (n_act <= 0) return 0;
+    k_splice_actions<<<blocks_for(n_act * 32, 256), 256, 0, STREAM>>>(n_act, act_text, reinterpret_cast<const long long*>(act_off),
+                                                                     reinterpret_cast<const long long*>(act_dst), text);
+    CHECK_LAUNCH("vap_splice_actions");
+    return 0;
+}
+
 // =====================================================================================================
 // The whole hot path behind ONE call (SURVEY.md 8b): generate_motion_profile(spline_manager, constraints)
 // (motion_profile_generator.py:389-628, incl. build_path and rebuild_tables) for a batch, out of one caller workspace.

@@ -3,7 +3,8 @@
 f1  trajectory export (gui_manager.py:220-230, 284-316): rows [0, t, x*12, -y*12, heading, v*12, omega] per time sample
     (built on the device, vap_export_rows), action rows [1, *action_values] spliced at nodes_map[i] + i and
     actions_map[i] + i, text written as f"{v} " per value -- the same formatting expression as the reference, so the
-    text is identical for identical numbers.
+    text is identical for identical numbers.  trajectory_text builds one path's .txt body, save_text_batch every
+    path's at once on the device (the command save_routes re-saves a folder of routes with it).
 f2  node JSON codec (gui_manager.py:388-427, gui/path.py:590-644): [[x_in, y_in, start, end, reverse, stop, turn, wait,
     tangent, in_mag, out_mag, *actions], ...], [[x_in, y_in, t, stop, wait, *actions], ...] with the inch <-> pixel <->
     foot conversions of the GUI (145.308474301 in, 12.1090395251 ft per 2000 px).
@@ -42,19 +43,27 @@ def format_rows_device(eng: Engine, rows: torch.Tensor, int_time: Optional[torch
     kinds of row_kinds() (bit 1 alone = "the time prints as the int 0").
     Returns (text uint8[total], row_offsets int64[R+1]); line r is text[row_offsets[r]:row_offsets[r+1]]."""
     R = rows.shape[0]
-    stride = int(eng.lib.vap_row_text_stride())
-    slots = torch.empty((max(R, 1), stride), dtype=torch.uint8, device=eng.device)
-    lens = torch.zeros(max(R, 1), dtype=torch.int32, device=eng.device)
-    _lib.check(eng.lib.vap_format_rows(C.c_int64(R), _p(rows), _p(int_time), _p(slots), _p(lens), eng._stream()),
-               "vap_format_rows")
-    offsets = torch.zeros(R + 1, dtype=torch.int64, device=eng.device)
-    torch.cumsum(lens[:R], dim=0, out=offsets[1:])                 # plumbing: exclusive scan of the line lengths
+    slots, lens, offsets = _format_slots(eng, rows, int_time)
     total = int(offsets[R].item())
     text = torch.empty(max(total, 1), dtype=torch.uint8, device=eng.device)
     _lib.check(eng.lib.vap_compact_rows(C.c_int64(R), _p(slots), _p(lens), _p(offsets), _p(text), eng._stream()),
                "vap_compact_rows")
-    eng.launches += 2
+    eng.launches += 1
     return text[:total], offsets
+
+
+def _format_slots(eng: Engine, rows: torch.Tensor, kinds: Optional[torch.Tensor]):
+    """vap_format_rows: (slots[R, stride], lens[R], offsets[R+1] = exclusive scan of lens), nothing read back."""
+    R = rows.shape[0]
+    stride = int(eng.lib.vap_row_text_stride())
+    slots = torch.empty((max(R, 1), stride), dtype=torch.uint8, device=eng.device)
+    lens = torch.zeros(max(R, 1), dtype=torch.int32, device=eng.device)
+    _lib.check(eng.lib.vap_format_rows(C.c_int64(R), _p(rows), _p(kinds), _p(slots), _p(lens), eng._stream()),
+               "vap_format_rows")
+    eng.launches += 1
+    offsets = torch.zeros(R + 1, dtype=torch.int64, device=eng.device)
+    torch.cumsum(lens[:R], dim=0, out=offsets[1:])                 # plumbing: exclusive scan of the line lengths
+    return slots, lens, offsets
 
 
 RK_TIME_INT, RK_INSERTED, RK_OMEGA_INT, RK_POS_INT = 1, 2, 4, 8
@@ -141,6 +150,112 @@ def trajectory_text(eng: Engine, res: ProfileResult, b: int, node_actions: Seque
     for i in range(len(am)):
         lines.insert(int(am[i] / 1) + i, format_rows([[1] + list(action_rows[i])]))
     return "".join(lines)
+
+
+_CACHED_TYPES = (int, bool, str)      # f"{v}" of these depends on the value alone (unlike 0.0 == -0.0, 1 == 1.0 == True)
+
+
+def pack_action_rows(node_actions: Sequence[Sequence[Sequence]], ap_actions: Sequence[Sequence[Sequence]]):
+    """Text of every action row [1, *action_values] of a batch as format_rows writes it, laid out for vap_splice_plan.
+    node_actions[b][i] / ap_actions[b][j]: the action_values of path b's nodes / action points.
+    Returns (text uint8[n], act_off int64[rows+1], act_first int64[B], act_rows int32[B, 2]); the rows of path b start at
+    act_first[b], its node rows first.  A row of plain ints / bools / strings is formatted once per batch."""
+    B = len(node_actions)
+    if len(ap_actions) != B:
+        raise ValueError(f"node_actions has {B} paths, ap_actions {len(ap_actions)}")
+    cache, pieces = {}, []
+    act_rows = np.zeros((B, 2), dtype=np.int32)
+    for b in range(B):
+        na, aa = node_actions[b], ap_actions[b]
+        act_rows[b] = len(na), len(aa)
+        for v in (*na, *aa):
+            vals = tuple(v)
+            try:
+                key = (tuple(map(type, vals)), vals)
+                s = cache.get(key)
+            except TypeError:                              # unhashable values: format every time
+                key, s = None, None
+            if s is None:
+                s = format_rows([(1, *vals)]).encode()
+                if key is not None and all(t in _CACHED_TYPES for t in key[0]):
+                    cache[key] = s
+            pieces.append(s)
+    act_off = np.zeros(len(pieces) + 1, dtype=np.int64)
+    np.cumsum(np.fromiter(map(len, pieces), dtype=np.int64, count=len(pieces)), out=act_off[1:])
+    act_first = np.zeros(B, dtype=np.int64)
+    np.cumsum(act_rows.sum(axis=1, dtype=np.int64)[:-1], out=act_first[1:])
+    return np.frombuffer(bytearray(b"".join(pieces)), dtype=np.uint8), act_off, act_first, act_rows
+
+
+def splice_bodies(eng: Engine, slots: torch.Tensor, lens: torch.Tensor, line_off: torch.Tensor, row_off: torch.Tensor,
+                  status: torch.Tensor, nodes_map: torch.Tensor, actions_map: torch.Tensor, n_maps: torch.Tensor,
+                  node_actions: Sequence[Sequence[Sequence]], ap_actions: Sequence[Sequence[Sequence]]):
+    """The .txt bodies of B paths from their formatted trajectory lines (vap_format_rows: slots, lens, line_off = exclusive
+    scan of lens; path b owns lines row_off[b] .. row_off[b+1]) and the maps of the time stage: vap_splice_plan,
+    vap_compact_rows onto the gapped line positions, vap_splice_actions, one copy to pinned host memory.
+    Returns (text uint8[total] host, path_offsets int64[B+1] host, ok bool[B] host).  Raises ValueError when a path's maps
+    need more action rows than node_actions / ap_actions give it."""
+    B, R = status.shape[0], line_off.shape[0] - 1
+    dev = eng.device
+    text_h, act_off_h, act_first_h, act_rows_h = pack_action_rows(node_actions, ap_actions)
+    n_act = act_off_h.shape[0] - 1
+
+    def up(a):
+        return torch.from_numpy(a if a.size else np.zeros(1, dtype=a.dtype)).to(dev, non_blocking=True)
+    act_text, act_off, act_first, act_rows = up(text_h), up(act_off_h), up(act_first_h), up(act_rows_h)
+    path_off = torch.zeros(B + 1, dtype=torch.int64, device=dev)
+    line_dst = torch.empty(max(R, 1), dtype=torch.int64, device=dev)
+    act_dst = torch.empty(max(n_act, 1), dtype=torch.int64, device=dev)
+    flags = torch.zeros(max(B, 1), dtype=torch.int32, device=dev)
+    N_max, A_stride = nodes_map.shape[1] - 1, actions_map.shape[1]
+    with eng._stage("text_splice_plan"):
+        _lib.check(eng.lib.vap_splice_plan(C.c_int64(B), C.c_int(N_max), C.c_int(A_stride), _p(status), _p(nodes_map),
+                                           _p(actions_map), _p(n_maps), _p(row_off), _p(line_off), _p(act_first),
+                                           _p(act_rows), C.c_int64(n_act), _p(act_off), _p(path_off), _p(line_dst),
+                                           _p(act_dst), _p(flags), eng._stream()), "vap_splice_plan")
+    eng.launches += 2
+    flags = flags[:B]
+    head = torch.stack([path_off[B], (flags == 2).sum()]).cpu()          # the one read-back: size of the text
+    if int(head[1]):
+        bad = torch.nonzero(flags == 2).flatten()[:8].tolist()
+        raise ValueError(f"{int(head[1])} path(s) need more action rows than were passed (first: {bad}); node_actions[b] "
+                         "must cover n_maps[b, 0] rows and ap_actions[b] n_maps[b, 1]")
+    total = int(head[0])
+    text = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
+    with eng._stage("text_splice_copy"):
+        _lib.check(eng.lib.vap_compact_rows(C.c_int64(R), _p(slots), _p(lens), _p(line_dst), _p(text), eng._stream()),
+                   "vap_compact_rows")
+        _lib.check(eng.lib.vap_splice_actions(C.c_int64(n_act), _p(act_text), _p(act_off), _p(act_dst), _p(text),
+                                              eng._stream()), "vap_splice_actions")
+    eng.launches += 2
+    host = torch.empty(max(total, 1), dtype=torch.uint8, pin_memory=True)
+    offs = torch.empty(B + 1, dtype=torch.int64, pin_memory=True)
+    ok = torch.empty(max(B, 1), dtype=torch.bool, pin_memory=True)
+    with eng._stage("text_d2h"):
+        host.copy_(text, non_blocking=True)
+    offs.copy_(path_off, non_blocking=True)
+    ok[:B].copy_(flags == 0, non_blocking=True)
+    torch.cuda.current_stream(dev).synchronize()
+    return host.numpy()[:total], offs.numpy(), ok.numpy()[:B]
+
+
+def save_text_batch(eng: Engine, res: ProfileResult, db, node_actions: Sequence[Sequence[Sequence]],
+                    ap_actions: Sequence[Sequence[Sequence]]):
+    """The .txt body save_nodes_to_file writes (gui_manager.py:232-316) for every path of a batch, assembled on the device.
+    node_actions[b][i] / ap_actions[b][j]: the action_values of path b's nodes (widget list order) and action points, as
+    trajectory_text takes them for one path.  db: the DeviceBatch res was profiled from.
+    Returns (text, path_offsets, ok), all on the host: path b's body is text[path_offsets[b]:path_offsets[b+1]] (bytes,
+    equal to trajectory_text's for that path); ok[b] is False for a path with status != 0, whose body is empty.
+    Reads back from the device a fixed number of times, whatever B is.  Raises ValueError when a path's maps need more
+    action rows than were passed (the reference raises IndexError there)."""
+    if len(node_actions) != res.B or len(ap_actions) != res.B:
+        raise ValueError(f"{res.B} paths, but {len(node_actions)} node_actions and {len(ap_actions)} ap_actions")
+    with eng._stage("text_format"):
+        rows, poff = export_rows(eng, res)
+        kinds = row_kinds(eng, res, db, offsets=poff, n_rows=rows.shape[0])
+        slots, lens, line_off = _format_slots(eng, rows, kinds)
+    return splice_bodies(eng, slots, lens, line_off, poff, res.status, res.nodes_map, res.actions_map, res.n_maps,
+                         node_actions, ap_actions)
 
 
 ROUTES_DECL = "std::vector<std::vector<double>> "
