@@ -184,12 +184,6 @@ def same_bits(ref, got, rows=None):
     assert torch.equal(ref.actions_map[am], got.actions_map[am])
 
 
-def rows_of(db, lo, hi):
-    from vexautonomousplanner_b200.engine import DeviceBatch
-    return DeviceBatch(db.node_attr[lo:hi], db.node_flags[lo:hi], db.n_nodes[lo:hi], db.ap_attr[lo:hi], db.ap_flags[lo:hi],
-                       db.n_ap[lo:hi], db.cons[lo:hi], db.max_splines)
-
-
 def eager(packed):
     from vexautonomousplanner_b200.engine import Engine
     e = Engine("cuda:0")
@@ -256,16 +250,15 @@ def test_pipelined_replays_flag_exactly_the_paths_that_do_not_fit(ora):
     slot, st = pipe.graphs[pipe.n % 2], pipe.streams[pipe.n % 2]
     st.wait_stream(main)
     with torch.cuda.stream(st):
-        for name in ("node_attr", "node_flags", "n_nodes", "ap_attr", "ap_flags", "n_ap", "cons"):
-            getattr(slot.db, name).copy_(getattr(heavy_db, name), non_blocking=True)
+        slot.db.copy_(heavy_db)
     slots.append(slot)
     pipe.submit(None, consume)
     pipe.drain()
     torch.cuda.synchronize()
     assert len(snaps) == 4
     fresh = eng.upload(light_a)
-    for name in ("node_attr", "node_flags", "n_nodes", "ap_attr", "ap_flags", "n_ap", "cons"):
-        assert torch.equal(getattr(db_a, name), getattr(fresh, name)), name      # the caller's batch is not a slot's input
+    for name, a, b in zip(db_a.FIELDS, db_a.tensors(), fresh.tensors()):
+        assert torch.equal(a, b), name                      # the caller's batch is not a slot's input
     flagged_any = []
     for (name, p), slot, res in zip(order, slots, snaps):
         refs = oracle_refs(ora, name, p)
@@ -331,8 +324,8 @@ def test_replay_rejects_other_batch_shapes():
     first = snapshot(g.run())
     z = lambda *shape, dt=torch.float64: torch.zeros(shape, dtype=dt, device=db.node_attr.device)     # noqa: E731
     bad = {
-        "B=1": rows_of(db, 0, 1),
-        "B-1": rows_of(db, 0, B - 1),
+        "B=1": db.rows(0, 1),
+        "B-1": db.rows(0, B - 1),
         "N_max-1": replace(db, node_attr=db.node_attr[:, : N - 1], node_flags=db.node_flags[:, : N - 1]),
         "N_max=1": replace(db, node_attr=db.node_attr[:, :1], node_flags=db.node_flags[:, :1]),
         "A_max+1": replace(db, ap_attr=z(B, db.A_max + 1, 4), ap_flags=z(B, db.A_max + 1, dt=torch.int32)),

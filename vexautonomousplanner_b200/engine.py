@@ -26,6 +26,7 @@ ROW_LIMIT = 1.0e7      # more time samples than this per path: treated as a non-
 DIST_LIMIT = 5.0e7     # more distance samples than this per path (L / dd; an infinite length too): status -5
 _POISON = bool(int(os.environ.get("VAP_POISON", "0")))
 MAX_RETRIES = 2        # exact re-runs after a capacity overflow; a status that survives them is returned as it is
+PROFILE_BATCH_KERNELS = 18   # kernels of one vap_profile_batch call (besides one memset and one 24-byte device copy)
 
 
 def _p(t: Optional[torch.Tensor]):
@@ -35,6 +36,7 @@ def _p(t: Optional[torch.Tensor]):
 @dataclass
 class DeviceBatch:
     """PackedPaths resident on the device."""
+    FIELDS = ("node_attr", "node_flags", "n_nodes", "ap_attr", "ap_flags", "n_ap", "cons")   # the input tensors, in order
     node_attr: torch.Tensor
     node_flags: torch.Tensor
     n_nodes: torch.Tensor
@@ -56,13 +58,35 @@ class DeviceBatch:
     def A_max(self):
         return self.ap_attr.shape[1]
 
+    def tensors(self) -> list:
+        return [getattr(self, name) for name in self.FIELDS]
+
     @staticmethod
-    def from_packed(p: PackedPaths, device, pinned: Optional[dict] = None, non_blocking: bool = True) -> "DeviceBatch":
-        def up(a):
-            t = torch.from_numpy(a)
-            return t.to(device, non_blocking=non_blocking)
-        return DeviceBatch(up(p.node_attr), up(p.node_flags), up(p.n_nodes), up(p.ap_attr), up(p.ap_flags), up(p.n_ap),
-                           up(p.cons), p.max_splines())
+    def from_packed(p: PackedPaths, device, non_blocking: bool = True) -> "DeviceBatch":
+        return DeviceBatch(*(torch.from_numpy(getattr(p, name)).to(device, non_blocking=non_blocking)
+                             for name in DeviceBatch.FIELDS), p.max_splines())
+
+    def rows(self, lo: int, hi: int) -> "DeviceBatch":
+        """Paths lo..hi as views of these tensors."""
+        return DeviceBatch(*(t[lo:hi] for t in self.tensors()), self.max_splines)
+
+    def clone(self) -> "DeviceBatch":
+        return DeviceBatch(*(t.clone() for t in self.tensors()), self.max_splines)
+
+    def copy_(self, other, non_blocking: bool = True) -> None:
+        """Copy the inputs of `other` (a DeviceBatch of the same shape) into these tensors, on the current stream."""
+        for dst, src in zip(self.tensors(), other.tensors()):
+            dst.copy_(src, non_blocking=non_blocking)
+
+    def pinned(self) -> "DeviceBatch":
+        """Pinned host buffers of this batch's shape, for upload_()."""
+        return DeviceBatch(*(torch.empty(t.shape, dtype=t.dtype, pin_memory=True) for t in self.tensors()), self.max_splines)
+
+    def upload_(self, p: PackedPaths, pin: "DeviceBatch") -> None:
+        """Copy the host batch `p` into these tensors through the pinned buffers `pin` (from pinned())."""
+        for name, buf in zip(self.FIELDS, pin.tensors()):
+            buf.copy_(torch.from_numpy(getattr(p, name)))
+        self.copy_(pin)
 
 
 @dataclass
@@ -310,13 +334,13 @@ class Engine:
         return vel, ma, bidx, bval, n_ev, t_est
 
     def velocity_chunked(self, db: DeviceBatch, g: Geometry, t: Tables, status: torch.Tensor, D_cap: int, mode: int = 0,
-                         outs: Optional[dict] = None, want_t: bool = True):
+                         want_t: bool = True):
         """S3 + events + S4 + S5, fast path: sampling fused with the hoisted pre-pass (vap_velocity_profile), sample-parallel
         events, chunk-speculative passes.  want_t: also write t / kappa / theta per distance sample (inspection outputs)."""
         B = db.B
         E_cap = db.N_max + db.A_max + 2
         grid = self.dgrid(D_cap + 2)
-        n_samples = outs["n_samples"] if outs else self._empty((B,), torch.int32)
+        n_samples = self._empty((B,), torch.int32)
         tq = self._empty((B, D_cap)) if want_t else None      # t / kappa / theta per distance sample: inspection outputs
         kap = self._empty((B, D_cap)) if want_t else None
         th = self._empty((B, D_cap)) if want_t else None
@@ -330,7 +354,7 @@ class Engine:
         chunks = self.chunks if D_cap <= 65536 else 256
         RS = int(self.lib.vap_pass_row_slots(C.c_int64(D_cap), C.c_int(chunks)))     # chunk-interleaved rows of the pass arrays
         rec = self._empty((B, RS, 4)); statB = self._empty((B, RS))
-        vel_f = self._empty((B, RS)); vel = outs["vel"] if outs else self._empty((B, D_cap))
+        vel_f = self._empty((B, RS)); vel = self._empty((B, D_cap))
         t_est = self._empty((B,), torch.float32)
         rounds = torch.zeros((B, 2), dtype=torch.int32, device=self.device)
         inv = t.lut_inv if self.accelerators else None
@@ -391,24 +415,17 @@ class Engine:
             rows = torch.where(status == ST_OK, rows, torch.zeros_like(rows))
         return int(rows.max().item()) if rows.numel() else 0
 
-    def time_profile(self, db: DeviceBatch, g: Geometry, t: Tables, status, D_cap, n_samples, vel, T_cap,
-                     outs: Optional[dict] = None):
+    def time_profile(self, db: DeviceBatch, g: Geometry, t: Tables, status, D_cap, n_samples, vel, T_cap):
         """S6 + S7, fast path (vap_time_profile): state recurrence / parallel lookups / event replay / scatter."""
         B = db.B
         E_cap = db.N_max + db.A_max + 2
-        plane_stride = 0
-        if outs:
-            out, nodes_map, actions_map = outs["out"], outs["nodes_map"], outs["actions_map"]
-            n_maps, n_out, summary, n_main = outs["n_maps"], outs["n_out"], outs["summary"], outs["n_main"]
-            plane_stride = outs["plane_stride"]
-        else:
-            out = self._empty((8, B, T_cap))
-            nodes_map = self._empty((B, db.N_max + 1), torch.int32)
-            actions_map = self._empty((B, max(db.A_max, 1)), torch.int32)
-            n_maps = self._empty((B, 2), torch.int32)
-            n_out = self._empty((B,), torch.int32)
-            summary = self._empty((B, 5))
-            n_main = self._empty((B,), torch.int32)
+        out = self._empty((8, B, T_cap))
+        nodes_map = self._empty((B, db.N_max + 1), torch.int32)
+        actions_map = self._empty((B, max(db.A_max, 1)), torch.int32)
+        n_maps = self._empty((B, 2), torch.int32)
+        n_out = self._empty((B,), torch.int32)
+        summary = self._empty((B, 5))
+        n_main = self._empty((B,), torch.int32)
         rden = self.lerp_recip(D_cap + 2)
         stage = self._empty((8, B, T_cap + 1))
         seg_tab = self._empty((3 * B * E_cap + B,), torch.int32)
@@ -420,7 +437,7 @@ class Engine:
             _p(g.seg), _p(g.first_node), _p(g.param_end), _p(g.n_splines), C.c_int(t.samples), C.c_int64(t.Q_cap),
             _p(t.lut_d), _p(t.lut_t), _p(t.total_len), C.c_int(t.spn), C.c_int64(t.P_cap), _p(t.prop_k), _p(t.prop_h),
             C.c_int64(D_cap), _p(n_samples), _p(vel), C.c_int64(T_cap), _p(out), _p(nodes_map), _p(actions_map), _p(n_maps),
-            _p(n_out), _p(summary), _p(n_main), _p(stage), C.c_int(E_cap), _p(seg_tab), _p(scr), C.c_int64(plane_stride),
+            _p(n_out), _p(summary), _p(n_main), _p(stage), C.c_int(E_cap), _p(seg_tab), _p(scr), C.c_int64(0),
             _p(t.lut_inv if self.accelerators else None), _p(rden if self.accelerators else None), C.c_int64(rden.numel()),
             self._stream()), "vap_time_profile")
         self.launches += 5
@@ -429,23 +446,19 @@ class Engine:
 
     # ------------------------------------------------------------------ tiled, multi-stream execution
     def _profile_tiled(self, db: DeviceBatch, D_cap: int, T_cap: int, tiles: int, host: "Optional[HostResult]" = None,
-                       dense: Optional[torch.Tensor] = None, events: Optional[list] = None,
-                       stagger: bool = True) -> ProfileResult:
-        """The fast path over `tiles` row slices of the batch, each on its own CUDA stream.
+                       dense: Optional[torch.Tensor] = None, events: Optional[list] = None) -> ProfileResult:
+        """vap_profile_batch over `tiles` row slices of the batch, each on its own CUDA stream.
 
         The serial chains (time loop, chunked velocity passes) are latency-bound and leave most issue slots idle,
         while the table / sampling / pre-pass kernels are throughput-bound; running tiles on separate streams lets the
         block scheduler co-schedule one tile's chains with another tile's sample-parallel kernels.  Tiles write straight
-        into their rows of the batch-wide outputs (out_plane_stride).  Capacities come from the cached plan.
+        into their rows of the batch-wide outputs (out_plane_stride); row k of res.extra["need"] is tile k's `need`.
+        Capacities come from the cached plan.  Like every vap_profile_batch call this uses the inverse LUT index also
+        when the engine was built with accelerators=False (the same bits).
         """
         B = db.B
         main = torch.cuda.current_stream(self.device)
-        out = self._empty((8, B, T_cap))
-        whole = dict(nodes_map=self._empty((B, db.N_max + 1), torch.int32),
-                     actions_map=self._empty((B, max(db.A_max, 1)), torch.int32), n_maps=self._empty((B, 2), torch.int32),
-                     n_out=self._empty((B,), torch.int32), summary=self._empty((B, 5)), n_main=self._empty((B,), torch.int32),
-                     n_samples=self._empty((B,), torch.int32), vel=self._empty((B, D_cap)),
-                     status=self._empty((B,), torch.int32), status_pre=self._empty((B,), torch.int32))
+        res = self._batch_result(db, D_cap, T_cap, tiles)
         self.dgrid(D_cap + 2)                      # make sure the shared tables exist before the side streams read them
         self.lerp_recip(D_cap + 2)
         while len(self._streams) < tiles:
@@ -454,32 +467,13 @@ class Engine:
             k = len(self._streams)
             self._streams.append(torch.cuda.Stream(device=self.device, priority=max(-5, -(5 - min(k, 5)))))
         bounds = [(B * k // tiles, B * (k + 1) // tiles) for k in range(tiles)]
-        sampled = None          # event: the previous tile's throughput-bound front (tables, sampling, velocity passes) is done
         for k, (lo, hi) in enumerate(bounds):
             if hi <= lo:
                 continue
             s = self._streams[k]
             s.wait_stream(main)
-            if sampled is not None and stagger:
-                # software pipeline: the throughput-bound front of tile k starts when tile k-1 enters its latency-bound
-                # time loop (one thread per path, a few warps per SM), so the two overlap instead of running in lockstep;
-                # early tiles finish (and start streaming their rows to the host) first
-                s.wait_event(sampled)
-            sampled = torch.cuda.Event()
             with torch.cuda.stream(s):
-                sub = DeviceBatch(db.node_attr[lo:hi], db.node_flags[lo:hi], db.n_nodes[lo:hi], db.ap_attr[lo:hi],
-                                  db.ap_flags[lo:hi], db.n_ap[lo:hi], db.cons[lo:hi], db.max_splines)
-                outs = {key: val[lo:hi] for key, val in whole.items()}
-                outs["out"] = out[:, lo:hi]          # only its data_ptr() is used: rows lo.. of plane 0
-                outs["plane_stride"] = B * T_cap
-                g = self.build_geometry(sub)
-                t = self.build_lut(sub, g)
-                self.build_props(sub, g, t)
-                outs["status"].copy_(g.status)
-                n_samples, vel, _, _ = self.velocity_chunked(sub, g, t, outs["status"], D_cap, outs=outs, want_t=False)
-                sampled.record(s)
-                outs["status_pre"].copy_(outs["status"])
-                self.time_profile(sub, g, t, outs["status"], D_cap, n_samples, vel, T_cap, outs=outs)
+                self._profile_rows(db, res, lo, hi, k)
                 if host is not None:
                     # dense rows straight into pinned host memory (the kernel streams them over PCIe), then the small
                     # per-path arrays with ordinary async copies; all of it overlaps the other tiles' kernels
@@ -489,20 +483,16 @@ class Engine:
                     base = host.packed if dense is None else dense
                     dst = C.c_void_p(base.data_ptr() + 8 * 8 * lo * T_cap)
                     _lib.check(self.lib.vap_pack_rows(C.c_int64(hi - lo), C.c_int64(T_cap), C.c_int64(B * T_cap),
-                                                      _p(outs["out"]), _p(outs["n_out"]), _p(outs["status"]), _p(offs), dst,
-                                                      self._stream()), "vap_pack_rows")
+                                                      _p(res.out[:, lo:hi]), _p(res.n_out[lo:hi]), _p(res.status[lo:hi]),
+                                                      _p(offs), dst, self._stream()), "vap_pack_rows")
                     self.launches += 2
                     host.offsets[lo + k: hi + k + 1].copy_(offs, non_blocking=True)
                     for name in ("n_out", "status", "nodes_map", "actions_map", "n_maps", "summary"):
-                        getattr(host, name)[lo:hi].copy_(outs[name], non_blocking=True)
+                        getattr(host, name)[lo:hi].copy_(getattr(res, name)[lo:hi], non_blocking=True)
                     if events is not None:
                         events[k].record(s)
         for k in range(tiles):
             main.wait_stream(self._streams[k])
-        self._n_main = whole["n_main"]
-        res = ProfileResult(B, T_cap, out, whole["n_out"], whole["nodes_map"], whole["actions_map"], whole["n_maps"],
-                            whole["status"], whole["summary"], whole["vel"], whole["n_samples"])
-        res.extra = dict(status_pre=whole["status_pre"])
         return res
 
     def profile_many(self, packed: PackedPaths, tile_paths: int = 16384, sink=None) -> torch.Tensor:
@@ -534,20 +524,13 @@ class Engine:
         return dict(key=key, db=db, D_cap=D_cap, T_cap=T_cap, tiles=tiles,
                     host=HostResult(self, B, db.N_max, db.A_max, T_cap, tiles),
                     dense=self._empty((8 * B * T_cap,)), events=[torch.cuda.Event() for _ in range(tiles)],
-                    copy_stream=torch.cuda.Stream(device=self.device),
-                    pin=[torch.empty(t.shape, dtype=t.dtype, pin_memory=True) for t in
-                         (db.node_attr, db.node_flags, db.n_nodes, db.ap_attr, db.ap_flags, db.n_ap, db.cons)])
+                    copy_stream=torch.cuda.Stream(device=self.device), pin=db.pinned())
 
     def _host_submit(self, packed: PackedPaths, st: dict) -> None:
         """Enqueue one batch: inputs host -> device, every tile's kernels, dense packing, small result arrays."""
-        db = st["db"]
-        srcs = (packed.node_attr, packed.node_flags, packed.n_nodes, packed.ap_attr, packed.ap_flags, packed.n_ap, packed.cons)
-        dsts = (db.node_attr, db.node_flags, db.n_nodes, db.ap_attr, db.ap_flags, db.n_ap, db.cons)
-        for pin, src, dst in zip(st["pin"], srcs, dsts):
-            pin.copy_(torch.from_numpy(src))
-            dst.copy_(pin, non_blocking=True)
-        self._profile_tiled(db, st["D_cap"], st["T_cap"], st["tiles"], host=st["host"], dense=st["dense"],
-                            events=st["events"], stagger=True)
+        st["db"].upload_(packed, st["pin"])
+        self._profile_tiled(st["db"], st["D_cap"], st["T_cap"], st["tiles"], host=st["host"], dense=st["dense"],
+                            events=st["events"])
 
     def _host_issue_d2h(self, st: dict) -> None:
         """As each tile's row count reaches the host, queue the copy of exactly those bytes on the copy stream (the copy
@@ -654,45 +637,61 @@ class Engine:
         workspace, capacities checked on the device.  Without capacities the cached plan (or one exact profile()) sizes
         the call; a path that outgrows them comes back as ST_CAPACITY and the call is redone with the sizes the device
         reported in `need` (bounded retries)."""
-        B = db.B
         if D_cap is None or T_cap is None:
             D_cap, T_cap = self.plan_capacities(db)
-        D_cap = (int(D_cap) + 127) // 128 * 128
+        res = self._batch_result(db, (int(D_cap) + 127) // 128 * 128, int(T_cap), 1)
+        self._profile_rows(db, res, 0, db.B, 0)
+        return self._redo_overflow(db, res, _retry)
+
+    def _batch_result(self, db: DeviceBatch, D_cap: int, T_cap: int, parts: int) -> ProfileResult:
+        """Outputs of vap_profile_batch for the whole batch, filled by `parts` calls on row slices (_profile_rows)."""
+        B = db.B
+        res = ProfileResult(B, T_cap, self._empty((8, B, T_cap)), self._empty((B,), torch.int32),
+                            self._empty((B, db.N_max + 1), torch.int32), self._empty((B, max(db.A_max, 1)), torch.int32),
+                            self._empty((B, 2), torch.int32), self._empty((B,), torch.int32), self._empty((B, 5)),
+                            self._empty((B, D_cap)), self._empty((B,), torch.int32))
+        res.extra = dict(need=self._empty((parts, 3), torch.int64), workspace=[])
+        return res
+
+    def _profile_rows(self, db: DeviceBatch, res: ProfileResult, lo: int, hi: int, part: int) -> None:
+        """One vap_profile_batch call on paths lo..hi of `db`, on the current stream, into the same rows of `res`, with
+        res.extra["need"][part] as its `need`.  Its workspace stays alive with `res` (a captured graph replays into it).
+        The inverse LUT index is always used; the lerp reciprocals only with accelerators (both give the same bits)."""
+        B, D_cap, T_cap = hi - lo, res.vel.shape[1], res.T_cap
+        S = max(db.max_splines, 1)
         chunks = self.chunks if D_cap <= 65536 else 256
         grid, rden = self.dgrid(D_cap + 2), self.lerp_recip(D_cap + 2)
-        nbytes = int(self.lib.vap_workspace_bytes(C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), C.c_int(max(db.max_splines, 1)),
+        nbytes = int(self.lib.vap_workspace_bytes(C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), C.c_int(S),
                                                   C.c_int(self.samples), C.c_int(self.spn), C.c_int64(D_cap), C.c_int64(T_cap),
                                                   C.c_int(chunks)))
         if nbytes < 0:
             raise _lib.VapError("vap_workspace_bytes: " + self.lib.vap_last_error().decode())
         ws = torch.empty((nbytes + 255,), dtype=torch.uint8, device=self.device)
-        ws_ptr = (ws.data_ptr() + 255) // 256 * 256
-        out = self._empty((8, B, T_cap))
-        nodes_map = self._empty((B, db.N_max + 1), torch.int32)
-        actions_map = self._empty((B, max(db.A_max, 1)), torch.int32)
-        n_maps = self._empty((B, 2), torch.int32); n_out = self._empty((B,), torch.int32)
-        status = self._empty((B,), torch.int32); summary = self._empty((B, 5))
-        vel = self._empty((B, D_cap)); n_samples = self._empty((B,), torch.int32)
-        need = torch.zeros((3,), dtype=torch.int64, device=self.device)
+        res.extra["workspace"].append(ws)
+        sub = db.rows(lo, hi)
         _lib.check(self.lib.vap_profile_batch(
-            C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), C.c_int(max(db.max_splines, 1)), _p(db.node_attr),
-            _p(db.node_flags), _p(db.n_nodes), _p(db.ap_attr), _p(db.ap_flags), _p(db.n_ap), _p(db.cons), C.c_double(self.dt),
-            C.c_double(self.dd), C.c_double(self.start_vel), C.c_double(self.end_vel), C.c_int(self.samples), C.c_int(self.spn),
-            C.c_int64(D_cap), C.c_int64(T_cap), C.c_int(chunks), _p(grid), C.c_int64(grid.numel()),
-            _p(rden if self.accelerators else None), C.c_int64(rden.numel()), C.c_void_p(ws_ptr), C.c_int64(nbytes), _p(out),
-            C.c_int64(0), _p(n_out), _p(nodes_map), _p(actions_map), _p(n_maps), _p(status), _p(summary), _p(vel), _p(n_samples),
-            _p(need), self._stream()), "vap_profile_batch")
-        self.launches += 20
-        res = ProfileResult(B, T_cap, out, n_out, nodes_map, actions_map, n_maps, status, summary, vel, n_samples)
-        res.extra = dict(need=need, workspace=ws)
-        if _retry < MAX_RETRIES and bool((status == ST_CAPACITY).any().item()):
-            d_need, t_est, t_exact = (int(v) for v in need.tolist())
-            # need[] does not cover paths with more splines than db.max_splines (they were stopped before sampling): the
-            # redo carries the true count, which can only be short once, so that redo does not use up a retry
-            exact = self._with_true_splines(db)
-            return self.profile_batch(exact, max(D_cap, d_need + 8), max(T_cap, int(max(t_est, t_exact) * 1.10) + 64),
-                                      _retry + (1 if exact is db else 0))
-        return res
+            C.c_int64(B), C.c_int(db.N_max), C.c_int(db.A_max), C.c_int(S), *(_p(t) for t in sub.tensors()),
+            C.c_double(self.dt), C.c_double(self.dd), C.c_double(self.start_vel), C.c_double(self.end_vel),
+            C.c_int(self.samples), C.c_int(self.spn), C.c_int64(D_cap), C.c_int64(T_cap), C.c_int(chunks), _p(grid),
+            C.c_int64(grid.numel()), _p(rden if self.accelerators else None), C.c_int64(rden.numel()),
+            C.c_void_p((ws.data_ptr() + 255) // 256 * 256), C.c_int64(nbytes), C.c_void_p(res.out.data_ptr() + 8 * lo * T_cap),
+            C.c_int64(res.B * T_cap), _p(res.n_out[lo:hi]), _p(res.nodes_map[lo:hi]), _p(res.actions_map[lo:hi]),
+            _p(res.n_maps[lo:hi]), _p(res.status[lo:hi]), _p(res.summary[lo:hi]), _p(res.vel[lo:hi]),
+            _p(res.n_samples[lo:hi]), _p(res.extra["need"][part]), self._stream()), "vap_profile_batch")
+        self.launches += PROFILE_BATCH_KERNELS
+
+    def _redo_overflow(self, db: DeviceBatch, res: ProfileResult, retry: int = 0) -> ProfileResult:
+        """`res` (from vap_profile_batch calls on db), or, when a path outgrew the capacities (ST_CAPACITY), its redo through
+        profile_batch with the sizes the device reported in res.extra["need"] (the maximum over its calls); bounded by
+        MAX_RETRIES.  db is only read: a redo runs on a new DeviceBatch over the same tensors."""
+        if retry >= MAX_RETRIES or not bool((res.status == ST_CAPACITY).any().item()):
+            return res
+        d_need, t_est, t_exact = (int(v) for v in res.extra["need"].max(dim=0).values.tolist())
+        # need[] does not cover paths with more splines than db.max_splines (they were stopped before sampling): the
+        # redo carries the true count, which can only be short once, so that redo does not use up a retry
+        exact = self._with_true_splines(db)
+        return self.profile_batch(exact, max(res.vel.shape[1], d_need + 8),
+                                  max(res.T_cap, int(max(t_est, t_exact) * 1.10) + 64), retry + (1 if exact is db else 0))
 
     # ------------------------------------------------------------------ whole path
     def _plan_distance(self, t: Tables, status: torch.Tensor) -> int:
@@ -721,16 +720,15 @@ class Engine:
         keep: also return geometry / tables / distance-domain intermediates.
         reuse_plan: size D_cap / T_cap from the previous call with the same batch shape instead of synchronising
         to read the maxima; capacity overflows are detected on the device and the call is redone exactly.
+        tiles > 1 (with reuse_plan and a plan for this shape): vap_profile_batch on `tiles` row slices on their own
+        streams (_profile_tiled); a redo of an overflow becomes the plan of this shape.
         """
         B = db.B
         key = (B, db.N_max, db.A_max, db.max_splines)
         if (tiles > 1 and reuse_plan and not keep and key in self._plan and self.stage_events is None
                 and self.velocity_impl == "chunked" and self.time_impl == "split"):
-            D_cap, T_cap = self._plan[key]
-            res = self._profile_tiled(db, D_cap, T_cap, min(tiles, B))
-            if bool((res.status == ST_CAPACITY).any().item()) and _retry < MAX_RETRIES:   # undersized plan: redo exactly, untiled
-                self._plan.pop(key, None)
-                return self.profile(db, keep=keep, reuse_plan=False, _retry=_retry + 1)
+            res = self._redo_overflow(db, self._profile_tiled(db, *self._plan[key], min(tiles, B)), _retry)
+            self._plan[key] = (res.vel.shape[1], res.T_cap)
             return res
         with self._stage("S0_build_path"):
             g = self.build_geometry(db)
@@ -761,24 +759,23 @@ class Engine:
         tfun = self.time_profile if self.time_impl == "split" else self.resample
         with self._stage("S6_resample"):
             out, nodes_map, actions_map, n_maps, n_out, summary = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
-        if True:
-            # capacity check (one small read-back; also what a caller needs to trim the rows)
-            if bool((status == ST_CAPACITY).any().item()):
-                if bool((status_pre == ST_CAPACITY).any().item()):
-                    # distance capacity (or db.max_splines, which sizes the distance table) was too small: drop the plan
-                    # and redo with exact sizing and the geometry's true spline count (bounded: a status that survives
-                    # the exact re-runs is reported, never retried forever)
-                    self._plan.pop(key, None)
-                    if _retry < MAX_RETRIES:
-                        return self.profile(self._with_true_splines(db, g.n_splines), keep=keep, reuse_plan=False,
-                                            _retry=_retry + 1)
-                if self.time_impl == "split":
-                    # n_main is exact even on overflow; inserted rows are bounded by the insert estimate
-                    T_cap = int(self._n_main.max().item()) + min(int(self._insert_bound(db, status_pre)), int(ROW_LIMIT)) + 8
-                else:
-                    T_cap = int(n_out.max().item()) + 8
-                status = status_pre.clone()
-                out, nodes_map, actions_map, n_maps, n_out, summary = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
+        # capacity check (one small read-back; also what a caller needs to trim the rows)
+        if bool((status == ST_CAPACITY).any().item()):
+            if bool((status_pre == ST_CAPACITY).any().item()):
+                # distance capacity (or db.max_splines, which sizes the distance table) was too small: drop the plan
+                # and redo with exact sizing and the geometry's true spline count (bounded: a status that survives
+                # the exact re-runs is reported, never retried forever)
+                self._plan.pop(key, None)
+                if _retry < MAX_RETRIES:
+                    return self.profile(self._with_true_splines(db, g.n_splines), keep=keep, reuse_plan=False,
+                                        _retry=_retry + 1)
+            if self.time_impl == "split":
+                # n_main is exact even on overflow; inserted rows are bounded by the insert estimate
+                T_cap = int(self._n_main.max().item()) + min(int(self._insert_bound(db, status_pre)), int(ROW_LIMIT)) + 8
+            else:
+                T_cap = int(n_out.max().item()) + 8
+            status = status_pre.clone()
+            out, nodes_map, actions_map, n_maps, n_out, summary = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
         self._plan[key] = (D_cap, T_cap)
         res = ProfileResult(B, T_cap, out, n_out, nodes_map, actions_map, n_maps, status, summary, vel, n_samples)
         if keep:
@@ -835,7 +832,8 @@ class GraphedProfile:
     small batch is how quickly independent tiles can be put in flight; a graph removes the per-launch host cost.
 
     Inputs live in static device tensors (`self.db`); `run(new_batch)` copies a new batch of the same shape into them.
-    An undersized plan is detected after the replay and the step is redone exactly through Engine.profile.
+    An undersized plan is detected after the replay and the step is redone through Engine.profile_batch, with the sizes
+    the device reported; the static inputs are only read by the redo.
     """
 
     def __init__(self, eng: Engine, db: DeviceBatch, tiles: int = 4, to_host: bool = False, margin: float = 1.0):
@@ -848,8 +846,7 @@ class GraphedProfile:
         self.D_cap, self.T_cap = eng.plan_capacities(db, margin)
         if to_host:
             self.host = HostResult(eng, db.B, db.N_max, db.A_max, self.T_cap, self.tiles)
-            self.host_in = [torch.empty(t.shape, dtype=t.dtype, pin_memory=True) for t in
-                            (db.node_attr, db.node_flags, db.n_nodes, db.ap_attr, db.ap_flags, db.n_ap, db.cons)]
+            self.host_in = db.pinned()
         l0 = eng.launches
         eng._profile_tiled(db, self.D_cap, self.T_cap, self.tiles, host=self.host)   # warm the per-stream allocator pools
         self._launches_warm = eng.launches - l0                # kernels of one step (what a replay launches)
@@ -871,13 +868,10 @@ class GraphedProfile:
     def run(self, new_db: Optional[DeviceBatch] = None, check: bool = True) -> ProfileResult:
         if new_db is not None:
             self.check_shape(new_db)
-            for name in ("node_attr", "node_flags", "n_nodes", "ap_attr", "ap_flags", "n_ap", "cons"):
-                getattr(self.db, name).copy_(getattr(new_db, name), non_blocking=True)
+            self.db.copy_(new_db)
         self.graph.replay()
         self.eng.launches += self.launches_per_run
-        if check and bool((self.res.status == ST_CAPACITY).any().item()):
-            return self.eng.profile(self.db, reuse_plan=False)
-        return self.res
+        return self.eng._redo_overflow(self.db, self.res) if check else self.res
 
     def run_host(self, packed: PackedPaths) -> HostResult:
         """Host buffers in, host buffers out: copy the packed inputs to the device, replay the graph (whose pack kernels
@@ -885,12 +879,7 @@ class GraphedProfile:
         if self.host is None:
             raise ValueError("capture(..., to_host=True) first")
         self.check_shape(packed)
-        srcs = (packed.node_attr, packed.node_flags, packed.n_nodes, packed.ap_attr, packed.ap_flags, packed.n_ap, packed.cons)
-        dsts = (self.db.node_attr, self.db.node_flags, self.db.n_nodes, self.db.ap_attr, self.db.ap_flags, self.db.n_ap,
-                self.db.cons)
-        for pin, src, dst in zip(self.host_in, srcs, dsts):
-            pin.copy_(torch.from_numpy(src))
-            dst.copy_(pin, non_blocking=True)
+        self.db.upload_(packed, self.host_in)
         self.graph.replay()
         self.eng.launches += self.launches_per_run
         torch.cuda.current_stream(self.eng.device).synchronize()
@@ -899,7 +888,7 @@ class GraphedProfile:
         return self.host
 
     def h2d_bytes(self) -> int:
-        return sum(t.numel() * t.element_size() for t in self.host_in)
+        return sum(t.numel() * t.element_size() for t in self.host_in.tensors())
 
 
 class PipelinedProfiler:
@@ -917,12 +906,8 @@ class PipelinedProfiler:
 
     def __init__(self, eng: Engine, db: DeviceBatch, depth: int = 2, margin: float = 1.0):
         self.eng, self.depth = eng, max(1, int(depth))
-
-        def clone(d: DeviceBatch) -> DeviceBatch:
-            return DeviceBatch(d.node_attr.clone(), d.node_flags.clone(), d.n_nodes.clone(), d.ap_attr.clone(),
-                               d.ap_flags.clone(), d.n_ap.clone(), d.cons.clone(), d.max_splines)
         # every slot owns its static inputs: none aliases the caller's `db`, which submit(new_db) would overwrite
-        self.graphs = [eng.capture(clone(db), tiles=1, margin=margin) for _ in range(self.depth)]
+        self.graphs = [eng.capture(db.clone(), tiles=1, margin=margin) for _ in range(self.depth)]
         self.streams = [torch.cuda.Stream(device=eng.device) for _ in range(self.depth)]
         self.n = 0
 
@@ -934,8 +919,7 @@ class PipelinedProfiler:
         st.wait_stream(torch.cuda.current_stream(self.eng.device))          # inputs prepared on the caller's stream
         with torch.cuda.stream(st):
             if new_db is not None:
-                for name in ("node_attr", "node_flags", "n_nodes", "ap_attr", "ap_flags", "n_ap", "cons"):
-                    getattr(g.db, name).copy_(getattr(new_db, name), non_blocking=True)
+                g.db.copy_(new_db)
             g.graph.replay()
             if consume is not None:
                 consume(g.res)
