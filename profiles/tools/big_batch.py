@@ -4,7 +4,7 @@ from vexautonomousplanner_b200 import synth
 from vexautonomousplanner_b200.engine import Engine
 B = int(sys.argv[1]); N = int(sys.argv[2]) if len(sys.argv) > 2 else 8
 packed = synth.random_paths(B, N, seed=1)
-for vi, ti in (("chunked", "split"), ("serial", "split"), ("serial", "serial")):
+for vi, ti in (("chunked", "split"), ("serial", "serial")):
     eng = Engine("cuda:0", velocity_impl=vi, time_impl=ti)
     db = eng.upload(packed)
     for _ in range(2):

@@ -6,10 +6,11 @@ import json
 import sys
 
 STAGE = {"k_build_path": "S0_build_path", "k_build_lut": "S1_lut", "k_build_lut_index": "S1_lut", "k_build_props": "S2_props",
-         "k_count_samples": "S345_velocity", "k_sample_prepass": "S345_velocity", "k_resolve_events": "S345_velocity",
-         "k_prepass_ovr": "S345_velocity", "k_fwd_chunked": "S345_velocity", "k_bwd_chunked": "S345_velocity",
+         "k_flag_lengths": "S345_velocity", "k_count_samples": "S345_velocity", "k_sample_prepass": "S345_velocity",
+         "k_resolve_events": "S345_velocity", "k_prepass_ovr": "S345_velocity", "k_fwd_chunked": "S345_velocity",
+         "k_bwd_chunked": "S345_velocity", "k_flag_times": "S345_velocity",
          "k_time_state": "S6_resample", "k_time_sample": "S6_resample", "k_time_events": "S6_resample",
-         "k_time_finalize": "S6_resample"}
+         "k_time_finalize": "S6_resample", "k_need_rows": "S6_resample"}
 M = {"ms": "gpu__time_duration.sum", "rd": "dram__bytes_read.sum", "wr": "dram__bytes_write.sum", "inst": "smsp__inst_executed.sum",
      "issue": "smsp__issue_active.avg.pct_of_peak_sustained_active", "fp64": "sm__pipe_fp64_cycles_active.avg.pct_of_peak_sustained_active",
      "warps": "sm__warps_active.avg.pct_of_peak_sustained_active"}

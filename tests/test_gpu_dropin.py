@@ -159,6 +159,17 @@ def test_error_conventions():
         mpg.generate_motion_profile(sm, mpg.Constraints(*g["constraints"]))
 
 
+def test_forward_backward_pass_refuses_an_absurd_length():
+    """A 2.5e6 ft path needs more distance samples than the engine accepts (the reference's sampling loop would not fit in
+    memory): forward_backward_pass raises with status -5 instead of sizing its buffers on it."""
+    from vexautonomousplanner_b200.motion_profiling_v2 import motion_profile_generator as mpg
+    from vexautonomousplanner_b200.splines.spline_manager import QuinticHermiteSplineManager
+    sm = QuinticHermiteSplineManager()
+    assert sm.build_path(np.array([[0.0, 0.0], [2.5e6, -2.5e6]]), [Node(), Node()], []) is True
+    with pytest.raises(RuntimeError, match="status -5"):
+        mpg.forward_backward_pass(sm, mpg.Constraints(4.0, 8.0, 8.0, 0.8, 16.0, 12.5 / 12), 0.005)
+
+
 def test_misc_api_matches_reference():
     from vexautonomousplanner_b200.motion_profiling_v2 import motion_profile_generator as mpg
     from vexautonomousplanner_b200.motion_profiling_v2.one_dim_mp_generator import generate_trapezoidal_profile

@@ -392,12 +392,12 @@ def test_time_loop_fuzz_constraints_bitwise(dt, dd):
     ser = Engine("cuda:0", dt=dt, dd=dd, time_impl="serial")
     fast = Engine("cuda:0", dt=dt, dd=dd)
     ref = ser.profile(ser.upload(packed))
-    got = fast.profile(fast.upload(packed))
+    got = fast.profile(fast.upload(packed), keep=True)
     torch.cuda.synchronize()
     assert torch.equal(ref.status, got.status)
     assert int((ref.status == 0).sum()) > B // 2
     bad = (ref.n_out != got.n_out).nonzero().flatten().tolist()
-    assert not bad, [(b, int(ref.n_out[b]), int(got.n_out[b]), int(fast._n_main[b])) for b in bad[:6]]
+    assert not bad, [(b, int(ref.n_out[b]), int(got.n_out[b]), int(got.extra["n_main"][b])) for b in bad[:6]]
     n = ref.n_out.long()
     Tm = min(ref.T_cap, got.T_cap)
     mt = torch.arange(Tm, device=n.device)[None, :] < n[:, None]
@@ -449,23 +449,64 @@ def test_short_paths_and_chunk_edges():
             os.environ["VAP_CHUNK_WARM"] = old
 
 
+def _same_valid_bits(ref, got):
+    assert torch.equal(ref.status, got.status) and torch.equal(ref.n_out, got.n_out)
+    assert torch.equal(ref.n_samples, got.n_samples)
+    n = ref.n_out.long()
+    Tm = min(ref.T_cap, got.T_cap)
+    mt = torch.arange(Tm, device=n.device)[None, :] < n[:, None]
+    for i in range(8):
+        assert torch.equal(ref.out[i][:, :Tm][mt].view(torch.int64), got.out[i][:, :Tm][mt].view(torch.int64)), i
+    D = ref.n_samples.long()
+    md = torch.arange(min(ref.vel.shape[1], got.vel.shape[1]), device=n.device)[None, :] < D[:, None]
+    assert torch.equal(ref.vel[:, :md.shape[1]][md].view(torch.int64), got.vel[:, :md.shape[1]][md].view(torch.int64))
+    assert torch.equal(ref.summary.view(torch.int64), got.summary.view(torch.int64))
+
+
 def test_capacity_retry():
-    """A deliberately undersized plan must be detected on the device and redone exactly."""
+    """A deliberately undersized plan (through vap_profile_batch) and an undersized row estimate of the staged run must
+    be detected on the device and redone exactly."""
     from vexautonomousplanner_b200 import synth
     from vexautonomousplanner_b200.engine import Engine
     packed = synth.mixed_paths(64, 8, seed=9)
     e1 = Engine("cuda:0")
     db = e1.upload(packed)
     ref = e1.profile(db)
+    torch.cuda.synchronize()
+    assert bool((ref.status == 0).all())
     e2 = Engine("cuda:0")
     key = (db.B, db.N_max, db.A_max, db.max_splines)
-    e2._plan[key] = (int(ref.n_samples.max()) + 8, 300)          # T_cap far too small
-    got = e2.profile(db, reuse_plan=True)
+    for plan in ((int(ref.n_samples.max()) + 8, 300),            # T_cap far too small
+                 (1000, ref.T_cap)):                              # D_cap far too small
+        e2._plan[key] = plan
+        got = e2.profile(db, reuse_plan=True)
+        torch.cuda.synchronize()
+        assert "need" in got.extra                                # the planned step is vap_profile_batch
+        _same_valid_bits(ref, got)
+        assert e2._plan[key] == (got.vel.shape[1], got.T_cap)
+    # the staged run: its T_cap estimate (Engine._plan_rows) replaced by one far too small; the time stage is redone with
+    # T_cap = max(n_main + ceil(ins_est)) + 8
+    e3 = Engine("cuda:0")
+    forced = []
+
+    def small(est, status):
+        forced.append(Engine._plan_rows(e3, est, status) // 5)
+        return forced[-1]
+
+    e3._plan_rows = small
+    got = e3.profile(db)
     torch.cuda.synchronize()
-    assert torch.equal(ref.n_out, got.n_out) and (got.status == 0).all()
-    e2._plan[key] = (1000, ref.T_cap)                             # D_cap far too small
-    got = e2.profile(db, reuse_plan=True)
-    assert torch.equal(ref.n_out, got.n_out) and (got.status == 0).all()
+    assert len(forced) == 1 and int(ref.n_out.max()) > forced[0]      # the rows overflowed once
+    _same_valid_bits(ref, got)
+    assert e3._plan[key] == (got.vel.shape[1], got.T_cap)
+
+
+def test_split_time_stage_needs_the_chunked_velocity_stage():
+    """The split time stage redoes an overflow with the chunked velocity stage's bound of the inserted rows, which the
+    serial velocity stage does not compute: that combination is refused."""
+    from vexautonomousplanner_b200.engine import Engine
+    with pytest.raises(ValueError):
+        Engine("cuda:0", velocity_impl="serial", time_impl="split")
 
 
 def test_const_division_is_ieee():

@@ -1,6 +1,6 @@
-"""The tiled, graphed, pipelined and host-streamed steps are vap_profile_batch calls: they flag absurd paths as eager
-Engine.profile does, return its bits on every healthy path, and redo a capacity overflow once with the sizes the device
-reported."""
+"""The planned eager, tiled, graphed, pipelined and host-streamed steps are vap_profile_batch calls: they flag absurd
+paths as the staged Engine.profile does, return its bits on every healthy path, and redo a capacity overflow once with the
+sizes the device reported."""
 from dataclasses import replace
 
 import numpy as np
@@ -71,6 +71,25 @@ def test_every_step_flags_absurd_paths_as_eager_profile():
         want, got = ref.path(b), host.path(b)
         for name in ("times", "x", "y", "linear_vels", "headings", "nodes_map"):
             assert np.array_equal(want[name], got[name]), (b, name)
+
+
+def test_planned_eager_step_is_one_profile_batch_call():
+    """profile(db, reuse_plan=True) with a plan for the shape (tiles = 1) is one vap_profile_batch call on the current
+    stream: exactly its kernels, and the bits of profile_batch and of the staged run that planned the shape."""
+    from vexautonomousplanner_b200 import synth
+    from vexautonomousplanner_b200.engine import PROFILE_BATCH_KERNELS, Engine
+    eng = Engine("cuda:0")
+    db = eng.upload(synth.mixed_paths(320, 8, seed=9))
+    staged = eng.profile(db)
+    torch.cuda.synchronize()
+    l0 = eng.launches
+    planned = eng.profile(db, reuse_plan=True)
+    assert eng.launches - l0 == PROFILE_BATCH_KERNELS
+    batch = eng.profile_batch(db)
+    torch.cuda.synchronize()
+    assert bool((staged.status == 0).all())
+    for got in (planned, batch):
+        same_bits(staged, got, range(db.B))
 
 
 def test_tiled_run_that_outgrows_its_plan_is_redone_once():

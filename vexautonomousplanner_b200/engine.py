@@ -166,6 +166,9 @@ class Engine:
         self.velocity_impl, self.chunks = velocity_impl, int(chunks)
         if time_impl not in ("split", "serial"):
             raise ValueError("time_impl must be 'split' or 'serial'")
+        if (velocity_impl, time_impl) == ("serial", "split"):
+            # the split time stage sizes its row redo from the chunked velocity stage's bound of the inserted rows
+            raise ValueError("time_impl='split' needs velocity_impl='chunked'")
         self.time_impl = time_impl
         # accelerators=False passes NULL for the inverse LUT index and the lerp reciprocals (binary search / plain division
         # instead: same bits, slower); tests use it to pin the equivalence
@@ -336,7 +339,9 @@ class Engine:
     def velocity_chunked(self, db: DeviceBatch, g: Geometry, t: Tables, status: torch.Tensor, D_cap: int, mode: int = 0,
                          want_t: bool = True):
         """S3 + events + S4 + S5, fast path: sampling fused with the hoisted pre-pass (vap_velocity_profile), sample-parallel
-        events, chunk-speculative passes.  want_t: also write t / kappa / theta per distance sample (inspection outputs)."""
+        events, chunk-speculative passes.  want_t: also write t / kappa / theta per distance sample (inspection outputs).
+        Returns n_samples, vel, t_est (time samples of the main loop), ins_est (bound of the rows that waits and turns
+        insert) and the intermediates."""
         B = db.B
         E_cap = db.N_max + db.A_max + 2
         grid = self.dgrid(D_cap + 2)
@@ -372,18 +377,20 @@ class Engine:
             self.launches += 6
         extra = dict(t=tq, kap=kap, th=th, max_accels=ma, bidx=bidx, bval=bval, n_ev=n_ev, vel_f=vel_f, rounds=rounds,
                      vr_idx=vr_idx, vr_val=vr_val, st_idx=st_idx, n_vr=n_vr)
-        return n_samples, vel, t_est + ins_est, extra
+        return n_samples, vel, t_est, ins_est, extra
 
     def velocity_serial(self, db: DeviceBatch, g: Geometry, t: Tables, status: torch.Tensor, D_cap: int, mode: int = 0):
-        """S3 + events + S4 + S5, reference-shaped variant: one thread walks each path (kept as a cross-check)."""
+        """S3 + events + S4 + S5, reference-shaped variant: one thread walks each path (kept as a cross-check).  Returns
+        what velocity_chunked does, except that t_est already counts the inserted rows and ins_est is None."""
         with self._stage("S3_dist_sample"):
             n_samples, tq, kap, th = self.dist_sample(db, g, t, status, D_cap)
         with self._stage("S45_fwd_bwd"):
             vel, ma, bidx, bval, n_ev, t_est = self.fwd_bwd(db, status, D_cap, n_samples, tq, kap, th, mode)
         extra = dict(t=tq, kap=kap, th=th, max_accels=ma, bidx=bidx, bval=bval, n_ev=n_ev)
-        return n_samples, vel, t_est, extra
+        return n_samples, vel, t_est, None, extra
 
     def resample(self, db: DeviceBatch, g: Geometry, t: Tables, status, D_cap, n_samples, vel, T_cap):
+        """S6 + S7, reference-shaped variant: returns what time_profile does, with None for n_main (not counted)."""
         B = db.B
         out = self._empty((8, B, T_cap))
         nodes_map = self._empty((B, db.N_max + 1), torch.int32)
@@ -400,23 +407,11 @@ class Engine:
                                          _p(vel), C.c_int64(T_cap), _p(out), _p(nodes_map), _p(actions_map), _p(n_maps),
                                          _p(n_out), _p(summary), self._stream()), "vap_resample")
         self.launches += 1
-        return out, nodes_map, actions_map, n_maps, n_out, summary
-
-    def _insert_bound(self, db: DeviceBatch, status: Optional[torch.Tensor] = None) -> int:
-        """Upper bound of the rows one (healthy) path can insert for waits and turn profiles (sizing only)."""
-        na = db.node_attr
-        waits = (na[:, :, 3] / self.dt).floor().clamp(min=0).sum(dim=1) + (db.ap_attr[:, :, 1] / self.dt).floor().clamp(min=0).sum(dim=1)
-        V, A, w = db.cons[:, 0:1], db.cons[:, 1:2], db.cons[:, 5:6]
-        arc = (na[:, :, 2].abs() * (3.141592653589793 / 180.0)) * w / 2
-        # trapezoid / triangle duration: never longer than 2 V/A + arc / V, plus two samples of slack per turn
-        turn_rows = torch.where(na[:, :, 2] != 0, ((2 * V / A + arc / V) / self.dt).ceil() + 3, torch.zeros_like(arc)).sum(dim=1)
-        rows = torch.nan_to_num(waits + turn_rows, nan=0.0, posinf=0.0)
-        if status is not None:
-            rows = torch.where(status == ST_OK, rows, torch.zeros_like(rows))
-        return int(rows.max().item()) if rows.numel() else 0
+        return out, nodes_map, actions_map, n_maps, n_out, summary, None
 
     def time_profile(self, db: DeviceBatch, g: Geometry, t: Tables, status, D_cap, n_samples, vel, T_cap):
-        """S6 + S7, fast path (vap_time_profile): state recurrence / parallel lookups / event replay / scatter."""
+        """S6 + S7, fast path (vap_time_profile): state recurrence / parallel lookups / event replay / scatter.  n_main, the
+        last output, counts each path's main-loop rows (exact also when the rows did not fit)."""
         B = db.B
         E_cap = db.N_max + db.A_max + 2
         out = self._empty((8, B, T_cap))
@@ -441,8 +436,7 @@ class Engine:
             _p(t.lut_inv if self.accelerators else None), _p(rden if self.accelerators else None), C.c_int64(rden.numel()),
             self._stream()), "vap_time_profile")
         self.launches += 5
-        self._n_main = n_main
-        return out, nodes_map, actions_map, n_maps, n_out, summary
+        return out, nodes_map, actions_map, n_maps, n_out, summary, n_main
 
     # ------------------------------------------------------------------ tiled, multi-stream execution
     def _profile_tiled(self, db: DeviceBatch, D_cap: int, T_cap: int, tiles: int, host: "Optional[HostResult]" = None,
@@ -713,21 +707,36 @@ class Engine:
                                 "tile the batch (Engine.profile_many) or bucket the paths by length")
         return D_cap
 
+    def _plan_rows(self, est: torch.Tensor, status: torch.Tensor) -> int:
+        """T_cap from the estimated time samples of every path (inserted rows included).  Paths whose profile would need an
+        absurd number of rows (the reference would effectively never return) are flagged ST_DIVERGED here, so that they
+        neither size the buffers nor spin in the time loop."""
+        absurd = ~(est < ROW_LIMIT)
+        status[absurd & (status == ST_OK)] = ST_DIVERGED
+        return int(float(torch.where(absurd, torch.zeros_like(est), est).max().item()) * 1.10) + 64
+
     def profile(self, db: DeviceBatch, keep: bool = False, reuse_plan: bool = False, tiles: int = 1,
                 _retry: int = 0) -> ProfileResult:
         """build_path + generate_motion_profile for every path of the batch.
 
+        reuse_plan, with a plan for this batch shape (and the fast implementations, keep=False, no stage_events): the
+        planned step, vap_profile_batch sized by the plan -- one call on the current stream (tiles == 1) or `tiles` row
+        slices on their own streams (_profile_tiled).  Capacity overflows are detected on the device and redone
+        (_redo_overflow); the capacities that ran become the plan of this shape.
+        Every other call is the staged run, one C entry per stage: it measures D_cap / T_cap from the data (two
+        read-backs), records per-stage timings when stage_events is a list, and plans this batch shape.
         keep: also return geometry / tables / distance-domain intermediates.
-        reuse_plan: size D_cap / T_cap from the previous call with the same batch shape instead of synchronising
-        to read the maxima; capacity overflows are detected on the device and the call is redone exactly.
-        tiles > 1 (with reuse_plan and a plan for this shape): vap_profile_batch on `tiles` row slices on their own
-        streams (_profile_tiled); a redo of an overflow becomes the plan of this shape.
         """
         B = db.B
         key = (B, db.N_max, db.A_max, db.max_splines)
-        if (tiles > 1 and reuse_plan and not keep and key in self._plan and self.stage_events is None
+        if (reuse_plan and not keep and key in self._plan and self.stage_events is None
                 and self.velocity_impl == "chunked" and self.time_impl == "split"):
-            res = self._redo_overflow(db, self._profile_tiled(db, *self._plan[key], min(tiles, B)), _retry)
+            D_cap, T_cap = self._plan[key]
+            tiles = min(tiles, B)
+            if tiles > 1:
+                res = self._redo_overflow(db, self._profile_tiled(db, D_cap, T_cap, tiles), _retry)
+            else:
+                res = self.profile_batch(db, D_cap, T_cap, _retry)
             self._plan[key] = (res.vel.shape[1], res.T_cap)
             return res
         with self._stage("S0_build_path"):
@@ -736,51 +745,38 @@ class Engine:
             t = self.build_lut(db, g)
         with self._stage("S2_props"):
             self.build_props(db, g, t)
-        plan = self._plan.get(key) if reuse_plan else None
         status = g.status.clone()
-        if plan is None:
-            D_cap = self._plan_distance(t, status)
+        D_cap = self._plan_distance(t, status)
+        if self.velocity_impl == "chunked":
+            n_samples, vel, t_est, ins_est, extra = self.velocity_chunked(db, g, t, status, D_cap, want_t=keep)
+            t_est = t_est + ins_est
         else:
-            D_cap = plan[0]
-            status[(t.total_len / self.dd > DIST_LIMIT) & (status == ST_OK)] = ST_DIVERGED
-        D_cap = (D_cap + 127) // 128 * 128
-        vfun = self.velocity_chunked if self.velocity_impl == "chunked" else self.velocity_serial
-        n_samples, vel, t_est, extra = (vfun(db, g, t, status, D_cap, want_t=keep) if self.velocity_impl == "chunked"
-                                        else vfun(db, g, t, status, D_cap))
-        # paths whose profile would need an absurd number of rows (the reference would effectively never return) are
-        # flagged here, so that they neither size the buffers nor spin in the time loop
-        absurd = ~(t_est < ROW_LIMIT)
-        status[absurd & (status == ST_OK)] = ST_DIVERGED
-        if plan is None:
-            T_cap = int(float(torch.where(absurd, torch.zeros_like(t_est), t_est).max().item()) * 1.10) + 64
-        else:
-            T_cap = plan[1]
+            n_samples, vel, t_est, ins_est, extra = self.velocity_serial(db, g, t, status, D_cap)
+        T_cap = self._plan_rows(t_est, status)
         status_pre = status.clone()
         tfun = self.time_profile if self.time_impl == "split" else self.resample
         with self._stage("S6_resample"):
-            out, nodes_map, actions_map, n_maps, n_out, summary = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
+            out, nodes_map, actions_map, n_maps, n_out, summary, n_main = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
         # capacity check (one small read-back; also what a caller needs to trim the rows)
         if bool((status == ST_CAPACITY).any().item()):
-            if bool((status_pre == ST_CAPACITY).any().item()):
-                # distance capacity (or db.max_splines, which sizes the distance table) was too small: drop the plan
-                # and redo with exact sizing and the geometry's true spline count (bounded: a status that survives
-                # the exact re-runs is reported, never retried forever)
-                self._plan.pop(key, None)
-                if _retry < MAX_RETRIES:
-                    return self.profile(self._with_true_splines(db, g.n_splines), keep=keep, reuse_plan=False,
-                                        _retry=_retry + 1)
+            if bool((status_pre == ST_CAPACITY).any().item()) and _retry < MAX_RETRIES:
+                # D_cap is measured, so only an understated db.max_splines (it sizes the distance table) overflows it:
+                # redo with the geometry's true spline count (bounded: a status that survives the re-runs is reported)
+                return self.profile(self._with_true_splines(db, g.n_splines), keep=keep, _retry=_retry + 1)
             if self.time_impl == "split":
-                # n_main is exact even on overflow; inserted rows are bounded by the insert estimate
-                T_cap = int(self._n_main.max().item()) + min(int(self._insert_bound(db, status_pre)), int(ROW_LIMIT)) + 8
+                # k_need_rows' rule: n_main is exact even on overflow, the inserted rows are bounded by ins_est
+                live = (status == ST_OK) | (status == ST_CAPACITY)
+                rows = n_main.clamp(min=0).long() + ins_est.ceil().long()
+                T_cap = int(torch.where(live, rows, torch.zeros_like(rows)).max().item()) + 8
             else:
                 T_cap = int(n_out.max().item()) + 8
             status = status_pre.clone()
-            out, nodes_map, actions_map, n_maps, n_out, summary = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
+            out, nodes_map, actions_map, n_maps, n_out, summary, n_main = tfun(db, g, t, status, D_cap, n_samples, vel, T_cap)
         self._plan[key] = (D_cap, T_cap)
         res = ProfileResult(B, T_cap, out, n_out, nodes_map, actions_map, n_maps, status, summary, vel, n_samples)
         if keep:
             res.geometry, res.tables = g, t
-            res.extra = dict(extra, t_est=t_est)
+            res.extra = dict(extra, t_est=t_est, n_main=n_main)
         return res
 
 

@@ -104,8 +104,8 @@ def forward_backward_pass(spline_manager, constraints: Constraints, delta_dist: 
     eng.build_props(db, g, t)
     _raise_for(int(g.status.item()))
     status = g.status.clone()
-    D_cap = (int(float(t.total_len.item()) / eng.dd) + 8 + 127) // 128 * 128
-    n_samples, vel, _, _ = eng.velocity_chunked(db, g, t, status, D_cap)
+    D_cap = eng._plan_distance(t, status)                   # an absurd length is status -5, not a buffer of its size
+    n_samples, vel, _, _, _ = eng.velocity_chunked(db, g, t, status, D_cap)
     _raise_for(int(status.item()))
     return [np.float64(v) for v in vel[0, : int(n_samples.item())].cpu().numpy()]
 
