@@ -341,6 +341,53 @@ int vap_splice_plan(int64_t B, int N_max, int A_max, const int32_t* status, cons
 int vap_splice_actions(int64_t n_act, const char* act_text, const int64_t* act_off, const int64_t* act_dst, char* text,
                        void* stream);
 
+/* "Next" row f1 read back: the text of saved .txt bodies on the device.  A token is [-]digits[.digits][e[+|-]digits],
+ * [-]inf or [-]nan; its value is bit-equal to Python's float(token) (Clinger's fast path, then Eisel-Lemire with a
+ * 128-bit truncated 5^q).  A token the device does not decide (more than 19 significant digits whose rounding the
+ * digits kept cannot settle, or an ambiguous 128-bit product) is left to the caller's float(), never guessed.
+ *   vap_parse_doubles: token i = text[tok_off[i] .. tok_off[i+1]) (tok_off[n+1] i64) -> out[i] and flags[i] (i8): 0 parsed,
+ *     1 left for float() (out NaN), 2 not a token of the grammar (out NaN).                                          */
+int vap_parse_doubles(int64_t n, const char* text, const int64_t* tok_off, double* out, int8_t* flags, void* stream);
+
+/* Lines of B bodies concatenated in one buffer: body b is text[path_off[b] .. path_off[b+1]) (path_off[B+1] i64,
+ * path_off[B] = n_bytes).  A line ends after '\n' or at the end of its body.  Four calls, the caller scanning between:
+ *   vap_line_starts: starts[n_bytes] (u8) = 1 where a line starts.
+ *   vap_line_offsets: scan[n_bytes] (i32) = inclusive prefix sum of starts; L = scan[n_bytes - 1] lines.  Writes
+ *     line_off[L+1] (i64, line_off[L] = n_bytes) and path_line_off[B+1] (i64): body b owns lines path_line_off[b] ..
+ *     path_line_off[b+1].
+ *   vap_line_kinds: kinds[L] (u8) 0 trajectory row (first token "0"), 1 action row (first token "1"), 2 other;
+ *     errors[L] (i32) 0, 1 blank line, 2 first token neither 0 nor 1; counts[L] (i64) = (kind == 0) + 2^32 (kind == 1).
+ *   vap_parse_rows: count_scan[L] (i64) = inclusive prefix sum of counts (both running counts at once).  Writes path_row_off[B+1]
+ *     and path_act_off[B+1] (i64): body b owns trajectory rows path_row_off[b] .. and action rows path_act_off[b] ..;
+ *     act_line[] (i64, one per action row) = its line; for the trajectory rows of the first parse_paths bodies
+ *     rows[r][7] = {0, t, x, y, heading, v, omega} as written, host_mask[l] (u8, cleared by the call) bit c = token c of
+ *     line l left for float(), errors[l] = 3 when the row has not exactly 7 tokens, 4 + c when token c is not a token
+ *     of the grammar.  rows, act_line: at most L entries.                                                          */
+int vap_line_starts(int64_t B, int64_t n_bytes, const char* text, const int64_t* path_off, uint8_t* starts, void* stream);
+int vap_line_offsets(int64_t B, int64_t n_bytes, const uint8_t* starts, const int32_t* scan, const int64_t* path_off,
+                     int64_t* line_off, int64_t* path_line_off, void* stream);
+int vap_line_kinds(int64_t L, const char* text, const int64_t* line_off, uint8_t* kinds, int32_t* errors, int64_t* counts,
+                   void* stream);
+int vap_parse_rows(int64_t B, int64_t L, const char* text, const int64_t* line_off, const uint8_t* kinds,
+                   const int64_t* count_scan, const int64_t* path_line_off, int64_t parse_paths, int64_t* path_row_off,
+                   int64_t* path_act_off, int64_t* act_line, double* rows, uint8_t* host_mask, int32_t* errors, void* stream);
+
+/* A saved body against a fresh one, per path b (one warp each): saved body text[old_off[b] .. old_off[b+1]), fresh body
+ * text[new_off[b] .. new_off[b+1]) (the same buffer, e.g. both sets split by the calls above with 2B bodies).  line_off,
+ * line_err, act_line as above; the saved body's lines start at old_path_line_off[b]; the saved and fresh action rows of
+ * b start at old_path_act_off[b] / new_path_act_off[b] in act_line; old_rows / new_rows [.][7] with their per-path row
+ * offsets (the parsed rows, and the rows of vap_export_rows).
+ *   out_i64[B][7]: first differing byte from the body start (-1 equal), its line in the saved body from 1 (0 equal),
+ *     saved and fresh trajectory rows, action rows that differ (the k-th saved against the k-th fresh; unpaired ones
+ *     count), first saved line with an error from 1 (0 none), its error code.
+ *   out_f64[B][8]: t of the last saved and of the last fresh row (NaN without rows), max |saved - fresh| of t, x, y,
+ *     heading, v, omega over the common rows (row k against row k; inf where exactly one is NaN).                  */
+int vap_compare_bodies(int64_t B, const char* text, const int64_t* old_off, const int64_t* new_off, const int64_t* line_off,
+                       const int32_t* line_err, const int64_t* old_path_line_off, const int64_t* act_line,
+                       const int64_t* old_path_act_off, const int64_t* new_path_act_off, const double* old_rows,
+                       const int64_t* old_row_off, const double* new_rows, const int64_t* new_row_off, int64_t* out_i64,
+                       double* out_f64, void* stream);
+
 /* Bounds diagnostics of a -DVAP_BOUNDS_CHECK build (profiles/tools/bounds_check.py; compute-sanitizer is closed on the GPU
  * pool this was developed on): out_host[32] (HOST memory) = violations per check site (0..15) and checks executed per site
  * (16..31); returns <0 in a release build, where the checks are compiled away.                                          */

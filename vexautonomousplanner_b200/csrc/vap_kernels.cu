@@ -16,6 +16,7 @@
 #include "vap_velocity.cuh"
 #include "vap_timeloop.cuh"
 #include "vap_format.cuh"
+#include "vap_parse.cuh"
 
 static thread_local char g_err[512] = "";
 static int set_err(const char* where, cudaError_t e)
@@ -1681,6 +1682,94 @@ extern "C" int vap_splice_actions(int64_t n_act, const char* act_text, const int
     k_splice_actions<<<blocks_for(n_act * 32, 256), 256, 0, STREAM>>>(n_act, act_text, reinterpret_cast<const long long*>(act_off),
                                                                      reinterpret_cast<const long long*>(act_dst), text);
     CHECK_LAUNCH("vap_splice_actions");
+    return 0;
+}
+
+// ---- reading the text back (vap_parse.cuh) ------------------------------------------------------------------------
+extern "C" int vap_parse_doubles(int64_t n, const char* text, const int64_t* tok_off, double* out, int8_t* flags, void* stream)
+{
+    if (n <= 0) return 0;
+    k_parse_doubles<<<blocks_for(n, 256), 256, 0, STREAM>>>(n, text, reinterpret_cast<const long long*>(tok_off), out,
+                                                           reinterpret_cast<signed char*>(flags));
+    CHECK_LAUNCH("vap_parse_doubles");
+    return 0;
+}
+
+extern "C" int vap_line_starts(int64_t B, int64_t n_bytes, const char* text, const int64_t* path_off, uint8_t* starts,
+                               void* stream)
+{
+    if (B < 0 || n_bytes < 0) return arg_err("vap_line_starts: B >= 0 and n_bytes >= 0 required");
+    if (n_bytes == 0) return 0;
+    k_line_starts<<<blocks_for(n_bytes, 256), 256, 0, STREAM>>>(n_bytes, text, starts);
+    CHECK_LAUNCH("vap_line_starts");
+    if (B > 0) {
+        k_body_starts<<<blocks_for(B, 256), 256, 0, STREAM>>>(B, n_bytes, reinterpret_cast<const long long*>(path_off), starts);
+        CHECK_LAUNCH("vap_line_starts/bodies");
+    }
+    return 0;
+}
+
+extern "C" int vap_line_offsets(int64_t B, int64_t n_bytes, const uint8_t* starts, const int32_t* scan, const int64_t* path_off,
+                                int64_t* line_off, int64_t* path_line_off, void* stream)
+{
+    if (B < 0 || n_bytes < 0) return arg_err("vap_line_offsets: B >= 0 and n_bytes >= 0 required");
+    if (n_bytes > 0) {
+        k_line_offsets<<<blocks_for(n_bytes, 256), 256, 0, STREAM>>>(n_bytes, starts, scan, reinterpret_cast<long long*>(line_off));
+        CHECK_LAUNCH("vap_line_offsets");
+    }
+    k_path_lines<<<blocks_for(B + 1, 256), 256, 0, STREAM>>>(B, n_bytes, reinterpret_cast<const long long*>(path_off), scan,
+                                                            reinterpret_cast<long long*>(line_off),
+                                                            reinterpret_cast<long long*>(path_line_off));
+    CHECK_LAUNCH("vap_line_offsets/paths");
+    return 0;
+}
+
+extern "C" int vap_line_kinds(int64_t L, const char* text, const int64_t* line_off, uint8_t* kinds, int32_t* errors,
+                              int64_t* counts, void* stream)
+{
+    if (L <= 0) return 0;
+    if (L >= (1LL << 31)) return arg_err("vap_line_kinds: at most 2^31 - 1 lines");
+    k_line_kinds<<<blocks_for(L, 256), 256, 0, STREAM>>>(L, text, reinterpret_cast<const long long*>(line_off), kinds, errors,
+                                                        reinterpret_cast<long long*>(counts));
+    CHECK_LAUNCH("vap_line_kinds");
+    return 0;
+}
+
+extern "C" int vap_parse_rows(int64_t B, int64_t L, const char* text, const int64_t* line_off, const uint8_t* kinds,
+                              const int64_t* count_scan, const int64_t* path_line_off, int64_t parse_paths,
+                              int64_t* path_row_off, int64_t* path_act_off, int64_t* act_line, double* rows,
+                              uint8_t* host_mask, int32_t* errors, void* stream)
+{
+    if (B < 0 || L < 0 || parse_paths < 0 || parse_paths > B)
+        return arg_err("vap_parse_rows: B >= 0, L >= 0 and 0 <= parse_paths <= B required");
+    const long long* cs = reinterpret_cast<const long long*>(count_scan);
+    const long long* pl = reinterpret_cast<const long long*>(path_line_off);
+    k_path_rows<<<blocks_for(B + 1, 256), 256, 0, STREAM>>>(B, pl, cs, reinterpret_cast<long long*>(path_row_off),
+                                                           reinterpret_cast<long long*>(path_act_off));
+    CHECK_LAUNCH("vap_parse_rows/paths");
+    if (L == 0) return 0;
+    cudaError_t e = cudaMemsetAsync(host_mask, 0, (size_t)L, STREAM);
+    if (e != cudaSuccess) return set_err("vap_parse_rows/memset", e);
+    k_parse_lines<<<blocks_for(L, 128), 128, 0, STREAM>>>(L, text, reinterpret_cast<const long long*>(line_off), kinds, cs,
+                                                         pl + parse_paths, reinterpret_cast<long long*>(act_line), rows,
+                                                         host_mask, errors);
+    CHECK_LAUNCH("vap_parse_rows");
+    return 0;
+}
+
+extern "C" int vap_compare_bodies(int64_t B, const char* text, const int64_t* old_off, const int64_t* new_off,
+                                  const int64_t* line_off, const int32_t* line_err, const int64_t* old_path_line_off,
+                                  const int64_t* act_line, const int64_t* old_path_act_off, const int64_t* new_path_act_off,
+                                  const double* old_rows, const int64_t* old_row_off, const double* new_rows,
+                                  const int64_t* new_row_off, int64_t* out_i64, double* out_f64, void* stream)
+{
+    if (B <= 0) return 0;
+    typedef const long long* P;
+    k_compare_bodies<<<blocks_for(B * 32, 128), 128, 0, STREAM>>>(B, text, P(old_off), P(new_off), P(line_off), line_err,
+                                                                  P(old_path_line_off), P(act_line), P(old_path_act_off),
+                                                                  P(new_path_act_off), old_rows, P(old_row_off), new_rows,
+                                                                  P(new_row_off), reinterpret_cast<long long*>(out_i64), out_f64);
+    CHECK_LAUNCH("vap_compare_bodies");
     return 0;
 }
 

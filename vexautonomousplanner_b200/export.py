@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 import json
+from dataclasses import dataclass
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -112,6 +113,195 @@ def format_doubles_device(eng: Engine, x: torch.Tensor) -> List[str]:
     eng.launches += 1
     o, l = out.cpu().numpy(), lens.cpu().numpy()
     return [bytes(o[i, : l[i]]).decode() for i in range(n)]
+
+
+def _host_finish(out: torch.Tensor, flat_idx: Sequence[int], tokens: Sequence) -> None:
+    """out.view(-1)[flat_idx[k]] = float(tokens[k]): the tokens the device left undecided, finished by Python."""
+    if len(flat_idx):
+        vals = torch.tensor([float(t) for t in tokens], dtype=torch.float64)
+        out.view(-1)[torch.tensor(list(flat_idx), dtype=torch.int64).to(out.device)] = vals.to(out.device)
+
+
+def parse_doubles_device(eng: Engine, strings: Sequence[str]):
+    """float() of every string, parsed on the device (vap_parse_doubles): the inverse of format_doubles_device.
+    Returns (x, flags): x fp64 device tensor, bit-equal to float(s) for every token of the grammar [-]digits[.digits]
+    [e[+|-]digits], [-]inf, [-]nan; flags int8 host array: 0 parsed on the device, 1 finished on the host with float()
+    (the device could not decide it), 2 not a token of the grammar (x is NaN)."""
+    enc = [s.encode() for s in strings]
+    n = len(enc)
+    tok_off = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(np.fromiter(map(len, enc), dtype=np.int64, count=n), out=tok_off[1:])
+    text = np.frombuffer(b"".join(enc) or b"\0", dtype=np.uint8)
+    text_d = torch.from_numpy(text.copy()).to(eng.device)
+    off_d = torch.from_numpy(tok_off).to(eng.device)
+    out = torch.empty(max(n, 1), dtype=torch.float64, device=eng.device)
+    flags = torch.empty(max(n, 1), dtype=torch.int8, device=eng.device)
+    _lib.check(eng.lib.vap_parse_doubles(C.c_int64(n), _p(text_d), _p(off_d), _p(out), _p(flags), eng._stream()),
+               "vap_parse_doubles")
+    eng.launches += 1
+    fl = flags[:n].cpu().numpy()
+    host = np.flatnonzero(fl == 1)
+    _host_finish(out, host.tolist(), [strings[i] for i in host])
+    return out[:n], fl
+
+
+LINE_TRAJ, LINE_ACTION, LINE_OTHER = 0, 1, 2
+LINE_ERRORS = {1: "blank line", 2: "the first token is neither 0 nor 1", 3: "a trajectory row without 7 tokens"}
+ROW_COLUMNS = ("kind", "t", "x", "y", "heading", "v", "omega")
+
+
+def line_error_text(code: int) -> str:
+    """What a line error code of parse_text_batch means."""
+    if code >= 4:
+        c = code - 4
+        return f"token {c + 1} ({ROW_COLUMNS[c] if c < 7 else '?'}) is not a number"
+    return LINE_ERRORS.get(code, f"error {code}")
+
+
+@dataclass
+class ParsedText:
+    """Bodies read back on the device (parse_text_batch).  Body b owns lines path_line_offsets[b] .. [b+1], trajectory
+    rows row_offsets[b] .. [b+1] and action rows act_offsets[b] .. [b+1]; line l is text[line_offsets[l] ..
+    line_offsets[l+1]).  All tensors are on the device."""
+    text: torch.Tensor                # uint8[n_bytes], the uploaded bodies
+    path_offsets: torch.Tensor        # int64[B+1]
+    rows: torch.Tensor                # fp64[R, 7] {0, t, x, y, heading, v, omega} as written
+    row_offsets: torch.Tensor         # int64[B+1]
+    line_offsets: torch.Tensor        # int64[L+1]
+    path_line_offsets: torch.Tensor   # int64[B+1]
+    line_kinds: torch.Tensor          # uint8[L]: LINE_TRAJ, LINE_ACTION, LINE_OTHER
+    line_errors: torch.Tensor         # int32[L]: 0, or a code line_error_text explains
+    act_lines: torch.Tensor           # int64[A]: the line of every action row
+    act_offsets: torch.Tensor         # int64[B+1]
+    n_host: int                       # tokens finished on the host with float()
+
+
+def _as_u8(text) -> np.ndarray:
+    if isinstance(text, torch.Tensor):
+        return text.numpy()
+    if isinstance(text, (bytes, bytearray, memoryview)):
+        return np.frombuffer(text, dtype=np.uint8)
+    return np.asarray(text, dtype=np.uint8)
+
+
+def _pinned_text(text) -> torch.Tensor:
+    if isinstance(text, torch.Tensor) and text.is_pinned():
+        return text
+    a = _as_u8(text)
+    t = torch.empty(max(a.size, 1), dtype=torch.uint8, pin_memory=True)
+    t[:a.size].numpy()[:] = a
+    return t[:a.size]
+
+
+def _read_bodies(eng: Engine, text, path_offsets, parse_paths: int) -> ParsedText:
+    """parse_text_batch, with the trajectory rows parsed for the first parse_paths bodies only (the lines, kinds,
+    first-token errors and action rows of every body)."""
+    poff = np.ascontiguousarray(path_offsets, dtype=np.int64)
+    B, N = poff.shape[0] - 1, int(poff[-1])
+    host = _pinned_text(text)
+    if host.numel() < N or poff[0] != 0 or (np.diff(poff) < 0).any():
+        raise ValueError("path_offsets must start at 0, never decrease and end within the text")
+    if N >= 2 ** 31:
+        raise ValueError(f"{N} bytes: at most 2^31 - 1 bytes per call (tile the batch)")
+    dev, st, L_ = eng.device, eng._stream(), eng.lib
+    with eng._stage("read_upload"):
+        text_d = host[:max(N, 1)].to(dev, non_blocking=True) if N else torch.zeros(1, dtype=torch.uint8, device=dev)
+    poff_d = torch.from_numpy(poff).to(dev)
+    with eng._stage("read_lines"):
+        starts = torch.empty(max(N, 1), dtype=torch.uint8, device=dev)
+        _lib.check(L_.vap_line_starts(C.c_int64(B), C.c_int64(N), _p(text_d), _p(poff_d), _p(starts), st), "vap_line_starts")
+        scan = torch.cumsum(starts[:N], 0, dtype=torch.int32) if N else torch.zeros(1, dtype=torch.int32, device=dev)
+        L = int(scan[-1].item()) if N else 0                               # read-back 1: the number of lines
+        line_off = torch.empty(L + 1, dtype=torch.int64, device=dev)
+        pl = torch.empty(B + 1, dtype=torch.int64, device=dev)
+        _lib.check(L_.vap_line_offsets(C.c_int64(B), C.c_int64(N), _p(starts), _p(scan), _p(poff_d), _p(line_off), _p(pl), st),
+                   "vap_line_offsets")
+        del starts, scan
+        Lc = max(L, 1)
+        kinds = torch.empty(Lc, dtype=torch.uint8, device=dev)
+        errors = torch.zeros(Lc, dtype=torch.int32, device=dev)
+        counts = torch.empty(Lc, dtype=torch.int64, device=dev)
+        _lib.check(L_.vap_line_kinds(C.c_int64(L), _p(text_d), _p(line_off), _p(kinds), _p(errors), _p(counts), st),
+                   "vap_line_kinds")
+        cscan = torch.cumsum(counts[:L], 0) if L else torch.zeros(1, dtype=torch.int64, device=dev)   # rows + 2^32 actions
+        del counts
+    with eng._stage("read_parse"):
+        row_off = torch.empty(B + 1, dtype=torch.int64, device=dev)
+        act_off = torch.empty(B + 1, dtype=torch.int64, device=dev)
+        act_line = torch.empty(Lc, dtype=torch.int64, device=dev)
+        rows = torch.empty((Lc, 7), dtype=torch.float64, device=dev)
+        host_mask = torch.empty(Lc, dtype=torch.uint8, device=dev)
+        _lib.check(L_.vap_parse_rows(C.c_int64(B), C.c_int64(L), _p(text_d), _p(line_off), _p(kinds), _p(cscan), _p(pl),
+                                     C.c_int64(parse_paths), _p(row_off), _p(act_off), _p(act_line), _p(rows),
+                                     _p(host_mask), _p(errors), st), "vap_parse_rows")
+    eng.launches += 8
+    flagged = host_mask[:L] != 0
+    head = torch.stack([row_off[parse_paths], act_off[B], flagged.sum()]).cpu().tolist()   # read-back 2
+    R, A, n_flag = head
+    n_host = 0
+    if n_flag:                                                              # read-back 3: the lines left for float()
+        idx = torch.nonzero_static(flagged, size=n_flag).flatten()
+        info = torch.stack([host_mask[idx].long(), line_off[idx], line_off[idx + 1], (cscan[idx] & 0xffffffff) - 1]).cpu().numpy()
+        hb = host.numpy()
+        flat, toks = [], []
+        for mask, s, e, r in info.T:
+            words = bytes(hb[s:e]).split()
+            for c in range(1, 7):
+                if mask >> c & 1:
+                    flat.append(int(r) * 7 + c)
+                    toks.append(words[c])
+        _host_finish(rows, flat, toks)
+        n_host = len(flat)
+    return ParsedText(text_d, poff_d, rows[:R], row_off, line_off, pl, kinds[:L], errors[:L], act_line[:A], act_off, n_host)
+
+
+def parse_text_batch(eng: Engine, text, path_offsets) -> ParsedText:
+    """Read saved .txt bodies back on the device: text holds B bodies back to back (bytes, a uint8 array, or a pinned
+    uint8 CPU tensor), body b is text[path_offsets[b] .. path_offsets[b+1]).  Returns a ParsedText: the trajectory rows
+    [R, 7] as written (bit-equal to float() of every token), per-body row, line and action-row offsets, line kinds and
+    per-line errors; tokens the device could not decide are already finished with float() (their count: n_host).
+    The text goes to the device in one copy from pinned memory; the call reads back from the device at most three
+    times, whatever B is."""
+    return _read_bodies(eng, text, path_offsets, len(path_offsets) - 1)
+
+
+CMP_I = ("diff_byte", "diff_line", "old_rows", "new_rows", "action_rows_differ", "error_line", "error_code")
+CMP_F = ("old_t", "new_t", "max_dt", "max_dx", "max_dy", "max_dheading", "max_dv", "max_domega")
+
+
+def compare_text_batch(eng: Engine, old_text, old_offsets, new_text, new_offsets, new_rows: torch.Tensor,
+                       new_row_offsets: torch.Tensor):
+    """Saved bodies against fresh ones, path by path, on the device (vap_compare_bodies).  old_text / old_offsets: the
+    saved bodies as parse_text_batch takes them (old_text may be a pinned tensor with room for the fresh text behind
+    old_offsets[-1]: the fresh text then goes there and both travel in one copy); new_text / new_offsets: the fresh
+    bodies (save_text_batch); new_rows / new_row_offsets: their numeric rows (export_rows).
+    Returns (ints int64[B, 7] named by CMP_I, floats fp64[B, 8] named by CMP_F, n_host), host arrays: first differing
+    byte (-1 equal) and its line in the saved body, saved and fresh row counts, differing action rows, first saved line
+    with an error and its code (line_error_text), last saved and fresh t, max |saved - fresh| of t, x, y, heading, v,
+    omega over the common rows (as written: inches and inch/s)."""
+    oo = np.ascontiguousarray(old_offsets, dtype=np.int64)
+    no = np.ascontiguousarray(new_offsets, dtype=np.int64)
+    B, n_old, n_new = oo.shape[0] - 1, int(oo[-1]), int(no[-1])
+    if no.shape[0] != B + 1:
+        raise ValueError(f"{B} saved bodies but {no.shape[0] - 1} fresh ones")
+    if isinstance(old_text, torch.Tensor) and old_text.is_pinned() and old_text.numel() >= n_old + n_new:
+        buf = old_text
+    else:
+        buf = torch.empty(max(n_old + n_new, 1), dtype=torch.uint8, pin_memory=True)
+        buf[:n_old].numpy()[:] = _as_u8(old_text)[:n_old]
+    buf[n_old:n_old + n_new].numpy()[:] = _as_u8(new_text)[:n_new]
+    poff = np.concatenate([oo, n_old + no[1:]])
+    p = _read_bodies(eng, buf[:n_old + n_new], poff, B)
+    out_i = torch.empty((max(B, 1), len(CMP_I)), dtype=torch.int64, device=eng.device)
+    out_f = torch.empty((max(B, 1), len(CMP_F)), dtype=torch.float64, device=eng.device)
+    with eng._stage("read_compare"):
+        _lib.check(eng.lib.vap_compare_bodies(C.c_int64(B), _p(p.text), _p(p.path_offsets), _p(p.path_offsets[B:]),
+                                              _p(p.line_offsets), _p(p.line_errors), _p(p.path_line_offsets), _p(p.act_lines),
+                                              _p(p.act_offsets), _p(p.act_offsets[B:]), _p(p.rows), _p(p.row_offsets),
+                                              _p(new_rows), _p(new_row_offsets), _p(out_i), _p(out_f), eng._stream()),
+                   "vap_compare_bodies")
+    eng.launches += 1
+    return out_i[:B].cpu().numpy(), out_f[:B].cpu().numpy(), p.n_host                # read-back 4
 
 
 def splice_action_rows(traj_rows: Sequence[Sequence[float]], nodes_map: Sequence[int], node_actions: Sequence[Sequence],

@@ -12,6 +12,13 @@ ConfigManager does), and the explicit flags override them; without either, the f
 Files that are not route JSON and routes the GUI's save refuses (it needs more than two nodes, a start node and an end
 node, gui_manager.py:263-267) are listed and not written; so are routes whose profile fails (status != 0).  The exit
 status is 0 only when every route was written.
+
+With --check nothing is written: every route's fresh body is compared with OUT_DIR/<name>.txt on the device (the saved
+file is read back with export.compare_text_batch) and one line per route says "up to date" (the bytes are equal),
+"stale" (the first differing line, old -> new trajectory rows, old -> new duration, the largest moves of x, y, v and
+heading over the common rows, the action rows that differ), "missing" or "unreadable" (the line and the reason).  The
+exit status is 0 only when every route is up to date.  Use it in CI to see that committed trajectory files are current,
+or after a constant changed to see what the change does to each route.
 """
 from __future__ import annotations
 
@@ -101,6 +108,71 @@ def save_routes(routes: Sequence, out_dir: str, cons, tile_paths: int = 8192, de
     return failed
 
 
+def check_line(name: str, ints, floats) -> Tuple[str, str]:
+    """(state, report line) of one route from its compare_text_batch result (ints named by CMP_I, floats by CMP_F)."""
+    from .export import CMP_F, CMP_I, line_error_text
+    i = dict(zip(CMP_I, (int(v) for v in ints)))
+    f = dict(zip(CMP_F, (float(v) for v in floats)))
+    if i["diff_byte"] < 0:
+        return "up to date", f"up to date: {name}"
+    if i["error_line"] > 0:
+        return "unreadable", f"unreadable: {name}: line {i['error_line']}: {line_error_text(i['error_code'])}"
+    return "stale", (f"stale: {name}: first difference on line {i['diff_line']}; rows {i['old_rows']} -> {i['new_rows']}; "
+                     f"duration {f['old_t']!r} -> {f['new_t']!r} s; max |dx| {f['max_dx']:.6g} in, |dy| {f['max_dy']:.6g} in, "
+                     f"|dv| {f['max_dv']:.6g} in/s, |dheading| {f['max_dheading']:.6g}; "
+                     f"{i['action_rows_differ']} action rows differ")
+
+
+def check_batch(eng, db, node_actions, ap_actions, files: Sequence[str]):
+    """One batch of --check: profile db, assemble the fresh bodies, read the saved files[b] (missing ones as empty
+    bodies) into one pinned buffer and compare on the device.  Returns (res, ok, present, ints, floats) with ints /
+    floats as export.compare_text_batch gives them."""
+    import numpy as np
+    import torch
+    from .export import compare_text_batch, export_rows, save_text_batch
+    res = eng.profile(db)
+    text, offs, ok = save_text_batch(eng, res, db, node_actions, ap_actions)
+    rows, row_off = export_rows(eng, res)
+    present = [os.path.isfile(p) for p in files]
+    sizes = np.array([os.path.getsize(p) if there else 0 for p, there in zip(files, present)], dtype=np.int64)
+    old_off = np.zeros(len(files) + 1, dtype=np.int64)
+    np.cumsum(sizes, out=old_off[1:])
+    buf = torch.empty(max(int(old_off[-1] + offs[-1]), 1), dtype=torch.uint8, pin_memory=True)
+    view = memoryview(buf.numpy())
+    for p, there, a, z in zip(files, present, old_off[:-1], old_off[1:]):
+        if there:
+            with open(p, "rb") as f:
+                f.readinto(view[a:z])
+    ints, floats, _ = compare_text_batch(eng, buf, old_off, text, offs, rows, row_off)
+    return res, ok, present, ints, floats
+
+
+def check_routes(routes: Sequence, out_dir: str, cons, tile_paths: int = 8192, device: str = "cuda:0"):
+    """Compare every route's fresh body with out_dir/<name>, tile_paths routes at a time; writes nothing.
+    Returns [(name, state, report line)], state one of "up to date", "stale", "missing", "unreadable", "not checked"."""
+    from .engine import Engine
+    from .packing import pack_paths
+    eng = Engine(device)
+    out = []
+    for lo in range(0, len(routes), tile_paths):
+        tile = routes[lo: lo + tile_paths]
+        db = eng.upload(pack_paths([(pts, nodes, aps) for _, pts, nodes, aps in tile], cons))
+        res, ok, present, ints, floats = check_batch(eng, db, [[n.action_values for n in nodes] for _, _, nodes, _ in tile],
+                                                     [[a.action_values for a in aps] for _, _, _, aps in tile],
+                                                     [os.path.join(out_dir, name) for name, _, _, _ in tile])
+        status = res.status.cpu().tolist() if not ok.all() else None
+        for b, (name, _, _, _) in enumerate(tile):
+            if not ok[b]:
+                s = int(status[b])
+                out.append((name, "not checked", f"not checked: {name}: profile failed, status {s} "
+                                                 f"({STATUS_NAMES.get(s, 'unknown')})"))
+            elif not present[b]:
+                out.append((name, "missing", f"missing: {name}"))
+            else:
+                out.append((name, *check_line(name, ints[b], floats[b])))
+    return out
+
+
 def parse_args(argv: Optional[List[str]] = None) -> argparse.Namespace:
     p = argparse.ArgumentParser(prog="python -m vexautonomousplanner_b200.save_routes",
                                 description="Re-save every route of a folder: write each route's trajectory .txt.")
@@ -115,6 +187,8 @@ def parse_args(argv: Optional[List[str]] = None) -> argparse.Namespace:
                    help=f"track width in inches (factory {DEFAULTS['track_width_in']})")
     p.add_argument("--tile-paths", type=int, default=8192, help="routes profiled per batch (default 8192)")
     p.add_argument("--device", default="cuda:0")
+    p.add_argument("--check", action="store_true",
+                   help="write nothing: report which files of OUT_DIR are up to date, stale, missing or unreadable")
     args = p.parse_args(argv)
     if args.tile_paths < 1:
         p.error("--tile-paths must be at least 1")
@@ -129,6 +203,16 @@ def main(argv: Optional[List[str]] = None) -> int:
         return 2
     cons = constraints(args)
     routes, skipped = read_routes(args.routes_dir)
+    cons_text = (f"max_velocity {cons[0]}, max_acceleration {cons[1]}, max_jerk {cons[4]}, track_width {cons[5]} ft")
+    if args.check:
+        checked = check_routes(routes, args.out_dir, cons, args.tile_paths, args.device) if routes else []
+        for name, why in skipped:
+            print(f"not checked: {name}: {why}")
+        for _, _, line in checked:
+            print(line)
+        n_up = sum(state == "up to date" for _, state, _ in checked)
+        print(f"{n_up} of {len(routes) + len(skipped)} files up to date in {args.out_dir} ({cons_text})")
+        return 0 if n_up == len(routes) + len(skipped) else 1
     os.makedirs(args.out_dir, exist_ok=True)
     failed = save_routes(routes, args.out_dir, cons, args.tile_paths, args.device) if routes else []
     for name, why in skipped:
@@ -136,8 +220,7 @@ def main(argv: Optional[List[str]] = None) -> int:
     for name, why in failed:
         print(f"not written: {name}: profile failed, {why}")
     n_written = len(routes) - len(failed)
-    print(f"wrote {n_written} of {len(routes) + len(skipped)} files to {args.out_dir} "
-          f"(max_velocity {cons[0]}, max_acceleration {cons[1]}, max_jerk {cons[4]}, track_width {cons[5]} ft)")
+    print(f"wrote {n_written} of {len(routes) + len(skipped)} files to {args.out_dir} ({cons_text})")
     return 0 if not skipped and not failed else 1
 
 
