@@ -226,23 +226,16 @@ def test_reference_saved_files_parse():
     assert p.path_line_offsets.cpu().tolist() == [0, bodies[0].count(b"\n"), len(want_kinds)]
 
 
-@pytest.mark.gpu
-def test_check_command_on_a_folder(tmp_path, capsys):
-    """save, then --check: every route up to date (exit 0); with --max-velocity halved every route is stale, with the
-    fresh profile's t_end as the new duration and the first run's as the old one; a deleted file is missing, a
-    corrupted token unreadable with its line (exit 1)."""
+def _route_folder(eng, rdir, half):
+    """Write to rdir the GUI reference routes that the save accepts and that profile at the factory constraints and
+    at `half`; returns {file name: [t_end at the factory constraints, t_end at half]}."""
     from test_next_rows import _gui_ref
-    from vexautonomousplanner_b200 import export as ex, save_routes as sr
-    from vexautonomousplanner_b200.engine import Engine
+    from vexautonomousplanner_b200 import export as ex
     from vexautonomousplanner_b200.packing import pack_paths
     from vexautonomousplanner_b200.synth import FACTORY
-    ref = _gui_ref()
-    eng = Engine("cuda:0")
-    half = (FACTORY[0] / 2,) + tuple(FACTORY[1:])
-    rdir, odir = tmp_path / "routes", tmp_path / "out"
     rdir.mkdir()
     t_end = {}
-    for n, r in ref.items():
+    for n, r in _gui_ref().items():
         if "built" not in r:
             continue
         pts, nodes, aps, _ = ex.load_nodes(r["built"]["json"])
@@ -252,29 +245,61 @@ def test_check_command_on_a_folder(tmp_path, capsys):
         if all(int(x.status[0]) == 0 for x in res):
             (rdir / f"{n}.txt").write_text(r["built"]["json"])
             t_end[f"{n}.txt"] = [float(x.summary[0, 2]) for x in res]
+    return t_end
+
+
+def _reader_lines(names, odir, fresh_dir):
+    """{name: the report line of the reader's comparison of odir/name with fresh_dir/name}."""
+    from test_check_vs_reference import ref_body, ref_compare
+    from vexautonomousplanner_b200 import save_routes as sr
+    out = {}
+    for n in names:
+        new = (fresh_dir / n).read_bytes()
+        out[n] = sr.check_line(n, *ref_compare((odir / n).read_bytes(), new, ref_body(new)[0]))[1]
+    return out
+
+
+@pytest.mark.gpu
+def test_check_command_on_a_folder(tmp_path, capsys):
+    """save, then --check: every route up to date (exit 0); with --max-velocity halved every route is stale, with the
+    fresh profile's t_end as the new duration and the first run's as the old one; a deleted file is missing, a
+    corrupted token unreadable with its line (exit 1).  Every stale and unreadable line is the one the Python reader
+    of test_check_vs_reference gives for the saved file and the fresh body."""
+    from vexautonomousplanner_b200 import save_routes as sr
+    from vexautonomousplanner_b200.engine import Engine
+    from vexautonomousplanner_b200.synth import FACTORY
+    eng = Engine("cuda:0")
+    half = (FACTORY[0] / 2,) + tuple(FACTORY[1:])
+    rdir, odir, hdir = tmp_path / "routes", tmp_path / "out", tmp_path / "half"
+    t_end = _route_folder(eng, rdir, half)
     names = sorted(t_end)
     assert len(names) >= 4
     assert all(t[1] > t[0] for t in t_end.values())
     base = [str(rdir), str(odir), "--tile-paths", "3"]
     assert sr.main(base) == 0
+    assert sr.main([str(rdir), str(hdir), "--tile-paths", "3", "--max-velocity", str(half[0])]) == 0
     capsys.readouterr()
     assert sr.main(base + ["--check"]) == 0
     out = capsys.readouterr().out
     assert all(f"up to date: {n}" in out for n in names), out
 
-    assert sr.main(base + ["--check", "--max-velocity", str(FACTORY[0] / 2)]) == 1
+    assert sr.main(base + ["--check", "--max-velocity", str(half[0])]) == 1
     out = capsys.readouterr().out.splitlines()
     stale = [line for line in out if line.startswith("stale: ")]
     assert len(stale) == len(names), out
+    want = _reader_lines(names, odir, hdir)
     for line in stale:
         name = line.split(": ")[1]
+        assert line == want[name]
         dur = line.split("; duration ")[1].split(" s;")[0].split(" -> ")
         assert [float(v) for v in dur] == t_end[name], line
-        assert "first difference on line " in line and "max |dx| " in line
 
     gone = names[0]
     (odir / gone).unlink()
     bad = names[1]
+    fresh = tmp_path / "fresh"
+    fresh.mkdir()
+    (fresh / bad).write_bytes((odir / bad).read_bytes())
     lines = (odir / bad).read_text().splitlines(keepends=True)
     k = next(i for i, l in enumerate(lines) if l.startswith("0 ") and i > 5)
     tok = lines[k].split(" ")
@@ -286,5 +311,6 @@ def test_check_command_on_a_folder(tmp_path, capsys):
     out = capsys.readouterr().out
     assert f"missing: {gone}" in out
     assert f"unreadable: {bad}: line {k + 1}: token 4 (y) is not a number" in out, out
+    assert _reader_lines([bad], odir, fresh)[bad] in out.splitlines()
     assert all(f"up to date: {n}" in out for n in names[2:]), out
     assert {p.name: p.read_bytes() for p in odir.iterdir()} == before

@@ -193,6 +193,9 @@ def _pinned_text(text) -> torch.Tensor:
     return t[:a.size]
 
 
+MAX_READ_BYTES = 2 ** 31 - 1     # bytes one parse_text_batch / compare_text_batch call reads: the line scan is int32
+
+
 def _read_bodies(eng: Engine, text, path_offsets, parse_paths: int) -> ParsedText:
     """parse_text_batch, with the trajectory rows parsed for the first parse_paths bodies only (the lines, kinds,
     first-token errors and action rows of every body)."""
@@ -201,8 +204,8 @@ def _read_bodies(eng: Engine, text, path_offsets, parse_paths: int) -> ParsedTex
     host = _pinned_text(text)
     if host.numel() < N or poff[0] != 0 or (np.diff(poff) < 0).any():
         raise ValueError("path_offsets must start at 0, never decrease and end within the text")
-    if N >= 2 ** 31:
-        raise ValueError(f"{N} bytes: at most 2^31 - 1 bytes per call (tile the batch)")
+    if N > MAX_READ_BYTES:
+        raise ValueError(f"{N} bytes: at most {MAX_READ_BYTES} bytes per call (tile the batch)")
     dev, st, L_ = eng.device, eng._stream(), eng.lib
     with eng._stage("read_upload"):
         text_d = host[:max(N, 1)].to(dev, non_blocking=True) if N else torch.zeros(1, dtype=torch.uint8, device=dev)
@@ -245,7 +248,9 @@ def _read_bodies(eng: Engine, text, path_offsets, parse_paths: int) -> ParsedTex
         hb = host.numpy()
         flat, toks = [], []
         for mask, s, e, r in info.T:
-            words = bytes(hb[s:e]).split()
+            # the device's tokens: runs of ' ' separate them, '\n' ends the line; any other byte ('\t', '\r') is part
+            # of a token, so bytes.split() would number the columns differently
+            words = [w for w in bytes(hb[s:e]).rstrip(b"\n").split(b" ") if w]
             for c in range(1, 7):
                 if mask >> c & 1:
                     flat.append(int(r) * 7 + c)

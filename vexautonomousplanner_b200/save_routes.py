@@ -123,28 +123,53 @@ def check_line(name: str, ints, floats) -> Tuple[str, str]:
                      f"{i['action_rows_differ']} action rows differ")
 
 
+def byte_groups(sizes: Sequence[int], limit: int) -> List[Tuple[int, int]]:
+    """Consecutive groups [g0, g1) of items whose sizes add up to at most limit each; an item larger than limit on its
+    own is a group of one."""
+    groups, g0, total = [], 0, 0
+    for b, s in enumerate(sizes):
+        if b > g0 and total + s > limit:
+            groups.append((g0, b))
+            g0, total = b, 0
+        total += s
+    if g0 < len(sizes):
+        groups.append((g0, len(sizes)))
+    return groups
+
+
 def check_batch(eng, db, node_actions, ap_actions, files: Sequence[str]):
     """One batch of --check: profile db, assemble the fresh bodies, read the saved files[b] (missing ones as empty
-    bodies) into one pinned buffer and compare on the device.  Returns (res, ok, present, ints, floats) with ints /
-    floats as export.compare_text_batch gives them."""
+    bodies) into one pinned buffer and compare on the device, in groups of routes whose saved and fresh bodies together
+    fit one read (export.MAX_READ_BYTES).  Returns (res, ok, present, ints, floats) with ints / floats as
+    export.compare_text_batch gives them."""
     import numpy as np
     import torch
-    from .export import compare_text_batch, export_rows, save_text_batch
+    from . import export
     res = eng.profile(db)
-    text, offs, ok = save_text_batch(eng, res, db, node_actions, ap_actions)
-    rows, row_off = export_rows(eng, res)
+    text, offs, ok = export.save_text_batch(eng, res, db, node_actions, ap_actions)
+    rows, row_off = export.export_rows(eng, res)
     present = [os.path.isfile(p) for p in files]
     sizes = np.array([os.path.getsize(p) if there else 0 for p, there in zip(files, present)], dtype=np.int64)
-    old_off = np.zeros(len(files) + 1, dtype=np.int64)
-    np.cumsum(sizes, out=old_off[1:])
-    buf = torch.empty(max(int(old_off[-1] + offs[-1]), 1), dtype=torch.uint8, pin_memory=True)
+    groups = byte_groups((sizes + np.diff(offs)).tolist(), export.MAX_READ_BYTES)
+    # group by group: the saved files, then room for the fresh bodies (compare_text_batch puts them there)
+    buf = torch.empty(max(int(sizes.sum() + offs[-1]), 1), dtype=torch.uint8, pin_memory=True)
     view = memoryview(buf.numpy())
-    for p, there, a, z in zip(files, present, old_off[:-1], old_off[1:]):
-        if there:
-            with open(p, "rb") as f:
-                f.readinto(view[a:z])
-    ints, floats, _ = compare_text_batch(eng, buf, old_off, text, offs, rows, row_off)
-    return res, ok, present, ints, floats
+    ints, floats, base = [], [], 0
+    for g0, g1 in groups:
+        old_off = np.zeros(g1 - g0 + 1, dtype=np.int64)
+        np.cumsum(sizes[g0:g1], out=old_off[1:])
+        for p, there, a, z in zip(files[g0:g1], present[g0:g1], base + old_off[:-1], base + old_off[1:]):
+            if there:
+                with open(p, "rb") as f:
+                    f.readinto(view[a:z])
+        n = int(old_off[-1] + offs[g1] - offs[g0])
+        # row_off[g0:g1 + 1] still indexes the whole batch's rows
+        gi, gf, _ = export.compare_text_batch(eng, buf[base:base + n], old_off, text[offs[g0]:offs[g1]],
+                                              offs[g0:g1 + 1] - offs[g0], rows, row_off[g0:g1 + 1])
+        ints.append(gi)
+        floats.append(gf)
+        base += n
+    return res, ok, present, np.concatenate(ints), np.concatenate(floats)
 
 
 def check_routes(routes: Sequence, out_dir: str, cons, tile_paths: int = 8192, device: str = "cuda:0"):
