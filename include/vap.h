@@ -388,6 +388,27 @@ int vap_compare_bodies(int64_t B, const char* text, const int64_t* old_off, cons
                        const int64_t* old_row_off, const double* new_rows, const int64_t* new_row_off, int64_t* out_i64,
                        double* out_f64, void* stream);
 
+/* The robot's rectangle along the export rows, per path b (one CTA each): rows[R][7] = {0, t, x, y, heading, v, omega}
+ * (inches, heading CCW from +x), path b owning rows row_off[b] .. row_off[b+1] (row_off[B+1] i64: vap_export_rows, or
+ * the rows vap_parse_rows read back).  The rectangle is centred on (x, y), hl inches to the front and back along the
+ * heading, hw inches to each side; the field is xmin..xmax by ymin..ymax; boxes (HOST memory, K <= 64) [K][4] =
+ * {x0, y0, x1, y1} are axis-aligned keep-out boxes.  Per row: wall margin = largest overhang of a corner past a field
+ * edge (negative: clearance), box distance = Euclidean distance between the rectangles, or minus the penetration depth
+ * (the smallest overlap of the four separating axes) when they overlap.  A row violates when its wall margin > tol, a
+ * box distance < -tol, or x, y or heading is not finite.  Row numbers count from 0 within the path; ties go to the
+ * lowest row, then the lowest box.
+ *   out_i64[B][7]: rows, first violating row (-1 none), its kind (-1 none, 0 wall, 1 not finite, 2 + k box k), number
+ *     of violating rows, row of the largest wall margin, row of the smallest box distance and that box (-1 / -1 when
+ *     K = 0; -1 everywhere without a finite row).
+ *   out_f64[B][6]: t of the first violation (NaN none), largest wall margin (-inf without a finite row) and its t,
+ *     smallest box distance (+inf when K = 0) and its t, largest displacement of a corner between consecutive finite
+ *     rows (what sampling can miss between two rows).
+ * Returns < 0 with vap_last_error for hl or hw not positive, an empty field box, K outside 0..64, an empty box, or a
+ * tolerance that is not finite.                                                                                    */
+int vap_footprint_check(int64_t B, const double* rows, const int64_t* row_off, double hl, double hw, double xmin, double xmax,
+                        double ymin, double ymax, int K, const double* boxes, double tol, int64_t* out_i64, double* out_f64,
+                        void* stream);
+
 /* Bounds diagnostics of a -DVAP_BOUNDS_CHECK build (profiles/tools/bounds_check.py; compute-sanitizer is closed on the GPU
  * pool this was developed on): out_host[32] (HOST memory) = violations per check site (0..15) and checks executed per site
  * (16..31); returns <0 in a release build, where the checks are compiled away.                                          */

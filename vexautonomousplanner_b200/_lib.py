@@ -26,6 +26,7 @@ SYMBOLS = [
     "vap_event_scratch_ints", "vap_pass_row_slots", "vap_velocity_profile", "vap_time_profile", "vap_workspace_bytes", "vap_profile_batch", "vap_summary", "vap_pack_rows", "vap_export_rows", "vap_format_doubles", "vap_row_text_stride",
     "vap_format_rows", "vap_compact_rows", "vap_splice_plan", "vap_splice_actions", "vap_row_kinds",
     "vap_parse_doubles", "vap_line_starts", "vap_line_offsets", "vap_line_kinds", "vap_parse_rows", "vap_compare_bodies",
+    "vap_footprint_check",
 "vap_bench_dfma", "vap_test_div_const", "vap_test_div_recip", "vap_build_lerp_recip", "vap_diag_read",
 ]
 

@@ -17,6 +17,7 @@
 #include "vap_timeloop.cuh"
 #include "vap_format.cuh"
 #include "vap_parse.cuh"
+#include "vap_footprint.cuh"
 
 static thread_local char g_err[512] = "";
 static int set_err(const char* where, cudaError_t e)
@@ -1770,6 +1771,38 @@ extern "C" int vap_compare_bodies(int64_t B, const char* text, const int64_t* ol
                                                                   P(new_path_act_off), old_rows, P(old_row_off), new_rows,
                                                                   P(new_row_off), reinterpret_cast<long long*>(out_i64), out_f64);
     CHECK_LAUNCH("vap_compare_bodies");
+    return 0;
+}
+
+// ---- the robot's footprint along the export rows (vap_footprint.cuh) ------------------------------------------------
+extern "C" int vap_footprint_check(int64_t B, const double* rows, const int64_t* row_off, double hl, double hw, double xmin,
+                                   double xmax, double ymin, double ymax, int K, const double* boxes, double tol,
+                                   int64_t* out_i64, double* out_f64, void* stream)
+{
+    if (B < 0) return arg_err("vap_footprint_check: B >= 0 required");
+    if (!(hl > 0) || !(hw > 0) || !isfinite(hl) || !isfinite(hw))
+        return arg_err("vap_footprint_check: the half-length and half-width must be positive and finite");
+    if (!(xmin < xmax) || !(ymin < ymax)) return arg_err("vap_footprint_check: empty field box (xmin < xmax and ymin < ymax required)");
+    if (!isfinite(tol)) return arg_err("vap_footprint_check: the tolerance must be finite");
+    if (K < 0 || K > FP_MAX_BOXES) return arg_err("vap_footprint_check: 0 <= K <= 64 keep-out boxes required");
+    if (K > 0 && boxes == nullptr) return arg_err("vap_footprint_check: boxes is NULL");
+    FpArgs a;
+    memset(&a, 0, sizeof(a));
+    a.hl = hl; a.hw = hw; a.xmin = xmin; a.xmax = xmax; a.ymin = ymin; a.ymax = ymax; a.tol = tol; a.K = K;
+    for (int k = 0; k < K; k++) {
+        const double* q = boxes + 4 * k;
+        if (!(q[0] < q[2]) || !(q[1] < q[3]) || !isfinite(q[0]) || !isfinite(q[1]) || !isfinite(q[2]) || !isfinite(q[3])) {
+            snprintf(g_err, sizeof(g_err), "vap_footprint_check: keep-out box %d is empty or not finite (x0 < x1 and y0 < y1 "
+                     "required, got %g, %g, %g, %g)", k, q[0], q[1], q[2], q[3]);
+            return -101;
+        }
+        for (int j = 0; j < 4; j++) a.box[k][j] = q[j];
+    }
+    if (B == 0) return 0;
+    const unsigned grid = (unsigned)(B < 1048576 ? B : 1048576);
+    k_footprint_check<<<grid, FP_THREADS, 0, STREAM>>>(B, rows, reinterpret_cast<const long long*>(row_off), a,
+                                                       reinterpret_cast<long long*>(out_i64), out_f64);
+    CHECK_LAUNCH("vap_footprint_check");
     return 0;
 }
 

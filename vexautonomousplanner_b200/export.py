@@ -309,6 +309,52 @@ def compare_text_batch(eng: Engine, old_text, old_offsets, new_text, new_offsets
     return out_i[:B].cpu().numpy(), out_f[:B].cpu().numpy(), p.n_host                # read-back 4
 
 
+FP_I = ("rows", "first_row", "first_kind", "violating_rows", "worst_wall_row", "nearest_box_row", "nearest_box")
+FP_F = ("first_t", "worst_wall_in", "worst_wall_t", "nearest_box_in", "nearest_box_t", "max_corner_step_in")
+FP_KIND_WALL, FP_KIND_NONFINITE, FP_KIND_BOX = 0, 1, 2
+FP_MAX_BOXES = 64
+
+
+def default_field():
+    """(xmin, xmax, ymin, ymax) in inches: the GUI's 2000-px canvas, which it clamps nodes into."""
+    lo, hi = px_to_in(0), px_to_in(2000)
+    return lo, hi, lo, hi
+
+
+def footprint_check(eng: Engine, rows, row_offsets, length_in: float, width_in: float, field=None, keep_out=(),
+                    tol_in: float = 0.0):
+    """Does a robot length_in long (along the heading) and width_in wide, centred on every export row, stay on the field
+    and clear the keep-out boxes?  Per path, on the device (vap_footprint_check).
+    rows / row_offsets: rows[R, 7] fp64 {0, t, x, y, heading, v, omega} in the .txt frame (inches, heading CCW from +x)
+    and int64[B+1] offsets, path b owning rows row_offsets[b] .. [b+1] -- export_rows(eng, res) gives them for fresh
+    profiles, parse_text_batch(...).rows / .row_offsets for saved files.  field: (xmin, xmax, ymin, ymax) in inches,
+    None = default_field(); keep_out: up to 64 boxes (x0, y0, x1, y1) in inches in the same frame; tol_in: overhangs
+    and penetrations up to tol_in inches do not count.
+    Returns (ints int64[B, 7] named by FP_I, floats fp64[B, 6] named by FP_F), host arrays, with one read-back:
+    rows, first violating row (-1 none) and its kind (-1, FP_KIND_WALL, FP_KIND_NONFINITE, FP_KIND_BOX + k for box k),
+    violating rows, row of the largest wall margin, row and index of the nearest box; t of the first violation, largest
+    wall margin (positive: overhang, negative: clearance) and its t, nearest box distance (negative: penetration
+    depth; +inf without boxes) and its t, and the largest corner displacement between consecutive rows (the sampling
+    resolution: an excursion shorter than this between two rows is not seen).  Rows count from 0 within the path.
+    Raises VapError for a non-positive size, an empty field or box, or more than 64 boxes."""
+    rows = torch.as_tensor(rows, dtype=torch.float64, device=eng.device).contiguous()
+    roff = torch.as_tensor(row_offsets, dtype=torch.int64, device=eng.device).contiguous()
+    B = roff.shape[0] - 1
+    xmin, xmax, ymin, ymax = default_field() if field is None else (float(v) for v in field)
+    boxes = np.ascontiguousarray(np.asarray(keep_out, dtype=np.float64).reshape(-1, 4))
+    K = boxes.shape[0]
+    buf = torch.empty(max(B, 1) * (len(FP_I) + len(FP_F)), dtype=torch.int64, device=eng.device)
+    out_f = buf[max(B, 1) * len(FP_I):].view(torch.float64)
+    _lib.check(eng.lib.vap_footprint_check(C.c_int64(B), _p(rows), _p(roff), C.c_double(length_in / 2),
+                                           C.c_double(width_in / 2), C.c_double(xmin), C.c_double(xmax), C.c_double(ymin),
+                                           C.c_double(ymax), C.c_int(K), boxes.ctypes.data_as(C.c_void_p),
+                                           C.c_double(tol_in), _p(buf), _p(out_f), eng._stream()), "vap_footprint_check")
+    eng.launches += 1
+    host = buf.cpu().numpy()                                                             # the one read-back
+    n_i = max(B, 1) * len(FP_I)
+    return host[:n_i].reshape(-1, len(FP_I))[:B], host[n_i:].view(np.float64).reshape(-1, len(FP_F))[:B]
+
+
 def splice_action_rows(traj_rows: Sequence[Sequence[float]], nodes_map: Sequence[int], node_actions: Sequence[Sequence],
                        actions_map: Sequence[int] = (), action_rows: Sequence[Sequence] = ()) -> List[list]:
     """gui_manager.py:284-310: trajectory rows with the node / action-point rows inserted at map[i] + i."""

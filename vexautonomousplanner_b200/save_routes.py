@@ -198,18 +198,23 @@ def check_routes(routes: Sequence, out_dir: str, cons, tile_paths: int = 8192, d
     return out
 
 
-def parse_args(argv: Optional[List[str]] = None) -> argparse.Namespace:
-    p = argparse.ArgumentParser(prog="python -m vexautonomousplanner_b200.save_routes",
-                                description="Re-save every route of a folder: write each route's trajectory .txt.")
-    p.add_argument("routes_dir", help="folder of node-JSON routes (*.txt), the GUI's routes folder")
-    p.add_argument("out_dir", help="folder for the trajectory files (must differ from routes_dir)")
-    p.add_argument("--config", help="config.yaml in the GUI's layout (motion.*, robot.track_width in inches)")
+def add_constraint_flags(p: argparse.ArgumentParser) -> None:
+    """--max-velocity, --max-acceleration, --max-jerk, --track-width-in (what constraints() reads besides --config)."""
     p.add_argument("--max-velocity", type=float, dest="max_velocity", help=f"ft/s (factory {DEFAULTS['max_velocity']})")
     p.add_argument("--max-acceleration", type=float, dest="max_acceleration",
                    help=f"ft/s^2, also the deceleration (factory {DEFAULTS['max_acceleration']})")
     p.add_argument("--max-jerk", type=float, dest="max_jerk", help=f"ft/s^3 (factory {DEFAULTS['max_jerk']})")
     p.add_argument("--track-width-in", type=float, dest="track_width_in",
                    help=f"track width in inches (factory {DEFAULTS['track_width_in']})")
+
+
+def parse_args(argv: Optional[List[str]] = None) -> argparse.Namespace:
+    p = argparse.ArgumentParser(prog="python -m vexautonomousplanner_b200.save_routes",
+                                description="Re-save every route of a folder: write each route's trajectory .txt.")
+    p.add_argument("routes_dir", help="folder of node-JSON routes (*.txt), the GUI's routes folder")
+    p.add_argument("out_dir", help="folder for the trajectory files (must differ from routes_dir)")
+    p.add_argument("--config", help="config.yaml in the GUI's layout (motion.*, robot.track_width in inches)")
+    add_constraint_flags(p)
     p.add_argument("--tile-paths", type=int, default=8192, help="routes profiled per batch (default 8192)")
     p.add_argument("--device", default="cuda:0")
     p.add_argument("--check", action="store_true",
