@@ -409,6 +409,38 @@ int vap_footprint_check(int64_t B, const double* rows, const int64_t* row_off, d
                         double ymin, double ymax, int K, const double* boxes, double tol, int64_t* out_i64, double* out_f64,
                         void* stream);
 
+/* Pose planes of a row set for vap_pair_check, one CTA per route b: rows[R][7] = {0, t, x, y, heading, v, omega} with
+ * route b owning rows row_off[b] .. row_off[b+1] (row_off[B+1] i64, row_off[B] <= R).  Writes planes[5][R] (fp64,
+ * plane-major) = t, x, y, cos heading, sin heading of every row, and bad[B][2] i64 = {first invalid row, reason}:
+ * {-1, 0} for a valid route, {-1, 1} for a route without rows, {r, 2} when row r is the first whose t, x, y or heading
+ * is not finite, {r, 3} when t at row r is smaller than at row r - 1.  Returns < 0 for B < 0 or R < 0.            */
+int vap_pose_planes(int64_t B, const double* rows, const int64_t* row_off, int64_t R, double* planes, int64_t* bad,
+                    void* stream);
+
+/* Two robots running two routes at the same time, one CTA per pair p: route pairs[p][0] of row set A against route
+ * pairs[p][1] of row set B (pairs[P][2] i64), each set given by its vap_pose_planes output (planes[5][R], bad[B][2])
+ * and its row_off[B+1].  Robot A is a rectangle centred on (x, y) reaching hl_a along the heading and hw_a across it
+ * (inches); robot B likewise with hl_b, hw_b.  Both start at t = 0 of their own rows.
+ *   Events: every row of either route.  At the event of A's row i, A is at row i and B at its held pose, its last row
+ *     with t <= t_i; before its first row B is at its first row, after its last row it stays parked there.  B's rows
+ *     likewise with the roles swapped.
+ *   Distance: with overlap on all four separating axes (each robot's heading and normal) minus the smallest overlap
+ *     (the penetration depth), else the Euclidean distance between the rectangles.  A contact is a distance < min_gap.
+ *   Order: events are keyed (t, side, row), side A = 0 before B = 1, rows from 0 within the route.  The first contact
+ *     is the contact with the smallest key; the nearest event has the smallest distance, the smallest key winning ties.
+ *   out_i64[P][7]: status (0 checked, 1 route A invalid, 2 route B invalid, 3 a pair index outside 0 .. B - 1),
+ *     events (na + nb; 0 when not checked), first-contact side and row (-1 none), contact events, nearest side and row.
+ *   out_f64[P][6]: first-contact t (NaN none), nearest distance (+inf when not checked) and its t, last t of A, last t
+ *     of B (NaN when not checked), largest move of a robot's corner between consecutive rows of its own route (the
+ *     resolution of the check: it does not sweep between rows).
+ * With strictly increasing t on both routes, swapping A and B gives bit-identical first-contact t, nearest distance,
+ * nearest t and contact count.  Returns < 0 with vap_last_error for P, B_a or B_b < 0, pairs NULL with P > 0, a
+ * half-size that is not positive and finite, or a min_gap that is not finite.                                   */
+int vap_pair_check(int64_t P, const int64_t* pairs, int64_t B_a, const double* planes_a, int64_t R_a, const int64_t* off_a,
+                   const int64_t* bad_a, double hl_a, double hw_a, int64_t B_b, const double* planes_b, int64_t R_b,
+                   const int64_t* off_b, const int64_t* bad_b, double hl_b, double hw_b, double min_gap, int64_t* out_i64,
+                   double* out_f64, void* stream);
+
 /* Bounds diagnostics of a -DVAP_BOUNDS_CHECK build (profiles/tools/bounds_check.py; compute-sanitizer is closed on the GPU
  * pool this was developed on): out_host[32] (HOST memory) = violations per check site (0..15) and checks executed per site
  * (16..31); returns <0 in a release build, where the checks are compiled away.                                          */

@@ -18,6 +18,7 @@
 #include "vap_format.cuh"
 #include "vap_parse.cuh"
 #include "vap_footprint.cuh"
+#include "vap_pairs.cuh"
 
 static thread_local char g_err[512] = "";
 static int set_err(const char* where, cudaError_t e)
@@ -1803,6 +1804,43 @@ extern "C" int vap_footprint_check(int64_t B, const double* rows, const int64_t*
     k_footprint_check<<<grid, FP_THREADS, 0, STREAM>>>(B, rows, reinterpret_cast<const long long*>(row_off), a,
                                                        reinterpret_cast<long long*>(out_i64), out_f64);
     CHECK_LAUNCH("vap_footprint_check");
+    return 0;
+}
+
+// ---- two robots at the same time (vap_pairs.cuh) ---------------------------------------------------------------------
+extern "C" int vap_pose_planes(int64_t B, const double* rows, const int64_t* row_off, int64_t R, double* planes, int64_t* bad,
+                               void* stream)
+{
+    if (B < 0 || R < 0) return arg_err("vap_pose_planes: B >= 0 and R >= 0 required");
+    if (B == 0) return 0;
+    const unsigned grid = (unsigned)(B < 1048576 ? B : 1048576);
+    k_pose_planes<<<grid, PC_THREADS, 0, STREAM>>>(B, rows, reinterpret_cast<const long long*>(row_off), R, planes,
+                                                   reinterpret_cast<long long*>(bad));
+    CHECK_LAUNCH("vap_pose_planes");
+    return 0;
+}
+
+extern "C" int vap_pair_check(int64_t P, const int64_t* pairs, int64_t B_a, const double* planes_a, int64_t R_a,
+                              const int64_t* off_a, const int64_t* bad_a, double hl_a, double hw_a, int64_t B_b,
+                              const double* planes_b, int64_t R_b, const int64_t* off_b, const int64_t* bad_b, double hl_b,
+                              double hw_b, double min_gap, int64_t* out_i64, double* out_f64, void* stream)
+{
+    if (P < 0 || B_a < 0 || B_b < 0) return arg_err("vap_pair_check: P >= 0, B_a >= 0 and B_b >= 0 required");
+    if (P > 0 && pairs == nullptr) return arg_err("vap_pair_check: pairs is NULL");
+    const double h[4] = {hl_a, hw_a, hl_b, hw_b};
+    for (double v : h)
+        if (!(v > 0) || !isfinite(v))
+            return arg_err("vap_pair_check: every half-length and half-width must be positive and finite");
+    if (!isfinite(min_gap)) return arg_err("vap_pair_check: min_gap must be finite");
+    if (P == 0) return 0;
+    const PcSide a = {planes_a, reinterpret_cast<const long long*>(off_a), reinterpret_cast<const long long*>(bad_a), B_a, R_a,
+                      hl_a, hw_a};
+    const PcSide b = {planes_b, reinterpret_cast<const long long*>(off_b), reinterpret_cast<const long long*>(bad_b), B_b, R_b,
+                      hl_b, hw_b};
+    const unsigned grid = (unsigned)(P < 1048576 ? P : 1048576);
+    k_pair_check<<<grid, PC_THREADS, 0, STREAM>>>(P, reinterpret_cast<const long long*>(pairs), a, b, min_gap,
+                                                  reinterpret_cast<long long*>(out_i64), out_f64);
+    CHECK_LAUNCH("vap_pair_check");
     return 0;
 }
 

@@ -355,6 +355,78 @@ def footprint_check(eng: Engine, rows, row_offsets, length_in: float, width_in: 
     return host[:n_i].reshape(-1, len(FP_I))[:B], host[n_i:].view(np.float64).reshape(-1, len(FP_F))[:B]
 
 
+PC_I = ("status", "events", "first_side", "first_row", "contacts", "nearest_side", "nearest_row")
+PC_F = ("first_t", "nearest_in", "nearest_t", "last_t_a", "last_t_b", "max_corner_step_in")
+PC_OK, PC_A_INVALID, PC_B_INVALID, PC_BAD_INDEX = 0, 1, 2, 3                 # status
+PC_BAD_NONE, PC_BAD_EMPTY, PC_BAD_NONFINITE, PC_BAD_DECREASING = 0, 1, 2, 3  # reason of bad[b] = (row, reason)
+
+
+def pair_reason_text(row: int, reason: int) -> str:
+    """What bad[b] = (row, reason) of pair_check says about a route."""
+    if reason == PC_BAD_EMPTY:
+        return "no trajectory rows"
+    if reason == PC_BAD_NONFINITE:
+        return f"row {row} is not finite"
+    if reason == PC_BAD_DECREASING:
+        return f"t decreases at row {row}"
+    return "valid" if reason == PC_BAD_NONE else f"reason {reason}"
+
+
+def _pose_planes(eng: Engine, rows, roff: torch.Tensor, bad: torch.Tensor):
+    """vap_pose_planes: planes fp64[5 * R] of rows, bad[b] = (row, reason) written into bad (int64[B, 2])."""
+    rows = torch.as_tensor(rows, dtype=torch.float64, device=eng.device).reshape(-1, 7).contiguous()
+    R = int(rows.shape[0])
+    planes = torch.empty(5 * max(R, 1), dtype=torch.float64, device=eng.device)
+    _lib.check(eng.lib.vap_pose_planes(C.c_int64(roff.shape[0] - 1), _p(rows), _p(roff), C.c_int64(R), _p(planes), _p(bad),
+                                       eng._stream()), "vap_pose_planes")
+    eng.launches += 1
+    return planes, R
+
+
+def pair_check(eng: Engine, rows_a, off_a, size_a, rows_b, off_b, size_b, pairs, min_gap_in: float = 0.0):
+    """Two robots driving two routes at the same time: where do their rectangles first come closer than min_gap_in?
+    On the device (vap_pose_planes, vap_pair_check).
+    rows_a / off_a: row set A, rows[R, 7] fp64 {0, t, x, y, heading, v, omega} in the .txt frame (inches, heading CCW
+    from +x) and int64[B_a+1] offsets -- export_rows(eng, res) for fresh profiles, parse_text_batch(...).rows /
+    .row_offsets for saved files; rows_b / off_b likewise.  When rows_b is rows_a and off_b is off_a (one route set on
+    both sides) the planes and the per-route checks are built once; other offsets into the same rows get their own,
+    since whether t decreases depends on where each route begins.  size_a, size_b: (length_in, width_in) of each
+    robot, length along the heading.  pairs: int64[P, 2] of (route of A, route of B).
+    Every row of either route is an event; at it the other robot holds its last row with t <= the event's t (its first
+    row before it starts, its last row once it has finished).  An event is a contact when the signed distance of the
+    rectangles (negative: penetration depth) is < min_gap_in; events are ordered by (t, side, row), side A = 0.
+    Returns host arrays (ints int64[P, 7] named by PC_I, floats fp64[P, 6] named by PC_F, bad_a int64[B_a, 2],
+    bad_b int64[B_b, 2]) with one read-back: per pair the status (PC_OK, PC_A_INVALID, PC_B_INVALID, PC_BAD_INDEX),
+    events, first contact's side and row (-1 none) and t (NaN), contact events, the nearest event's side, row, distance
+    and t, both routes' last t, and the largest corner move between consecutive rows of either route (the check's
+    resolution); per route (row, reason) of its first invalid row (pair_reason_text explains it).
+    Raises VapError for a size that is not positive and finite or a min_gap_in that is not finite."""
+    (la, wa), (lb, wb) = ((float(v) for v in size_a), (float(v) for v in size_b))
+    same = rows_b is rows_a and off_b is off_a
+    roff_a = torch.as_tensor(off_a, dtype=torch.int64, device=eng.device).contiguous()
+    roff_b = roff_a if same else torch.as_tensor(off_b, dtype=torch.int64, device=eng.device).contiguous()
+    B_a, B_b = roff_a.shape[0] - 1, roff_b.shape[0] - 1
+    pr = torch.from_numpy(np.ascontiguousarray(np.asarray(pairs, dtype=np.int64).reshape(-1, 2))).to(eng.device)
+    P = int(pr.shape[0])
+    n_i, n_f, n_a = max(P, 1) * len(PC_I), max(P, 1) * len(PC_F), 2 * max(B_a, 1)
+    buf = torch.empty(n_i + n_f + n_a + 2 * max(B_b, 1), dtype=torch.int64, device=eng.device)
+    out_f = buf[n_i:n_i + n_f].view(torch.float64)
+    bad_a, bad_b = buf[n_i + n_f:n_i + n_f + n_a], buf[n_i + n_f + n_a:]
+    pa, R_a = _pose_planes(eng, rows_a, roff_a, bad_a)
+    pb, R_b = (pa, R_a) if same else _pose_planes(eng, rows_b, roff_b, bad_b)
+    _lib.check(eng.lib.vap_pair_check(
+        C.c_int64(P), _p(pr), C.c_int64(B_a), _p(pa), C.c_int64(R_a), _p(roff_a), _p(bad_a), C.c_double(la / 2),
+        C.c_double(wa / 2), C.c_int64(B_b), _p(pb), C.c_int64(R_b), _p(roff_b), _p(bad_a if same else bad_b),
+        C.c_double(lb / 2), C.c_double(wb / 2), C.c_double(min_gap_in), _p(buf), _p(out_f), eng._stream()),
+        "vap_pair_check")
+    eng.launches += 1
+    host = buf.cpu().numpy()                                                             # the one read-back
+    o = n_i + n_f
+    ha = host[o:o + 2 * B_a].reshape(-1, 2)
+    hb = ha if same else host[o + n_a:o + n_a + 2 * B_b].reshape(-1, 2)
+    return host[:n_i].reshape(-1, len(PC_I))[:P], host[n_i:o].view(np.float64).reshape(-1, len(PC_F))[:P], ha, hb
+
+
 def splice_action_rows(traj_rows: Sequence[Sequence[float]], nodes_map: Sequence[int], node_actions: Sequence[Sequence],
                        actions_map: Sequence[int] = (), action_rows: Sequence[Sequence] = ()) -> List[list]:
     """gui_manager.py:284-310: trajectory rows with the node / action-point rows inserted at map[i] + i."""

@@ -149,20 +149,24 @@ def check_routes(routes: Sequence, cons, size, field, boxes, tol_in: float, tile
     return out
 
 
-def check_trajectories(folder: str, size, field, boxes, tol_in: float, device: str = "cuda:0"):
-    """Read every *.txt of folder back on the device (groups of at most export.MAX_READ_BYTES) and check its
-    footprint.  Returns [(name, state, report line)]."""
+def trajectory_files(folder: str) -> List[str]:
+    """The *.txt files of folder that trajectory_groups reads, sorted by name."""
+    return sorted(n for n in os.listdir(folder) if n.endswith(".txt") and os.path.isfile(os.path.join(folder, n)))
+
+
+def trajectory_groups(eng, folder: str):
+    """Read every *.txt of folder (sorted by name) back on the device, in consecutive groups of at most
+    export.MAX_READ_BYTES, each through one pinned buffer and one export.parse_text_batch call.  Yields
+    (names, parsed, errors) per group: parsed is the group's ParsedText, and errors maps the index of a file within
+    names to (line, reason) of its first line error.  A file larger than the limit comes alone with parsed None."""
     import numpy as np
     import torch
     from . import export
-    from .engine import Engine
-    names = sorted(n for n in os.listdir(folder) if n.endswith(".txt") and os.path.isfile(os.path.join(folder, n)))
+    names = trajectory_files(folder)
     sizes = [os.path.getsize(os.path.join(folder, n)) for n in names]
-    eng = Engine(device)
-    out = []
     for g0, g1 in byte_groups(sizes, export.MAX_READ_BYTES):
         if sizes[g0] > export.MAX_READ_BYTES:
-            out.append((names[g0], "not checked", f"not checked: {names[g0]}: more than {export.MAX_READ_BYTES} bytes"))
+            yield names[g0:g1], None, {}
             continue
         offs = np.zeros(g1 - g0 + 1, dtype=np.int64)
         np.cumsum(sizes[g0:g1], out=offs[1:])
@@ -172,19 +176,33 @@ def check_trajectories(folder: str, size, field, boxes, tol_in: float, device: s
             with open(os.path.join(folder, n), "rb") as f:
                 f.readinto(view[a:z])
         p = export.parse_text_batch(eng, buf[:int(offs[-1])], offs)
-        ints, floats = export.footprint_check(eng, p.rows, p.row_offsets, *size, field=field, keep_out=boxes,
-                                              tol_in=tol_in)
         bad = torch.nonzero(p.line_errors).flatten()
-        first_err = {}
+        errors = {}
         if bad.numel():
             codes = p.line_errors[bad].cpu().numpy()
             lines, pl = bad.cpu().numpy(), p.path_line_offsets.cpu().numpy()
             for line, code, b in zip(lines, codes, np.searchsorted(pl, lines, side="right") - 1):
-                first_err.setdefault(int(b), (int(line - pl[b]) + 1, int(code)))
-        for b, name in enumerate(names[g0:g1]):
-            if b in first_err:
-                line, code = first_err[b]
-                out.append((name, "unreadable", f"unreadable: {name}: line {line}: {export.line_error_text(code)}"))
+                errors.setdefault(int(b), (int(line - pl[b]) + 1, export.line_error_text(int(code))))
+        yield names[g0:g1], p, errors
+
+
+def check_trajectories(folder: str, size, field, boxes, tol_in: float, device: str = "cuda:0"):
+    """Read every *.txt of folder back on the device (trajectory_groups) and check its footprint.  Returns
+    [(name, state, report line)]."""
+    from . import export
+    from .engine import Engine
+    eng = Engine(device)
+    out = []
+    for names, p, errors in trajectory_groups(eng, folder):
+        if p is None:
+            out.append((names[0], "not checked", f"not checked: {names[0]}: more than {export.MAX_READ_BYTES} bytes"))
+            continue
+        ints, floats = export.footprint_check(eng, p.rows, p.row_offsets, *size, field=field, keep_out=boxes,
+                                              tol_in=tol_in)
+        for b, name in enumerate(names):
+            if b in errors:
+                line, why = errors[b]
+                out.append((name, "unreadable", f"unreadable: {name}: line {line}: {why}"))
             else:
                 out.append((name, *report_line(name, ints[b], floats[b], len(boxes))))
     return out
